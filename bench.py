@@ -2,7 +2,7 @@
 """bench.py — env-steps/s of the batched Astro tick on N B200s, as a fraction of the HBM roofline,
 next to the CPU step loop timed on the same box.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -335,6 +335,31 @@ def profile_entry(ticks_per_launch):
         return None
 
 
+DUMP_GAMES = 16384          # --dump-outputs: games in the fixed sample whose state is written
+DUMP_BYTES = 60 << 20       # ... and the most the sample may take (a large --bullet-cap shrinks it)
+
+
+def dump_outputs(out_dir, games, planes, stats):
+    """--dump-outputs: what the timed loop hands its caller after its last tick, as float64 DIR/<name>.npy, for comparing
+    two builds output for output.  A fixed sample of games (seeded, sorted; every game when there are fewer than
+    DUMP_GAMES): their state as get_arrays() returns it (bullet and planet rows past a game's counts zeroed) and their bits
+    of that tick's three event planes (ended, ship 0 hit, ship 1 hit); and the 14 episode counters (nat.STAT_NAMES order)."""
+    from astro_b200 import _native as nat
+    per_game = 8 * (games.S * 5 + nat.MAX_PLANETS * 4 + games.K * 4 + 5 + 3 + 1)    # state, 5 counters, 3 event bits, index
+    m = min(games.n, DUMP_GAMES, DUMP_BYTES // per_game)
+    idx = np.sort(np.random.default_rng(0).choice(games.n, size=m, replace=False))
+    out = games.get_arrays(idx)
+    out['bullets'][np.arange(out['bullets'].shape[1])[None, :] >= out['n_bullets'][:, None]] = 0.0
+    out['planets'][np.arange(out['planets'].shape[1])[None, :] >= out['n_planets'][:, None]] = 0.0
+    words = planes.cpu().numpy().view(np.uint32)                      # [3, n_tiles]: bit g % 32 of word g // 32 is game g
+    out['events'] = ((words[:, idx // 32] >> (idx % 32).astype(np.uint32)) & 1).T
+    out['game_index'] = idx
+    out['episode_stats'] = np.asarray(stats)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), np.asarray(a, dtype=np.float64))
+
+
 # --------------------------------------------------------------------------- our arm
 def run_ours(args):
     import torch
@@ -443,7 +468,7 @@ def run_ours(args):
             dist.barrier()
         return dict(games=games, ms=gather_ms(e0.elapsed_time(e1)), stats=dict(zip(nat.STAT_NAMES, (int(x) for x in st_t.cpu().numpy()))),
                     launches=games.launches - launches0, n_launches=n_launches, run_steps=run_steps, flags=flags, stats_reduce=peer or ('nccl' if world > 1 else 'none'),
-                    host_ring=host_ring, dev_ring=dev_ring, R=R)
+                    host_ring=host_ring, dev_ring=dev_ring, R=R, last_events=events_dev[(steps - 1) % R])
 
     plan = shard_plan(world, rank, args.games_per_gpu)
     n = plan['n_games']
@@ -451,6 +476,8 @@ def run_ours(args):
     sampler.start()
     main = timed_rollout(n, plan['first_game'], args.steps, args.warmup, args.fuse)
     games, flags, R, run_steps = main['games'], main['flags'], main['R'], main['run_steps']
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, games, main['last_events'], [main['stats'][k] for k in nat.STAT_NAMES])
     ms = max(main['ms'])
     per_rank_ms, timed_launches = [round(x, 4) for x in main['ms']], main['launches']
     total = main['stats']
@@ -722,6 +749,9 @@ def main():
     ap.add_argument('--fuse', type=int, default=64, help='ticks per launch of the timed loop (astro_tick_many); 1 = one launch per tick')
     ap.add_argument('--tick-flags', type=int, default=0, help='extra ASTRO_TICK_* bits (kernel A/B)')
     ap.add_argument('--timed-flags', type=int, default=0, help='extra tick bits after the pre-roll (experiment builds)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what their last tick handed back (rank 0: a fixed sample of game states '
+                         'and their events, and the episode counters) as float64 DIR/<name>.npy')
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.impl == 'reference':

@@ -43,6 +43,17 @@ from astro import core, util, script, rl  # noqa: E402  (the reference)
 from astro_b200 import rng  # noqa: E402  (shared counter-based control stream)
 
 
+def savez_lzma(path, arrays):
+    """np.savez with LZMA members instead of deflate: traj.npz stays under 1 MB (np.load reads either)."""
+    import io
+    import zipfile
+    with zipfile.ZipFile(path, 'w', compression=zipfile.ZIP_LZMA) as z:
+        for name, a in arrays.items():
+            buf = io.BytesIO()
+            np.save(buf, np.asanyarray(a), allow_pickle=False)
+            z.writestr(name + '.npy', buf.getvalue())
+
+
 def f64_state(s):
     """Canonicalise a reference State to float64 arrays (oracle definition)."""
     def b(x):
@@ -218,7 +229,7 @@ def make_traj():
     for c in it.islice(core.generate_configs(core.SOLO_CONFIG._replace(max_time=8)), 2):
         bot = script.ScriptBot.create(c)
         add('solo_script_timeout', c, lambda s, k, bot=bot: np.array([bot(s)]))
-    np.savez_compressed(os.path.join(HERE, 'traj.npz'), **arrays)
+    savez_lzma(os.path.join(HERE, 'traj.npz'), arrays)
     with open(os.path.join(HERE, 'traj.json'), 'w') as f:
         json.dump(meta, f, indent=1)
 
