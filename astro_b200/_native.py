@@ -6,11 +6,13 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('ASTRO_B200_LIB') or os.path.join(HERE, 'libastro_b200.so')   # env: A/B builds
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 TILE = 32
 MAX_PLANETS = 4
+MAX_PLANETS_WIDE = 8     # AstroConfig.planet_slots = 8: games of up to eight planets
 MAX_BULLET_CAP = 1023
 MAX_TICKS = 262143
+MAX_TICKS_WIDE = 131071   # 17-bit tick counter of 8-slot batches
 SINCOS_RANGE = 71476       # |bearing| over which util.direction (numpy float32 sin/cos) is reproduced bit for bit
 N_STATS = 14
 STAT_NAMES = ('episodes', 'wins0', 'wins1', 'both_lost', 'timeouts', 'env_steps', 'bullets_spawned',
@@ -34,7 +36,7 @@ EXPORTS = ('astro_abi_version', 'astro_last_error', 'astro_batch_create', 'astro
 class AstroConfig(C.Structure):
     _fields_ = [(n, C.c_double) for n in (
         'gravity', 'dt', 'max_time', 'reload_time', 'bullet_speed', 'ship_thrust', 'ship_rspeed',
-        'ship_radius', 'planet_mass', 'planet_radius')] + [('solo', C.c_int32), ('reserved', C.c_int32)]
+        'ship_radius', 'planet_mass', 'planet_radius')] + [('solo', C.c_int32), ('planet_slots', C.c_int32)]
 
 
 class AstroBuffers(C.Structure):
@@ -59,7 +61,7 @@ class AstroGameArrays(C.Structure):
 
 
 class AstroSingleGame(C.Structure):
-    _fields_ = [('ships', C.c_double * 5 * 2), ('planets', C.c_double * 4 * MAX_PLANETS),
+    _fields_ = [('ships', C.c_double * 5 * 2), ('planets', C.c_double * 4 * MAX_PLANETS_WIDE),
                 ('n_planets', C.c_int32), ('n_bullets', C.c_int32), ('tick', C.c_int32), ('reserved', C.c_int32),
                 ('episode', C.c_uint32), ('finished', C.c_uint8 * 4), ('control', C.c_uint8 * (TILE * 2)),
                 ('events', C.c_uint8 * TILE)]

@@ -24,13 +24,30 @@ def _torch():
     return torch
 
 
+def planet_slots_for(config):
+    """Planet slots per game of a batch playing `config`: 4 for max_planets <= 4 (the batch is laid out exactly as
+    before 8-slot batches existed), 8 for max_planets 5..8."""
+    mp = int(config.max_planets)
+    if mp > nat.MAX_PLANETS_WIDE:
+        raise ValueError('config.max_planets=%d: games of at most %d planets are supported' % (mp, nat.MAX_PLANETS_WIDE))
+    return nat.MAX_PLANETS if mp <= nat.MAX_PLANETS else nat.MAX_PLANETS_WIDE
+
+
 class BatchedGames:
-    def __init__(self, config, n_games, bullet_cap=32, precision=32, device=None, seed=0, first_game=0):
+    def __init__(self, config, n_games, bullet_cap=32, precision=32, device=None, seed=0, first_game=0, planet_slots=None):
+        """planet_slots: planet rows per game, 4 or 8; by default planet_slots_for(config).  8 slots hold games of up to
+        eight planets (the `planets` tensor is [tiles, 8, 32, 4], game-major arrays [m, 8, 4])."""
         torch = _torch()
         if precision not in (32, 64):
             raise ValueError('precision must be 32 or 64')
         if not 0 <= bullet_cap <= nat.MAX_BULLET_CAP:
             raise ValueError('bullet_cap out of range')
+        default_pl = planet_slots_for(config)
+        self.PL = default_pl if planet_slots is None else int(planet_slots)
+        if self.PL not in (nat.MAX_PLANETS, nat.MAX_PLANETS_WIDE):
+            raise ValueError('planet_slots must be %d or %d' % (nat.MAX_PLANETS, nat.MAX_PLANETS_WIDE))
+        if self.PL < default_pl:
+            raise ValueError('config.max_planets=%d needs planet_slots=%d' % (int(config.max_planets), default_pl))
         self.config = config
         self.S = 1 if config.solo else 2
         self.D = 1 + 5 * self.S + 4
@@ -46,10 +63,10 @@ class BatchedGames:
         dev, T, S, K = self.device, self.n_tiles, self.S, self.K
         self.ships = torch.zeros((T, S, 32, 4), dtype=self.rdtype, device=dev)
         self.ship_b = torch.zeros((T, S, 32), dtype=self.rdtype, device=dev)
-        self.planets = torch.zeros((T, nat.MAX_PLANETS, 32, 4), dtype=self.rdtype, device=dev)
+        self.planets = torch.zeros((T, self.PL, 32, 4), dtype=self.rdtype, device=dev)
         # tile lists, two buffers (include/astro_b200.h): the current one is astro_bullet_buffer()
         self.bullets = torch.zeros((2, T, 32 * max(K, 1), 4), dtype=self.rdtype, device=dev)
-        # every slot starts finished (empty); meta = nb | np<<10 | finished<<13 | tick<<14
+        # every slot starts finished (empty); meta = nb | np<<10 | finished<<13 | tick<<14 (8 slots: np's bit 3 in bit 31)
         self.meta = torch.full((self.n_pad,), 1 << 13, dtype=torch.int32, device=dev)
         self.episode = torch.zeros((self.n_pad,), dtype=torch.int32, device=dev)
         self._reward = torch.zeros((self.n_pad, S), dtype=torch.float32, device=dev)
@@ -65,6 +82,7 @@ class BatchedGames:
         for name, _ in nat.AstroConfig._fields_[:10]:
             setattr(cfg, name, float(getattr(config, name)))
         cfg.solo = int(bool(config.solo))
+        cfg.planet_slots = self.PL
         handle = C.c_void_p()
         nat.check(L.astro_batch_create(C.byref(cfg), self.n_pad, self.K, precision, self.device.index, C.byref(handle)))
         self._h = handle
@@ -87,7 +105,8 @@ class BatchedGames:
         """A game's tick counter 0 corresponds to (reload0, t0); see schedule.py."""
         if self.schedule is not None and self._origin == (reload0, t0):
             return
-        self.schedule = Schedule(self.config, reload0, t0)
+        self.schedule = Schedule(self.config, reload0, t0,
+                                 max_ticks=nat.MAX_TICKS_WIDE if self.PL == nat.MAX_PLANETS_WIDE else nat.MAX_TICKS)
         self._origin = (reload0, t0)
         s = self.schedule
         nat.check(nat.lib().astro_set_schedule(self._h, s.fire_bits.ctypes.data_as(C.c_void_p), s.n_ticks, s.timeout_tick))
@@ -119,7 +138,7 @@ class BatchedGames:
         torch = _torch()
         dev, f64, i32 = self.device, torch.float64, torch.int32
         t = dict(ships=torch.empty((m, self.S, 5), dtype=f64, device=dev),
-                 planets=torch.empty((m, nat.MAX_PLANETS, 4), dtype=f64, device=dev),
+                 planets=torch.empty((m, self.PL, 4), dtype=f64, device=dev),
                  bullets=torch.empty((m, max(rows, 1), 4), dtype=f64, device=dev),
                  n_planets=torch.empty((m,), dtype=i32, device=dev), n_bullets=torch.empty((m,), dtype=i32, device=dev),
                  tick=torch.empty((m,), dtype=i32, device=dev), finished=torch.empty((m,), dtype=torch.uint8, device=dev),
@@ -141,7 +160,7 @@ class BatchedGames:
 
     def set_arrays(self, ships, planets, n_planets, bullets=None, n_bullets=None, ticks=None, index=None,
                    episode=None, finished=None):
-        """Load games from game-major host arrays: ships [m,S,5] (x,y,dx,dy,b), planets [m,4,4],
+        """Load games from game-major host arrays: ships [m,S,5] (x,y,dx,dy,b), planets [m,PL,4],
         n_planets [m], bullets [m,<=K,4], n_bullets [m], ticks [m] (default 0) — ONE kernel
         (astro_import_games): the touched tiles' bullet lists are rebuilt on the device, every other
         game keeps its state."""
@@ -150,12 +169,14 @@ class BatchedGames:
         ships = np.ascontiguousarray(ships, dtype=np.float64)
         m = ships.shape[0]
         planets = np.ascontiguousarray(planets, dtype=np.float64)
+        if planets.shape[1:] != (self.PL, 4):
+            raise ValueError('planets must be [m, %d, 4] in a batch of %d planet slots' % (self.PL, self.PL))
         n_planets = np.asarray(n_planets, dtype=np.int64)
         n_bullets = np.zeros(m, dtype=np.int64) if n_bullets is None else np.asarray(n_bullets, dtype=np.int64)
         ticks = np.zeros(m, dtype=np.int64) if ticks is None else np.asarray(ticks, dtype=np.int64)
         if n_bullets.max(initial=0) > self.K:
             raise ValueError('a state holds more bullets than bullet_cap=%d' % self.K)
-        if ticks.max(initial=0) > nat.MAX_TICKS:
+        if ticks.max(initial=0) > (nat.MAX_TICKS_WIDE if self.PL == nat.MAX_PLANETS_WIDE else nat.MAX_TICKS):
             raise ValueError('tick counter out of range')
         if m and not (np.abs(ships[:, :, 4]) <= nat.SINCOS_RANGE).all():
             raise ValueError('a bearing lies beyond the +-%d rad over which util.direction is reproduced' % nat.SINCOS_RANGE)
@@ -185,7 +206,7 @@ class BatchedGames:
         lie on this batch's schedule (true for anything produced by create + step)."""
         m, S, K = len(states), self.S, self.K
         ships = np.zeros((m, S, 5))
-        planets = np.zeros((m, nat.MAX_PLANETS, 4))
+        planets = np.zeros((m, self.PL, 4))
         n_planets = np.zeros(m, dtype=np.int64)
         n_bullets = np.zeros(m, dtype=np.int64)
         kmax = max([np.shape(s.bullets.x)[0] for s in states] + [0])
@@ -198,8 +219,9 @@ class BatchedGames:
                 raise ValueError('cannot mix solo and duel games in one batch')
             ships[i, :, 0:2], ships[i, :, 2:4], ships[i, :, 4] = s.ships.x, s.ships.dx, s.ships.b
             p = np.shape(s.planets.x)[0]
-            if not 1 <= p <= nat.MAX_PLANETS:
-                raise ValueError('a state needs 1..%d planets' % nat.MAX_PLANETS)
+            if not 1 <= p <= self.PL:
+                raise ValueError('a state needs 1..%d planets (this batch has %d planet slots; at most %d with planet_slots=%d)'
+                                 % (self.PL, self.PL, nat.MAX_PLANETS_WIDE, nat.MAX_PLANETS_WIDE))
             planets[i, :p, 0:2], planets[i, :p, 2:4] = s.planets.x, s.planets.dx
             n_planets[i] = p
             b = np.shape(s.bullets.x)[0]
@@ -267,7 +289,7 @@ class BatchedGames:
         torch = _torch()
         M, S = len(states), self.S
         ships = np.zeros((M, S, 5), dtype=self.np_rdtype)
-        planets = np.zeros((M, nat.MAX_PLANETS, 4), dtype=self.np_rdtype)
+        planets = np.zeros((M, self.PL, 4), dtype=self.np_rdtype)
         npl = np.zeros(M, dtype=np.int32)
         for i, s in enumerate(states):
             ships[i, :, 0:2], ships[i, :, 2:4], ships[i, :, 4] = s.ships.x, s.ships.dx, s.ships.b
@@ -279,6 +301,8 @@ class BatchedGames:
     def set_reset_pool_arrays(self, ships, planets, n_planets):
         torch = _torch()
         dev = self.device
+        if np.shape(planets)[1:] != (self.PL, 4):
+            raise ValueError('reset pool planets must be [M, %d, 4] in a batch of %d planet slots' % (self.PL, self.PL))
         self._pool = (torch.from_numpy(np.ascontiguousarray(ships, dtype=self.np_rdtype)).to(dev),
                       torch.from_numpy(np.ascontiguousarray(planets, dtype=self.np_rdtype)).to(dev),
                       torch.from_numpy(np.ascontiguousarray(n_planets, dtype=np.int32)).to(dev))
@@ -288,7 +312,7 @@ class BatchedGames:
 
     def create_on_device(self, seeds):
         """`core.create` (core.py:86-135) for every seed, on the device: returns cuda tensors
-        (ships [m,S,5], planets [m,4,4], n_planets int32 [m]) in the batch precision, bit-identical
+        (ships [m,S,5], planets [m,PL,4], n_planets int32 [m]) in the batch precision, bit-identical
         to core.create(config._replace(seed=s)) (rounded to float32 in the float32 build)."""
         torch = _torch()
         seeds = torch.as_tensor(np.asarray(seeds, dtype=np.uint32).astype(np.int64), dtype=torch.int64).to(torch.int32) \
@@ -296,7 +320,7 @@ class BatchedGames:
         seeds = seeds.to(device=self.device, dtype=torch.int32).contiguous()   # same 32 bits as uint32
         m = int(seeds.numel())
         ships = torch.empty((m, self.S, 5), dtype=self.rdtype, device=self.device)
-        planets = torch.empty((m, nat.MAX_PLANETS, 4), dtype=self.rdtype, device=self.device)
+        planets = torch.empty((m, self.PL, 4), dtype=self.rdtype, device=self.device)
         n_planets = torch.empty((m,), dtype=torch.int32, device=self.device)
         c = self.config
         cc = nat.AstroCreateConfig(float(c.inner_ship_position), float(c.outer_ship_position), float(c.planet_orbit),
@@ -516,7 +540,7 @@ class BatchedGames:
                         the ship column groups exchanged (see rl.ValueNetwork.forward_both)."""
         torch = _torch()
         if n_rows is None:
-            n_rows = -(-(nat.MAX_PLANETS + self.K) // 4) * 4
+            n_rows = -(-(self.PL + self.K) // 4) * 4
         shape = (self.n_pad, n_rows, self.D) if shared else (self.n_pad, self.S, n_rows, self.D)
         if out is None:
             out = torch.empty(shape, dtype=torch.float32, device=self.device)

@@ -108,7 +108,7 @@ class _SingleGame:
     (entry 0, 1: nothing fires; 2: the ships fire; 3: the game times out)."""
     PLAIN, FIRE, TIMEOUT = 1, 2, 3
 
-    def __init__(self, config, cap):
+    def __init__(self, config, cap, planet_slots):
         import ctypes as C
         import torch
         from . import _native as nat
@@ -116,12 +116,15 @@ class _SingleGame:
         self.nat, self.C = nat, C
         self.S = 1 if config.solo else 2
         self.cap = cap
-        self.games = BatchedGames(config, nat.TILE, bullet_cap=cap, precision=64)
+        # (the handle's slots follow the state being stepped, not config.max_planets)
+        self.games = BatchedGames(config._replace(max_planets=planet_slots), nat.TILE, bullet_cap=cap, precision=64,
+                                  planet_slots=planet_slots)
         fire = np.array([1 << self.FIRE], dtype=np.uint32)
         nat.check(nat.lib().astro_set_schedule(self.games._h, fire.ctypes.data_as(C.c_void_p), 4, self.TIMEOUT))
         self.games.schedule = None       # (the batch's own reload / t tables do not apply to this handle)
         nbytes = int(nat.lib().astro_single_game_bytes(cap))
         self._pin = [torch.zeros(nbytes, dtype=torch.uint8).pin_memory() for _ in range(2)]
+        pl, wide = nat.AstroSingleGame.planets.offset, nat.MAX_PLANETS_WIDE
         views = []
         for buf in self._pin:
             raw = buf.numpy()
@@ -129,7 +132,7 @@ class _SingleGame:
             head = C.sizeof(nat.AstroSingleGame)
             views.append(dict(rec=rec, ptr=C.c_void_p(buf.data_ptr()),
                               ships=raw[0:80].view(np.float64).reshape(2, 5),
-                              planets=raw[80:208].view(np.float64).reshape(4, 4),
+                              planets=raw[pl:pl + 32 * wide].view(np.float64).reshape(wide, 4),
                               bullets=raw[head:].view(np.float64).reshape(cap, 4)))
         self.inp, self.out = views
 
@@ -150,13 +153,15 @@ class _SingleGame:
         return int(out.events[0]), out.n_bullets, o
 
 
-def _single_game(config, n_bullets):
+def _single_game(config, n_bullets, n_planets):
     nships = 1 if config.solo else 2
     cap = max(32, -(-(n_bullets + nships) // 32) * 32)
-    key = _world_key(config) + (cap,)
+    # a game of <= 4 planets always runs in a 4-slot batch: the layout and kernels it has always run in
+    slots = 4 if n_planets <= 4 else 8
+    key = _world_key(config) + (cap, slots)
     single = _SINGLE.get(key)
     if single is None:
-        single = _SINGLE[key] = _SingleGame(config, cap)
+        single = _SINGLE[key] = _SingleGame(config, cap, slots)
     return single
 
 
@@ -174,15 +179,15 @@ def step(state, control, config):
     if control.shape != (nships,) or control.min() < 0 or control.max() > 5:
         raise ValueError('control must hold %d codes 0..5 (core.py:220-227), got %r' % (nships, control))
     npl = np.shape(state.planets.x)[0]
-    if not 1 <= npl <= 4:
-        raise ValueError('a state needs 1..4 planets')
+    if not 1 <= npl <= 8:
+        raise ValueError('a state needs 1..8 planets, got %d' % npl)
     # reload / t: Python floats, the reference's operations (core.py:257, 263, 267, 280, 302)
     timeout = config.max_time <= state.t + config.dt
     next_reload = state.reload + config.dt
     fire = config.reload_time <= next_reload
     if fire:
         next_reload -= config.reload_time
-    single = _single_game(config, np.shape(state.bullets.x)[0])
+    single = _single_game(config, np.shape(state.bullets.x)[0], npl)
     code = _SingleGame.TIMEOUT if timeout else (_SingleGame.FIRE if fire else _SingleGame.PLAIN)
     # A state straight from create() holds float32 arrays: the reference's first tick then runs partly in float32
     # (NEP 50 promotion) — reproduced by the kernel's ASTRO_TICK_ALL_CREATE_DTYPES arithmetic.

@@ -80,14 +80,14 @@ struct TickParams {
 // entry pick(seed, global game id, key) with key = 1 + the stream step of the tick that ended the
 // game (0 for the initial fill) — no dependent load on the way; bullets cleared, tick 0.  The
 // per-slot episode counter is bumped with a fire-and-forget RED.
-template <typename R, int S>
+template <typename R, int S, int PL>
 __device__ __forceinline__ void recreate_from_pool(const TickParams& p, int g, uint32_t key, Body4<R>* ships,
                                                    R* ship_b, Body4<R>* planets) {
     using B4 = Body4<R>;
     atomicAdd(&p.episode[g], 1u);
     uint32_t k = pool_pick(p.seed, p.first_game + (uint32_t)g, key, (uint32_t)p.pool_size);
     const R* ps = reinterpret_cast<const R*>(p.pool_ships) + (size_t)k * (S * 5);
-    const R* pp = reinterpret_cast<const R*>(p.pool_planets) + (size_t)k * (ASTRO_MAX_PLANETS * 4);
+    const R* pp = reinterpret_cast<const R*>(p.pool_planets) + (size_t)k * (PL * 4);
     int np_new = p.pool_np[k];
 #pragma unroll
     for (int s = 0; s < S; s++) {
@@ -97,29 +97,32 @@ __device__ __forceinline__ void recreate_from_pool(const TickParams& p, int g, u
         ship_b[s * 32] = ps[5 * s + 4];
     }
 #pragma unroll
-    for (int j = 0; j < ASTRO_MAX_PLANETS; j++) {
+    for (int j = 0; j < PL; j++) {
         if (j < np_new) {
             B4 o;
             o.x = pp[4 * j]; o.y = pp[4 * j + 1]; o.dx = pp[4 * j + 2]; o.dy = pp[4 * j + 3];
             planets[j * 32] = o;
         }
     }
-    p.meta[g] = ASTRO_META_PACK(0, np_new, 0, 0);
+    p.meta[g] = meta_pack<PL>(0, np_new, 0, 0);
 }
 
 // The reset pool as one 128-byte record per entry, so that re-creating a game inside the tick is ONE
 // round trip (the three pool arrays need the planet count first): floats 0 .. 5S-1 = ships
-// (x, y, dx, dy, b each), word 10 = planet count, floats 16 .. 31 = planets.
-template <int S>
+// (x, y, dx, dy, b each), word 10 = planet count, floats 16 .. 31 = planets.  8-slot batches: 256-byte
+// records, planets in floats 16 .. 47.
+template <int PL>
+__host__ __device__ constexpr int pool_rec_float4s() { return PL > ASTRO_MAX_PLANETS ? 16 : 8; }
+template <int S, int PL>
 __global__ void pack_pool_kernel(const float* __restrict__ ships, const float* __restrict__ planets,
                                  const int32_t* __restrict__ np, float* __restrict__ rec, int m) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= m) return;
-    float* r = rec + (size_t)k * 32;
-    for (int i = 0; i < 32; i++) r[i] = 0.f;
+    float* r = rec + (size_t)k * (4 * pool_rec_float4s<PL>());
+    for (int i = 0; i < 4 * pool_rec_float4s<PL>(); i++) r[i] = 0.f;
     for (int i = 0; i < 5 * S; i++) r[i] = ships[(size_t)k * (5 * S) + i];
     r[10] = __int_as_float(np[k]);
-    for (int i = 0; i < 16; i++) r[16 + i] = planets[(size_t)k * 16 + i];
+    for (int i = 0; i < 4 * PL; i++) r[16 + i] = planets[(size_t)k * (4 * PL) + i];
 }
 
 // Warp-level reduction of the per-game flags and counts into the block's shared counters:
@@ -273,7 +276,7 @@ __device__ __forceinline__ unsigned warp_exclusive_sum(unsigned v, int lane) {
 // game ends it owns no bullets (nb = 0); ships/planets keep the pre-step state unless AUTO_RESET
 // re-initialises the slot from the pool.
 // ------------------------------------------------------------------------------------------
-template <typename R, int S, bool STATS>
+template <typename R, int S, bool STATS, int PL>
 __global__ void __launch_bounds__(kTickThreads) tick_kernel(const __grid_constant__ TickParams p) {
     using B4 = Body4<R>;
     __shared__ unsigned s_stats[ASTRO_N_STATS];
@@ -295,7 +298,7 @@ __global__ void __launch_bounds__(kTickThreads) tick_kernel(const __grid_constan
         const size_t tile = (size_t)(g >> 5);
         B4* ships = reinterpret_cast<B4*>(p.ships) + tile * (S * 32) + lane;
         R* ship_b = reinterpret_cast<R*>(p.ship_b) + tile * (S * 32) + lane;
-        B4* planets = reinterpret_cast<B4*>(p.planets) + tile * (ASTRO_MAX_PLANETS * 32) + lane;
+        B4* planets = reinterpret_cast<B4*>(p.planets) + tile * (PL * 32) + lane;
 
         const uint32_t meta = p.meta[g];
         // ships are loaded before meta is inspected: independent loads, one DRAM round trip
@@ -308,8 +311,8 @@ __global__ void __launch_bounds__(kTickThreads) tick_kernel(const __grid_constan
         }
         active = !ASTRO_META_FINISHED(meta);
         nb = active ? (int)ASTRO_META_NB(meta) : 0;
-        np = active ? (int)ASTRO_META_NP(meta) : 0;
-        const uint32_t tick = ASTRO_META_TICK(meta);
+        np = active ? (int)meta_np<PL>(meta) : 0;
+        const uint32_t tick = meta_tick<PL>(meta);
         // this game's run of the tile's list (read buffer); survivors are compacted inside it
         B4* const bullets = reinterpret_cast<B4*>(p.bullets_in) + tile * (size_t)(32 * p.K) + warp_exclusive_sum((unsigned)nb, lane);
         int m = 0, n_born = 0;
@@ -322,9 +325,9 @@ __global__ void __launch_bounds__(kTickThreads) tick_kernel(const __grid_constan
         if (!active) {
             ev = ASTRO_EV_SKIPPED;
         } else {
-            B4 pl[ASTRO_MAX_PLANETS];
+            B4 pl[PL];
 #pragma unroll
-            for (int j = 0; j < ASTRO_MAX_PLANETS; j++)
+            for (int j = 0; j < PL; j++)
                 if (j < np) pl[j] = planets[j * 32];
 
             // first group of bullets in flight while the ship/planet maths runs
@@ -372,7 +375,7 @@ __global__ void __launch_bounds__(kTickThreads) tick_kernel(const __grid_constan
                 if (raw) {
                     float f0 = 0.f, f1 = 0.f;
 #pragma unroll
-                    for (int j = 0; j < ASTRO_MAX_PLANETS; j++) {
+                    for (int j = 0; j < PL; j++) {
                         if (j < np) {
                             float t0, t1;
                             grav_term_np32((float)pl[j].x, (float)pl[j].y, (float)sh[s].x, (float)sh[s].y, c.gm_f, t0, t1);
@@ -383,7 +386,7 @@ __global__ void __launch_bounds__(kTickThreads) tick_kernel(const __grid_constan
                     g0 = (R)f0; g1 = (R)f1;
                 } else {
 #pragma unroll
-                for (int j = 0; j < ASTRO_MAX_PLANETS; j++) {
+                for (int j = 0; j < PL; j++) {
                     if (j < np) {
                         R t0, t1;
                         grav_term(pl[j].x, pl[j].y, sh[s].x, sh[s].y, c, t0, t1);
@@ -424,7 +427,7 @@ __global__ void __launch_bounds__(kTickThreads) tick_kernel(const __grid_constan
                             gone |= h;
                         }
 #pragma unroll
-                        for (int k = 0; k < ASTRO_MAX_PLANETS; k++)
+                        for (int k = 0; k < PL; k++)
                             if (k < np) gone |= collide(pl[k].x, pl[k].y, b.x, b.y, c.r2_pb, c.r2f_pb);
                         bool keep = advance_bullet(b, c);
                         if (keep && !gone) {
@@ -491,13 +494,13 @@ __global__ void __launch_bounds__(kTickThreads) tick_kernel(const __grid_constan
                 }
                 // ---- planets (core.py:289-294): gravity of every planet on every planet, the
                 // clamped self term included (f * 0 = 0)
-                R q0[ASTRO_MAX_PLANETS], q1[ASTRO_MAX_PLANETS];
+                R q0[PL], q1[PL];
 #pragma unroll
-                for (int i = 0; i < ASTRO_MAX_PLANETS; i++) {
+                for (int i = 0; i < PL; i++) {
                     q0[i] = 0; q1[i] = 0;
                     if (i < np) {
 #pragma unroll
-                        for (int j = 0; j < ASTRO_MAX_PLANETS; j++) {
+                        for (int j = 0; j < PL; j++) {
                             if (j < np) {
                                 R t0, t1;
                                 grav_term(pl[j].x, pl[j].y, pl[i].x, pl[i].y, c, t0, t1);
@@ -507,13 +510,13 @@ __global__ void __launch_bounds__(kTickThreads) tick_kernel(const __grid_constan
                     }
                 }
                 if (raw) {   // float32 field, float32 a * dt (a float32 array times the weak scalar dt), then float64
-                    float f0[ASTRO_MAX_PLANETS], f1[ASTRO_MAX_PLANETS];
+                    float f0[PL], f1[PL];
 #pragma unroll
-                    for (int i = 0; i < ASTRO_MAX_PLANETS; i++) {
+                    for (int i = 0; i < PL; i++) {
                         f0[i] = f1[i] = 0.f;
                         if (i < np) {
 #pragma unroll
-                            for (int j = 0; j < ASTRO_MAX_PLANETS; j++) {
+                            for (int j = 0; j < PL; j++) {
                                 if (j < np) {
                                     float t0, t1;
                                     grav_term_np32((float)pl[j].x, (float)pl[j].y, (float)pl[i].x, (float)pl[i].y, c.gm_f, t0, t1);
@@ -523,7 +526,7 @@ __global__ void __launch_bounds__(kTickThreads) tick_kernel(const __grid_constan
                         }
                     }
 #pragma unroll
-                    for (int i = 0; i < ASTRO_MAX_PLANETS; i++) {
+                    for (int i = 0; i < PL; i++) {
                         if (i < np) {
                             const double v0 = __dadd_rn((double)pl[i].dx, (double)__fmul_rn(f0[i], c.dt_f));
                             const double v1 = __dadd_rn((double)pl[i].dy, (double)__fmul_rn(f1[i], c.dt_f));
@@ -535,7 +538,7 @@ __global__ void __launch_bounds__(kTickThreads) tick_kernel(const __grid_constan
                     }
                 } else {
 #pragma unroll
-                for (int i = 0; i < ASTRO_MAX_PLANETS; i++) {
+                for (int i = 0; i < PL; i++) {
                     if (i < np) {
                         advance_body(pl[i], q0[i], q1[i], c);
                         planets[i * 32] = pl[i];
@@ -551,15 +554,15 @@ __global__ void __launch_bounds__(kTickThreads) tick_kernel(const __grid_constan
                     ship_b[s * 32] = add_rn(sb[s], db);
                 }
                 m_out = m + n_born;
-                p.meta[g] = ASTRO_META_PACK(m_out, np, 0, tick + 1);
+                p.meta[g] = meta_pack<PL>(m_out, np, 0, tick + 1);
             }
 
             if (bad_ctl) ev |= ASTRO_EV_BAD_CONTROL;
             if (ev & ASTRO_EV_DONE_MASK) {
                 if ((p.flags & ASTRO_TICK_AUTO_RESET) && p.pool_size > 0) {
-                    recreate_from_pool<R, S>(p, g, p.step + (p.step_base ? *p.step_base : 0u) + 1u, ships, ship_b, planets);
+                    recreate_from_pool<R, S, PL>(p, g, p.step + (p.step_base ? *p.step_base : 0u) + 1u, ships, ship_b, planets);
                 } else {
-                    p.meta[g] = ASTRO_META_PACK(0, np, 1, tick);
+                    p.meta[g] = meta_pack<PL>(0, np, 1, tick);
                 }
             }
         }
@@ -601,7 +604,7 @@ __global__ void __launch_bounds__(kTickThreads) tick_kernel(const __grid_constan
 // ------------------------------------------------------------------------------------------
 // reset_kernel: stand-alone form of AUTO_RESET — finished games are re-created from the pool.
 // ------------------------------------------------------------------------------------------
-template <typename R, int S>
+template <typename R, int S, int PL>
 __global__ void __launch_bounds__(kTickThreads) reset_kernel(const __grid_constant__ TickParams p) {
     using B4 = Body4<R>;
     const int g = blockIdx.x * kTickThreads + threadIdx.x;
@@ -612,8 +615,8 @@ __global__ void __launch_bounds__(kTickThreads) reset_kernel(const __grid_consta
     const int lane = g & 31;
     B4* ships = reinterpret_cast<B4*>(p.ships) + tile * (S * 32) + lane;
     R* ship_b = reinterpret_cast<R*>(p.ship_b) + tile * (S * 32) + lane;
-    B4* planets = reinterpret_cast<B4*>(p.planets) + tile * (ASTRO_MAX_PLANETS * 32) + lane;
-    recreate_from_pool<R, S>(p, g, p.step, ships, ship_b, planets);
+    B4* planets = reinterpret_cast<B4*>(p.planets) + tile * (PL * 32) + lane;
+    recreate_from_pool<R, S, PL>(p, g, p.step, ships, ship_b, planets);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -630,7 +633,7 @@ __host__ __device__ inline size_t observe_warp_floats(int n_rows, int D, int S, 
     return (((size_t)P * n_rows * D + 5 * S) + 3) & ~(size_t)3;
 }
 
-template <typename R, int S, bool BOTH>
+template <typename R, int S, bool BOTH, int PL>
 __global__ void __launch_bounds__(kObserveWarps * 32)
 observe_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_, const void* __restrict__ planets_,
                const void* __restrict__ bullets_, const uint32_t* __restrict__ meta_, float* __restrict__ obs,
@@ -651,7 +654,7 @@ observe_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_
     const int gl = g & 31;
     const uint32_t meta = meta_[g];
     const bool fin = ASTRO_META_FINISHED(meta);
-    const int np = fin ? 0 : (int)ASTRO_META_NP(meta);
+    const int np = fin ? 0 : (int)meta_np<PL>(meta);
     const int nb = fin ? 0 : (int)ASTRO_META_NB(meta);
 
     if (lane < S && !fin) {
@@ -664,7 +667,7 @@ observe_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_
         sf[5 * lane + 4] = norm_angle_over_pi((double)b);
     }
     __syncwarp();
-    const B4* planets = reinterpret_cast<const B4*>(planets_) + tile * (ASTRO_MAX_PLANETS * 32) + gl;
+    const B4* planets = reinterpret_cast<const B4*>(planets_) + tile * (PL * 32) + gl;
     // the game's run of its tile's bullet list
     const B4* bullets = reinterpret_cast<const B4*>(bullets_) + tile * (size_t)(32 * K) + tile_list_offset(meta_ + tile * 32, gl, lane);
     for (int r = lane; r < n_rows; r += 32) {
@@ -724,8 +727,11 @@ observe_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_
 #ifndef ASTRO_SCRIPT_MIN_BLOCKS
 #define ASTRO_SCRIPT_MIN_BLOCKS 6   /* 80 registers: 41.1 -> 32.9 us per 262,144 games (the kernel waits on its loads: more warps) */
 #endif
-template <typename R, int S>
-__global__ void __launch_bounds__(128, ASTRO_SCRIPT_MIN_BLOCKS) script_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_,
+#ifndef ASTRO_SCRIPT_MIN_BLOCKS_WIDE
+#define ASTRO_SCRIPT_MIN_BLOCKS_WIDE 2   /* 8 planet slots: five float64 candidates per planet stay in registers */
+#endif
+template <typename R, int S, int PL>
+__global__ void __launch_bounds__(128, PL > ASTRO_MAX_PLANETS ? ASTRO_SCRIPT_MIN_BLOCKS_WIDE : ASTRO_SCRIPT_MIN_BLOCKS) script_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_,
                                                      const void* __restrict__ planets_, const uint32_t* __restrict__ meta_,
                                                      uint8_t* __restrict__ actions, const __grid_constant__ ScriptParams q) {
     using B4 = Body4<R>;
@@ -739,18 +745,18 @@ __global__ void __launch_bounds__(128, ASTRO_SCRIPT_MIN_BLOCKS) script_kernel(co
         actions[idx] = 2;
         return;
     }
-    const int np = (int)ASTRO_META_NP(meta);
+    const int np = (int)meta_np<PL>(meta);
     const B4 mv = reinterpret_cast<const B4*>(ships_)[tile * (S * 32) + me * 32 + lane];
     const R mb = reinterpret_cast<const R*>(ship_b_)[tile * (S * 32) + me * 32 + lane];
-    B4 pl[ASTRO_MAX_PLANETS];
+    B4 pl[PL];
 #pragma unroll
-    for (int j = 0; j < ASTRO_MAX_PLANETS; j++) {
+    for (int j = 0; j < PL; j++) {
         pl[j] = B4();
-        if (j < np) pl[j] = reinterpret_cast<const B4*>(planets_)[tile * (ASTRO_MAX_PLANETS * 32) + j * 32 + lane];
+        if (j < np) pl[j] = reinterpret_cast<const B4*>(planets_)[tile * (PL * 32) + j * 32 + lane];
     }
     B4 ev = B4();
     if (S == 2 && !q.solo) ev = reinterpret_cast<const B4*>(ships_)[tile * (S * 32) + ((me + 1) % S) * 32 + lane];
-    actions[idx] = (uint8_t)script_decide<R, S>(mv, mb, ev, pl, np, q);
+    actions[idx] = (uint8_t)script_decide<R, S, PL>(mv, mb, ev, pl, np, q);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -824,14 +830,16 @@ struct Mt19937Head {
 
 // One created game in registers: float32 ship positions / bearings and planet positions, float64 planet velocities
 // (the reference's dtypes under numpy >= 2).
-struct CreatedGame {
+template <int PL>
+struct CreatedGameT {
     float sx[2][2], sb[2];
-    float px[ASTRO_MAX_PLANETS][2];
-    double pv[ASTRO_MAX_PLANETS][2];
+    float px[PL][2];
+    double pv[PL][2];
     int n;
 };
-template <int S>
-__device__ __forceinline__ void create_game(uint32_t seed, const CreateParams& q, CreatedGame& o) {
+using CreatedGame = CreatedGameT<ASTRO_MAX_PLANETS>;
+template <int S, int PL = ASTRO_MAX_PLANETS>
+__device__ __forceinline__ void create_game(uint32_t seed, const CreateParams& q, CreatedGameT<PL>& o) {
     const double TWO_PI = 6.283185307179586, PI = 3.141592653589793;
     Mt19937Head mt;
     mt.seed(seed);
@@ -863,7 +871,7 @@ __device__ __forceinline__ void create_game(uint32_t seed, const CreateParams& q
     for (int s = 0; s < S; s++) o.sb[s] = __fmul_rn(two_pi_f, (float)mt.rand());
     // 2. planets
 #pragma unroll
-    for (int j = 0; j < ASTRO_MAX_PLANETS; j++) { o.px[j][0] = o.px[j][1] = 0.f; o.pv[j][0] = o.pv[j][1] = 0.0; }
+    for (int j = 0; j < PL; j++) { o.px[j][0] = o.px[j][1] = 0.f; o.pv[j][0] = o.pv[j][1] = 0.0; }
     if (n > 1) {
         const double base = __dmul_rn(TWO_PI, mt.rand());
         const double step = __ddiv_rn(TWO_PI, (double)n);                    // np.linspace(0, 2 pi, n, endpoint=False)
@@ -872,7 +880,7 @@ __device__ __forceinline__ void create_game(uint32_t seed, const CreateParams& q
         const double speed = sqrt(__ddiv_rn(__dmul_rn(__dmul_rn(q.gravity, q.planet_mass), (double)(n - 1)), 2.0));
         const float orbit_f = (float)q.orbit;
 #pragma unroll
-        for (int j = 0; j < ASTRO_MAX_PLANETS; j++) {
+        for (int j = 0; j < PL; j++) {
             if (j < n) {
                 const double phase = __dadd_rn(base, __dadd_rn(__dmul_rn((double)j, step), 0.0));
                 float s0, c0, s1, c1;
@@ -888,23 +896,23 @@ __device__ __forceinline__ void create_game(uint32_t seed, const CreateParams& q
     o.n = n;
 }
 
-template <typename R, int S>
+template <typename R, int S, int PL>
 __global__ void __launch_bounds__(64) create_kernel(const uint32_t* __restrict__ seeds, R* __restrict__ ships,
                                                     R* __restrict__ planets, int32_t* __restrict__ np_out,
                                                     const __grid_constant__ CreateParams q) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= q.m) return;
-    CreatedGame o;
-    create_game<S>(seeds[i], q, o);
+    CreatedGameT<PL> o;
+    create_game<S, PL>(seeds[i], q, o);
 #pragma unroll
     for (int s = 0; s < S; s++) {
         R* d = ships + ((size_t)i * S + s) * 5;
         d[0] = (R)o.sx[s][0]; d[1] = (R)o.sx[s][1]; d[2] = (R)0; d[3] = (R)0;
         d[4] = (R)o.sb[s];
     }
-    R* pl = planets + (size_t)i * (ASTRO_MAX_PLANETS * 4);
+    R* pl = planets + (size_t)i * (PL * 4);
 #pragma unroll
-    for (int j = 0; j < ASTRO_MAX_PLANETS; j++) {
+    for (int j = 0; j < PL; j++) {
         pl[4 * j + 0] = (R)o.px[j][0];
         pl[4 * j + 1] = (R)o.px[j][1];
         pl[4 * j + 2] = (R)o.pv[j][0];
@@ -1149,7 +1157,7 @@ __device__ __forceinline__ void layer2_t(const float* __restrict__ wt, int strid
 #ifndef ASTRO_POL_MIN_BLOCKS
 #define ASTRO_POL_MIN_BLOCKS 4
 #endif
-template <typename R, int S>
+template <typename R, int S, int PL>
 __global__ void __launch_bounds__(kPolWarps * 32, ASTRO_POL_MIN_BLOCKS)
 policy_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_, const void* __restrict__ planets_,
               const void* __restrict__ bullets_, const uint32_t* __restrict__ meta_, uint8_t* __restrict__ actions,
@@ -1179,7 +1187,7 @@ policy_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_,
 
     const uint32_t meta = meta_[g];
     const bool fin = ASTRO_META_FINISHED(meta);
-    const int np = fin ? 0 : (int)ASTRO_META_NP(meta);
+    const int np = fin ? 0 : (int)meta_np<PL>(meta);
     const int rows = fin ? 0 : np + (int)ASTRO_META_NB(meta);
     // ship features (x, y, dx, dy, norm_angle(b) / pi), ship 0 then ship 1: lane 5 s + c holds feature c of ship s
     float feat = 0.f;
@@ -1198,7 +1206,7 @@ policy_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_,
             baseA = __fmaf_rn(w0[1 + 5 * s + c], f, baseA);
             baseB = __fmaf_rn(w0[1 + 5 * ((s + 1) % S) + c], f, baseB);
         }
-    const B4* pl = reinterpret_cast<const B4*>(planets_) + tile * (ASTRO_MAX_PLANETS * 32) + gl;
+    const B4* pl = reinterpret_cast<const B4*>(planets_) + tile * (PL * 32) + gl;
     const B4* bl = reinterpret_cast<const B4*>(bullets_) + tile * (size_t)(32 * K) + tile_list_offset(meta_ + tile * 32, gl, lane);
     // lane r fetches row r's object (coalesced for the bullets); rows beyond 32 are fetched in a second batch
     float bestA = -3.0e38f, bestB = -3.0e38f;
@@ -1417,7 +1425,7 @@ __device__ __forceinline__ void init_bias(float (&acc)[NT][4], const float2 (*bi
 #ifndef ASTRO_MMA_MIN_BLOCKS
 #define ASTRO_MMA_MIN_BLOCKS 4
 #endif
-template <typename R, int S>
+template <typename R, int S, int PL>
 __global__ void __launch_bounds__(kMmaWarps * 32, ASTRO_MMA_MIN_BLOCKS)
 policy_mma_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_, const void* __restrict__ planets_,
                   const void* __restrict__ bullets_, const uint32_t* __restrict__ meta_, uint8_t* __restrict__ actions,
@@ -1466,7 +1474,7 @@ policy_mma_kernel(const void* __restrict__ ships_, const void* __restrict__ ship
             if (lane >= d) incl += v;
         }
         const unsigned off_l = incl - nb_l;                                  // first list item of lane's game (tile_list_offset)
-        const int np_l = fin_l ? 0 : (int)ASTRO_META_NP(meta_l);
+        const int np_l = fin_l ? 0 : (int)meta_np<PL>(meta_l);
         const int rows_l = fin_l ? 0 : np_l + (int)nb_l;
         const unsigned live_mask = (__ballot_sync(0xffffffffu, rows_l > 0) >> gl0) & 0xffu;
         // ship features (x, y, dx, dy, norm_angle(b) / pi), ship 0 then ship 1, of the 8 games: the float64 bearings by
@@ -1481,7 +1489,7 @@ policy_mma_kernel(const void* __restrict__ ships_, const void* __restrict__ ship
             s_all.sf[warp][j8][5 * s_ + c] = (float)reinterpret_cast<const R*>(ships_)[(tile * (S * 32) + s_ * 32 + gl0 + j8) * 4 + c];
         }
         __syncwarp();
-        const Body4<R>* const pl_tile = reinterpret_cast<const Body4<R>*>(planets_) + tile * (ASTRO_MAX_PLANETS * 32);
+        const Body4<R>* const pl_tile = reinterpret_cast<const Body4<R>*>(planets_) + tile * (PL * 32);
         const Body4<R>* const bl_tile = reinterpret_cast<const Body4<R>*>(bullets_) + tile * (size_t)(32 * K);
         // this lane's object component(s) of row gq of a game's first 8 rows (the quad covers the object's 16 bytes)
         auto load_first_rows = [&](int j8, float (&ov)[4]) {
@@ -1832,7 +1840,7 @@ value_forward_kernel(const float* __restrict__ features, float* __restrict__ q_o
 __device__ __forceinline__ uint32_t explore_key(uint32_t seed, uint32_t game, uint32_t step, uint32_t ship) {
     return mix32(mix32(seed ^ 0x3C6EF372u ^ (game * 0x9E3779B1u)) ^ (step * 2u + ship));
 }
-template <int S>
+template <int S, int PL>
 __global__ void __launch_bounds__(128) explore_kernel(const uint32_t* __restrict__ meta_, int32_t* __restrict__ state,
                                                       uint8_t* __restrict__ actions, int n_games, int ship_mask, double dt,
                                                       double t_in, double t_out, uint32_t seed, uint32_t first_game, uint32_t step,
@@ -1843,7 +1851,7 @@ __global__ void __launch_bounds__(128) explore_kernel(const uint32_t* __restrict
     if (g >= n_games || !((ship_mask >> me) & 1)) return;
     const uint32_t meta = meta_[g];
     if (ASTRO_META_FINISHED(meta)) return;
-    const int tick = (int)ASTRO_META_TICK(meta);
+    const int tick = (int)meta_tick<PL>(meta);
     const int32_t st = state[idx];
     int policy = (st & 0xff) - 1;                     // -1 = idle
     const double gap = __dmul_rn(dt, (double)(tick - (st >> 8)));
@@ -1883,7 +1891,7 @@ struct GameArrays {          // device pointers, see AstroGameArrays
     uint32_t* episode;
 };
 
-template <typename R, int S>
+template <typename R, int S, int PL>
 __global__ void __launch_bounds__(128) export_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_,
                                                      const void* __restrict__ planets_, const void* __restrict__ bullets_,
                                                      const uint32_t* __restrict__ meta_, const uint32_t* __restrict__ episode_,
@@ -1898,17 +1906,17 @@ __global__ void __launch_bounds__(128) export_kernel(const void* __restrict__ sh
     const int gl = g & 31;
     const uint32_t meta = meta_[g];
     const bool fin = ASTRO_META_FINISHED(meta);
-    const int np = (int)ASTRO_META_NP(meta), nb = fin ? 0 : (int)ASTRO_META_NB(meta);
+    const int np = (int)meta_np<PL>(meta), nb = fin ? 0 : (int)ASTRO_META_NB(meta);
     if (lane < S) {
         const B4 v = reinterpret_cast<const B4*>(ships_)[tile * (S * 32) + lane * 32 + gl];
         double* o = a.ships + ((size_t)row * S + lane) * 5;
         o[0] = (double)v.x; o[1] = (double)v.y; o[2] = (double)v.dx; o[3] = (double)v.dy;
         o[4] = (double)reinterpret_cast<const R*>(ship_b_)[tile * (S * 32) + lane * 32 + gl];
     }
-    if (lane < ASTRO_MAX_PLANETS) {
+    if (lane < PL) {
         B4 v = B4();
-        if (lane < np) v = reinterpret_cast<const B4*>(planets_)[tile * (ASTRO_MAX_PLANETS * 32) + lane * 32 + gl];
-        double* o = a.planets + ((size_t)row * ASTRO_MAX_PLANETS + lane) * 4;
+        if (lane < np) v = reinterpret_cast<const B4*>(planets_)[tile * (PL * 32) + lane * 32 + gl];
+        double* o = a.planets + ((size_t)row * PL + lane) * 4;
         o[0] = (double)v.x; o[1] = (double)v.y; o[2] = (double)v.dx; o[3] = (double)v.dy;
     }
     const unsigned first = tile_list_offset(meta_ + tile * 32, gl, lane);
@@ -1922,7 +1930,7 @@ __global__ void __launch_bounds__(128) export_kernel(const void* __restrict__ sh
     if (lane == 0) {
         a.n_planets[row] = np;
         a.n_bullets[row] = nb;
-        a.tick[row] = (int32_t)ASTRO_META_TICK(meta);
+        a.tick[row] = (int32_t)meta_tick<PL>(meta);
         a.finished[row] = fin ? 1 : 0;
         if (a.episode) a.episode[row] = episode_[g];
     }
@@ -1935,7 +1943,7 @@ __global__ void import_map_kernel(const int32_t* __restrict__ index, int m, int 
     if (g >= 0 && g < n_games) src[g] = i;
 }
 
-template <typename R, int S>
+template <typename R, int S, int PL>
 __global__ void __launch_bounds__(128) import_kernel(void* __restrict__ ships_, void* __restrict__ ship_b_, void* __restrict__ planets_,
                                                      void* bullets_cur_, void* bullets_other_, uint32_t* __restrict__ meta_,
                                                      uint32_t* __restrict__ episode_, const int32_t* __restrict__ src, int m,
@@ -1974,7 +1982,7 @@ __global__ void __launch_bounds__(128) import_kernel(void* __restrict__ ships_, 
     __syncwarp();
     for (unsigned j = lane; j < new_total; j += 32u) cur[j] = scratch[j];
     if (row >= 0) {
-        const int np = min(max(a.n_planets[row], 0), ASTRO_MAX_PLANETS);
+        const int np = min(max(a.n_planets[row], 0), PL);
 #pragma unroll
         for (int s = 0; s < S; s++) {
             const double* o = a.ships + ((size_t)row * S + s) * 5;
@@ -1984,14 +1992,14 @@ __global__ void __launch_bounds__(128) import_kernel(void* __restrict__ ships_, 
             reinterpret_cast<R*>(ship_b_)[tile * (S * 32) + s * 32 + lane] = (R)o[4];
         }
 #pragma unroll
-        for (int j = 0; j < ASTRO_MAX_PLANETS; j++) {
-            const double* o = a.planets + ((size_t)row * ASTRO_MAX_PLANETS + j) * 4;
+        for (int j = 0; j < PL; j++) {
+            const double* o = a.planets + ((size_t)row * PL + j) * 4;
             B4 v = B4();
             if (j < np) { v.x = (R)o[0]; v.y = (R)o[1]; v.dx = (R)o[2]; v.dy = (R)o[3]; }
-            reinterpret_cast<B4*>(planets_)[tile * (ASTRO_MAX_PLANETS * 32) + j * 32 + lane] = v;
+            reinterpret_cast<B4*>(planets_)[tile * (PL * 32) + j * 32 + lane] = v;
         }
         const uint32_t tick = a.tick ? (uint32_t)a.tick[row] : 0u;
-        meta_[g] = ASTRO_META_PACK(new_nb, np, fin ? 1 : 0, tick);
+        meta_[g] = meta_pack<PL>(new_nb, np, fin ? 1 : 0, tick);
         if (a.episode) episode_[g] = a.episode[row];
     }
 }
@@ -2152,6 +2160,7 @@ constexpr int kSingleGraphs = 4;
 struct AstroBatch {
     AstroConfig cfg;
     int32_t n_games, K, precision, device, S;
+    int32_t PL;              // planet slots per game: ASTRO_MAX_PLANETS or ASTRO_MAX_PLANETS_WIDE (AstroConfig.planet_slots)
     bool bound;
     AstroBuffers bufs;
     AstroResetPool pool;
@@ -2289,13 +2298,13 @@ void fill_params(const AstroBatch* b, TickParams& p) {
     p.c = b->c;
 }
 
-template <typename R, int S>
+template <typename R, int S, int PL>
 cudaError_t launch_tick(const TickParams& p, cudaStream_t st) {
     const int grid = (p.n_games + kTickThreads - 1) / kTickThreads;
     if (p.flags & ASTRO_TICK_NO_STATS)
-        tick_kernel<R, S, false><<<grid, kTickThreads, 0, st>>>(p);
+        tick_kernel<R, S, false, PL><<<grid, kTickThreads, 0, st>>>(p);
     else
-        tick_kernel<R, S, true><<<grid, kTickThreads, 0, st>>>(p);
+        tick_kernel<R, S, true, PL><<<grid, kTickThreads, 0, st>>>(p);
     return cudaGetLastError();
 }
 
@@ -2347,6 +2356,21 @@ cudaError_t launch_tick_f32(const TickParams& p, cudaStream_t st) {
         } else if (p.flags & ASTRO_TICK_NO_STATS) tick_f32_kernel<S, false, false><<<grid, kTickThreads, extra, st>>>(p);
         else tick_f32_kernel<S, true, false><<<grid, kTickThreads, extra, st>>>(p);
 #endif
+    }
+    return cudaGetLastError();
+}
+
+// 8 planet slots: the generic instantiations, one tick or several per launch.  The FIX and BOT forms exist for 4 slots only
+// (astro_rollout_device runs ScriptBots of 8-slot batches as bot kernel -> tick kernel).
+template <int S>
+cudaError_t launch_tick_f32_wide(const TickParams& p, cudaStream_t st) {
+    const int grid = (p.tiles * 32 + kTickThreads - 1) / kTickThreads;
+    if (p.n_fused > 1) {
+        if (p.flags & ASTRO_TICK_NO_STATS) tick_f32_wide_kernel<S, false, true><<<grid, kTickThreads, 0, st>>>(p);
+        else tick_f32_wide_kernel<S, true, true><<<grid, kTickThreads, 0, st>>>(p);
+    } else {
+        if (p.flags & ASTRO_TICK_NO_STATS) tick_f32_wide_kernel<S, false, false><<<grid, kTickThreads, 0, st>>>(p);
+        else tick_f32_wide_kernel<S, true, false><<<grid, kTickThreads, 0, st>>>(p);
     }
     return cudaGetLastError();
 }
@@ -2478,12 +2502,20 @@ int do_ticks(AstroBatch* b, const uint8_t* actions, float* reward, uint8_t* done
             p.script = b->script_now;
         }
         cudaError_t e;
-        if (fused)
+        if (b->PL == ASTRO_MAX_PLANETS_WIDE) {
+            constexpr int PL = ASTRO_MAX_PLANETS_WIDE;
+            if (fused)
+                e = b->S == 2 ? launch_tick_f32_wide<2>(p, st) : launch_tick_f32_wide<1>(p, st);
+            else if (b->precision == 32)
+                e = b->S == 2 ? launch_tick<float, 2, PL>(p, st) : launch_tick<float, 1, PL>(p, st);
+            else
+                e = b->S == 2 ? launch_tick<double, 2, PL>(p, st) : launch_tick<double, 1, PL>(p, st);
+        } else if (fused)
             e = b->S == 2 ? launch_tick_f32<2>(p, st) : launch_tick_f32<1>(p, st);
         else if (b->precision == 32)
-            e = b->S == 2 ? launch_tick<float, 2>(p, st) : launch_tick<float, 1>(p, st);
+            e = b->S == 2 ? launch_tick<float, 2, ASTRO_MAX_PLANETS>(p, st) : launch_tick<float, 1, ASTRO_MAX_PLANETS>(p, st);
         else
-            e = b->S == 2 ? launch_tick<double, 2>(p, st) : launch_tick<double, 1>(p, st);
+            e = b->S == 2 ? launch_tick<double, 2, ASTRO_MAX_PLANETS>(p, st) : launch_tick<double, 1, ASTRO_MAX_PLANETS>(p, st);
         if (e != cudaSuccess) return fail(ASTRO_E_CUDA, "tick_kernel launch: %s", cudaGetErrorString(e));
         b->launches += 1;
         k0 += kc;
@@ -2518,6 +2550,9 @@ int astro_batch_create(const AstroConfig* cfg, int32_t n_games, int32_t bullet_c
     if (n_games <= 0 || n_games % ASTRO_TILE) return fail(ASTRO_E_INVALID, "n_games must be a positive multiple of %d", ASTRO_TILE);
     if (bullet_cap < 0 || bullet_cap > ASTRO_MAX_BULLET_CAP) return fail(ASTRO_E_INVALID, "bullet_cap out of range 0..%d", ASTRO_MAX_BULLET_CAP);
     if (precision != 32 && precision != 64) return fail(ASTRO_E_INVALID, "precision must be 32 or 64");
+    if (cfg->planet_slots != 0 && cfg->planet_slots != ASTRO_MAX_PLANETS && cfg->planet_slots != ASTRO_MAX_PLANETS_WIDE)
+        return fail(ASTRO_E_INVALID, "planet_slots must be 0 or %d (games of up to %d planets) or %d (up to %d planets), got %d",
+                    ASTRO_MAX_PLANETS, ASTRO_MAX_PLANETS, ASTRO_MAX_PLANETS_WIDE, ASTRO_MAX_PLANETS_WIDE, cfg->planet_slots);
     if ((int64_t)n_games * bullet_cap >= (int64_t)1 << 31)
         return fail(ASTRO_E_INVALID, "n_games * bullet_cap must stay below 2^31 bullet slots per batch (32-bit slot indexing)");
     int count = 0;
@@ -2536,6 +2571,7 @@ int astro_batch_create(const AstroConfig* cfg, int32_t n_games, int32_t bullet_c
     b->precision = precision;
     b->device = device;
     b->S = cfg->solo ? 1 : 2;
+    b->PL = cfg->planet_slots == ASTRO_MAX_PLANETS_WIDE ? ASTRO_MAX_PLANETS_WIDE : ASTRO_MAX_PLANETS;
     fill_consts(*cfg, b->c);
     if (cudaDeviceGetAttribute(&b->sm_count, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || b->sm_count <= 0) b->sm_count = 148;
     cudaError_t e = cudaMalloc(&b->d_stats, sizeof(unsigned long long) * 16 * kStatReplicas);
@@ -2619,8 +2655,9 @@ int astro_batch_bind(AstroBatch* b, const AstroBuffers* bufs) {
 
 int astro_set_schedule(AstroBatch* b, const uint32_t* fire_bits_host, int32_t n_ticks, int32_t timeout_tick) {
     if (int r = check(b, false)) return r;
-    if (!fire_bits_host || n_ticks <= 0 || n_ticks > ASTRO_MAX_TICKS + 1 || timeout_tick < 0 || timeout_tick >= n_ticks)
-        return fail(ASTRO_E_INVALID, "bad schedule (n_ticks %d, timeout_tick %d, max %d)", n_ticks, timeout_tick, ASTRO_MAX_TICKS);
+    const int32_t max_ticks = b->PL == ASTRO_MAX_PLANETS_WIDE ? ASTRO_MAX_TICKS_WIDE : ASTRO_MAX_TICKS;
+    if (!fire_bits_host || n_ticks <= 0 || n_ticks > max_ticks + 1 || timeout_tick < 0 || timeout_tick >= n_ticks)
+        return fail(ASTRO_E_INVALID, "bad schedule (n_ticks %d, timeout_tick %d, max %d)", n_ticks, timeout_tick, max_ticks);
     // util.direction (util.py:87-92) is restated for |b| <= 71476 (np_sincos_f32); beyond that numpy takes another
     // reduction path and the results would silently differ.  Bearings start below 2 pi (core.py:113) and turn by at
     // most dt * ship_rspeed per tick.
@@ -2657,15 +2694,22 @@ int astro_set_reset_pool(AstroBatch* b, const AstroResetPool* pool) {
     b->pool = *pool;
     b->config_epoch++;
     if (b->precision == 32) {
-        // the tick kernel reads a packed snapshot (one 128-byte record per entry)
+        // the tick kernel reads a packed snapshot (one 128-byte record per entry; 256 bytes with 8 planet slots)
         CUDA_TRY(cudaSetDevice(b->device));
         CUDA_TRY(cudaDeviceSynchronize());   // the pool may just have been written on another stream
         if (b->d_pool_rec) CUDA_TRY(cudaFree(b->d_pool_rec));
         b->d_pool_rec = nullptr;
-        CUDA_TRY(cudaMalloc(&b->d_pool_rec, (size_t)pool->size * 128));
+        const bool wide = b->PL == ASTRO_MAX_PLANETS_WIDE;
+        CUDA_TRY(cudaMalloc(&b->d_pool_rec, (size_t)pool->size * (wide ? 256 : 128)));
         const int grid = (pool->size + 127) / 128;
-        if (b->S == 2) pack_pool_kernel<2><<<grid, 128>>>((const float*)pool->ships, (const float*)pool->planets, pool->np, (float*)b->d_pool_rec, pool->size);
-        else pack_pool_kernel<1><<<grid, 128>>>((const float*)pool->ships, (const float*)pool->planets, pool->np, (float*)b->d_pool_rec, pool->size);
+        const float* ps = (const float*)pool->ships;
+        const float* pp = (const float*)pool->planets;
+        float* rec = (float*)b->d_pool_rec;
+        if (wide) {
+            if (b->S == 2) pack_pool_kernel<2, ASTRO_MAX_PLANETS_WIDE><<<grid, 128>>>(ps, pp, pool->np, rec, pool->size);
+            else pack_pool_kernel<1, ASTRO_MAX_PLANETS_WIDE><<<grid, 128>>>(ps, pp, pool->np, rec, pool->size);
+        } else if (b->S == 2) pack_pool_kernel<2, ASTRO_MAX_PLANETS><<<grid, 128>>>(ps, pp, pool->np, rec, pool->size);
+        else pack_pool_kernel<1, ASTRO_MAX_PLANETS><<<grid, 128>>>(ps, pp, pool->np, rec, pool->size);
         CUDA_TRY(cudaGetLastError());
         CUDA_TRY(cudaDeviceSynchronize());
         b->launches += 1;
@@ -2835,13 +2879,19 @@ int astro_reset_done(AstroBatch* b, void* stream) {
     fill_params(b, p);
     const int grid = (p.n_games + kTickThreads - 1) / kTickThreads;
     cudaStream_t st = (cudaStream_t)stream;
-    if (b->precision == 32) {
-        if (b->S == 2) reset_kernel<float, 2><<<grid, kTickThreads, 0, st>>>(p);
-        else reset_kernel<float, 1><<<grid, kTickThreads, 0, st>>>(p);
-    } else {
-        if (b->S == 2) reset_kernel<double, 2><<<grid, kTickThreads, 0, st>>>(p);
-        else reset_kernel<double, 1><<<grid, kTickThreads, 0, st>>>(p);
-    }
+#define LAUNCH_RESET(PL_)                                                                  \
+    do {                                                                                   \
+        if (b->precision == 32) {                                                          \
+            if (b->S == 2) reset_kernel<float, 2, PL_><<<grid, kTickThreads, 0, st>>>(p);  \
+            else reset_kernel<float, 1, PL_><<<grid, kTickThreads, 0, st>>>(p);            \
+        } else {                                                                           \
+            if (b->S == 2) reset_kernel<double, 2, PL_><<<grid, kTickThreads, 0, st>>>(p); \
+            else reset_kernel<double, 1, PL_><<<grid, kTickThreads, 0, st>>>(p);           \
+        }                                                                                  \
+    } while (0)
+    if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_RESET(ASTRO_MAX_PLANETS_WIDE);
+    else LAUNCH_RESET(ASTRO_MAX_PLANETS);
+#undef LAUNCH_RESET
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
     return ASTRO_OK;
@@ -2851,7 +2901,7 @@ static int observe_impl(AstroBatch* b, float* obs, int32_t n_rows, bool both, vo
     if (int r = check(b, true)) return r;
     if (!obs) return fail(ASTRO_E_INVALID, "null obs");
     const int D = 1 + 5 * b->S + 4;
-    if (n_rows < ASTRO_MAX_PLANETS + b->K) return fail(ASTRO_E_INVALID, "n_rows %d < 4 + bullet_cap %d", n_rows, b->K);
+    if (n_rows < b->PL + b->K) return fail(ASTRO_E_INVALID, "n_rows %d < %d planet slots + bullet_cap %d", n_rows, b->PL, b->K);
     if ((n_rows * D) % 4) return fail(ASTRO_E_INVALID, "n_rows * %d must be a multiple of 4", D);
     if ((uintptr_t)obs & 15) return fail(ASTRO_E_INVALID, "obs must be 16-byte aligned");
     CUDA_TRY(cudaSetDevice(b->device));
@@ -2861,19 +2911,25 @@ static int observe_impl(AstroBatch* b, float* obs, int32_t n_rows, bool both, vo
     cudaStream_t st = (cudaStream_t)stream;
     const AstroBuffers& u = b->bufs;
     const void* cur_bullets = current_bullets(b);
-#define LAUNCH_OBS(R, S_, BOTH_)                                                                                       \
-    do {                                                                                                               \
-        CUDA_TRY(cudaFuncSetAttribute(observe_kernel<R, S_, BOTH_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        observe_kernel<R, S_, BOTH_><<<grid, kObserveWarps * 32, smem, st>>>(u.ships, u.ship_b, u.planets, cur_bullets, u.meta, \
-                                                                             obs, b->n_games, b->K, n_rows);             \
+#define LAUNCH_OBS(R, S_, BOTH_, PL_)                                                                                       \
+    do {                                                                                                                    \
+        CUDA_TRY(cudaFuncSetAttribute(observe_kernel<R, S_, BOTH_, PL_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+        observe_kernel<R, S_, BOTH_, PL_><<<grid, kObserveWarps * 32, smem, st>>>(u.ships, u.ship_b, u.planets, cur_bullets, u.meta, \
+                                                                                  obs, b->n_games, b->K, n_rows);             \
     } while (0)
-    if (b->precision == 32) {
-        if (b->S == 2) { if (both) LAUNCH_OBS(float, 2, true); else LAUNCH_OBS(float, 2, false); }
-        else LAUNCH_OBS(float, 1, false);
-    } else {
-        if (b->S == 2) { if (both) LAUNCH_OBS(double, 2, true); else LAUNCH_OBS(double, 2, false); }
-        else LAUNCH_OBS(double, 1, false);
-    }
+#define LAUNCH_OBS_PL(PL_)                                                                                        \
+    do {                                                                                                          \
+        if (b->precision == 32) {                                                                                 \
+            if (b->S == 2) { if (both) LAUNCH_OBS(float, 2, true, PL_); else LAUNCH_OBS(float, 2, false, PL_); }   \
+            else LAUNCH_OBS(float, 1, false, PL_);                                                                \
+        } else {                                                                                                  \
+            if (b->S == 2) { if (both) LAUNCH_OBS(double, 2, true, PL_); else LAUNCH_OBS(double, 2, false, PL_); } \
+            else LAUNCH_OBS(double, 1, false, PL_);                                                               \
+        }                                                                                                         \
+    } while (0)
+    if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_OBS_PL(ASTRO_MAX_PLANETS_WIDE);
+    else LAUNCH_OBS_PL(ASTRO_MAX_PLANETS);
+#undef LAUNCH_OBS_PL
 #undef LAUNCH_OBS
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
@@ -2903,13 +2959,19 @@ int astro_script_controls(AstroBatch* b, double avoid_distance, double avoid_thr
     const int grid = (b->n_games * b->S + 127) / 128;
     cudaStream_t st = (cudaStream_t)stream;
     const AstroBuffers& u = b->bufs;
-    if (b->precision == 32) {
-        if (b->S == 2) script_kernel<float, 2><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, u.meta, actions, q);
-        else script_kernel<float, 1><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, u.meta, actions, q);
-    } else {
-        if (b->S == 2) script_kernel<double, 2><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, u.meta, actions, q);
-        else script_kernel<double, 1><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, u.meta, actions, q);
-    }
+#define LAUNCH_SCRIPT(PL_)                                                                                              \
+    do {                                                                                                                \
+        if (b->precision == 32) {                                                                                       \
+            if (b->S == 2) script_kernel<float, 2, PL_><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, u.meta, actions, q);  \
+            else script_kernel<float, 1, PL_><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, u.meta, actions, q);            \
+        } else {                                                                                                        \
+            if (b->S == 2) script_kernel<double, 2, PL_><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, u.meta, actions, q); \
+            else script_kernel<double, 1, PL_><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, u.meta, actions, q);           \
+        }                                                                                                               \
+    } while (0)
+    if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_SCRIPT(ASTRO_MAX_PLANETS_WIDE);
+    else LAUNCH_SCRIPT(ASTRO_MAX_PLANETS);
+#undef LAUNCH_SCRIPT
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
     return ASTRO_OK;
@@ -2919,8 +2981,9 @@ int astro_create_games(AstroBatch* b, const AstroCreateConfig* cc, const uint32_
                        void* planets, int32_t* n_planets, void* stream) {
     if (int r = check(b, false)) return r;
     if (!cc || !seeds || !ships || !planets || !n_planets || m <= 0) return fail(ASTRO_E_INVALID, "bad create arguments");
-    if (cc->max_planets < 1 || cc->max_planets > ASTRO_MAX_PLANETS)
-        return fail(ASTRO_E_INVALID, "max_planets must be 1..%d", ASTRO_MAX_PLANETS);
+    if (cc->max_planets < 1 || cc->max_planets > b->PL)
+        return fail(ASTRO_E_INVALID, "max_planets must be 1..%d (the batch's planet slots; at most %d with planet_slots = %d)",
+                    b->PL, ASTRO_MAX_PLANETS_WIDE, ASTRO_MAX_PLANETS_WIDE);
     CUDA_TRY(cudaSetDevice(b->device));
     CreateParams q;
     q.inner = cc->inner_ship_position;
@@ -2934,13 +2997,19 @@ int astro_create_games(AstroBatch* b, const AstroCreateConfig* cc, const uint32_
     q.pad = 0;
     const int grid = (m + 63) / 64;
     cudaStream_t st = (cudaStream_t)stream;
-    if (b->precision == 32) {
-        if (b->S == 2) create_kernel<float, 2><<<grid, 64, 0, st>>>(seeds, (float*)ships, (float*)planets, n_planets, q);
-        else create_kernel<float, 1><<<grid, 64, 0, st>>>(seeds, (float*)ships, (float*)planets, n_planets, q);
-    } else {
-        if (b->S == 2) create_kernel<double, 2><<<grid, 64, 0, st>>>(seeds, (double*)ships, (double*)planets, n_planets, q);
-        else create_kernel<double, 1><<<grid, 64, 0, st>>>(seeds, (double*)ships, (double*)planets, n_planets, q);
-    }
+#define LAUNCH_CREATE(PL_)                                                                                                  \
+    do {                                                                                                                    \
+        if (b->precision == 32) {                                                                                           \
+            if (b->S == 2) create_kernel<float, 2, PL_><<<grid, 64, 0, st>>>(seeds, (float*)ships, (float*)planets, n_planets, q);   \
+            else create_kernel<float, 1, PL_><<<grid, 64, 0, st>>>(seeds, (float*)ships, (float*)planets, n_planets, q);             \
+        } else {                                                                                                            \
+            if (b->S == 2) create_kernel<double, 2, PL_><<<grid, 64, 0, st>>>(seeds, (double*)ships, (double*)planets, n_planets, q); \
+            else create_kernel<double, 1, PL_><<<grid, 64, 0, st>>>(seeds, (double*)ships, (double*)planets, n_planets, q);           \
+        }                                                                                                                   \
+    } while (0)
+    if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_CREATE(ASTRO_MAX_PLANETS_WIDE);
+    else LAUNCH_CREATE(ASTRO_MAX_PLANETS);
+#undef LAUNCH_CREATE
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
     return ASTRO_OK;
@@ -3071,23 +3140,28 @@ int astro_policy_controls(AstroBatch* b, uint8_t* actions, float* q_out, int32_t
         int mgrid = ((b->n_games + 7) / 8 + kMmaWarps - 1) / kMmaWarps;      // a warp takes 8 games at a time
         if (mgrid > sms * ASTRO_MMA_MIN_BLOCKS) mgrid = sms * ASTRO_MMA_MIN_BLOCKS;
         const int msmem = (int)sizeof(PolicyFrags);
-#define LAUNCH_MMA(R, S_) \
-    do { CUDA_TRY(cudaFuncSetAttribute(policy_mma_kernel<R, S_>, cudaFuncAttributeMaxDynamicSharedMemorySize, msmem)); \
-    policy_mma_kernel<R, S_><<<mgrid, kMmaWarps * 32, msmem, st>>>(u.ships, u.ship_b, u.planets, current_bullets(b), u.meta, actions, q_out, b->n_games, b->K, b->policy_nout, ship_mask, b->d_pol_frags); } while (0)
-        if (b->precision == 32) { if (b->S == 2) LAUNCH_MMA(float, 2); else LAUNCH_MMA(float, 1); }
-        else { if (b->S == 2) LAUNCH_MMA(double, 2); else LAUNCH_MMA(double, 1); }
+#define LAUNCH_MMA(R, S_, PL_) \
+    do { CUDA_TRY(cudaFuncSetAttribute(policy_mma_kernel<R, S_, PL_>, cudaFuncAttributeMaxDynamicSharedMemorySize, msmem)); \
+    policy_mma_kernel<R, S_, PL_><<<mgrid, kMmaWarps * 32, msmem, st>>>(u.ships, u.ship_b, u.planets, current_bullets(b), u.meta, actions, q_out, b->n_games, b->K, b->policy_nout, ship_mask, b->d_pol_frags); } while (0)
+#define LAUNCH_MMA_PL(PL_) \
+    do { if (b->precision == 32) { if (b->S == 2) LAUNCH_MMA(float, 2, PL_); else LAUNCH_MMA(float, 1, PL_); } \
+         else { if (b->S == 2) LAUNCH_MMA(double, 2, PL_); else LAUNCH_MMA(double, 1, PL_); } } while (0)
+        if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_MMA_PL(ASTRO_MAX_PLANETS_WIDE);
+        else LAUNCH_MMA_PL(ASTRO_MAX_PLANETS);
+#undef LAUNCH_MMA_PL
 #undef LAUNCH_MMA
         CUDA_TRY(cudaGetLastError());
         b->launches += 1;
         return ASTRO_OK;
     }
-#define LAUNCH_POL(R, S_) \
-    policy_kernel<R, S_><<<grid, kPolWarps * 32, 0, st>>>(u.ships, u.ship_b, u.planets, current_bullets(b), u.meta, actions, q_out, b->n_games, b->K, b->policy_nout, ship_mask, b->d_pol)
-    if (b->precision == 32) {
-        if (b->S == 2) LAUNCH_POL(float, 2); else LAUNCH_POL(float, 1);
-    } else {
-        if (b->S == 2) LAUNCH_POL(double, 2); else LAUNCH_POL(double, 1);
-    }
+#define LAUNCH_POL(R, S_, PL_) \
+    policy_kernel<R, S_, PL_><<<grid, kPolWarps * 32, 0, st>>>(u.ships, u.ship_b, u.planets, current_bullets(b), u.meta, actions, q_out, b->n_games, b->K, b->policy_nout, ship_mask, b->d_pol)
+#define LAUNCH_POL_PL(PL_) \
+    do { if (b->precision == 32) { if (b->S == 2) LAUNCH_POL(float, 2, PL_); else LAUNCH_POL(float, 1, PL_); } \
+         else { if (b->S == 2) LAUNCH_POL(double, 2, PL_); else LAUNCH_POL(double, 1, PL_); } } while (0)
+    if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_POL_PL(ASTRO_MAX_PLANETS_WIDE);
+    else LAUNCH_POL_PL(ASTRO_MAX_PLANETS);
+#undef LAUNCH_POL_PL
 #undef LAUNCH_POL
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
@@ -3114,12 +3188,16 @@ int astro_explore_controls(AstroBatch* b, double t_in, double t_out, uint32_t se
     CUDA_TRY(cudaSetDevice(b->device));
     const int grid = (b->n_games * b->S + 127) / 128;
     cudaStream_t st = (cudaStream_t)stream;
-    if (b->S == 2)
-        explore_kernel<2><<<grid, 128, 0, st>>>(b->bufs.meta, state, actions, b->n_games, ship_mask, b->cfg.dt, t_in, t_out, seed,
-                                                (uint32_t)b->first_game, b->step, b->step_base_now);
-    else
-        explore_kernel<1><<<grid, 128, 0, st>>>(b->bufs.meta, state, actions, b->n_games, ship_mask, b->cfg.dt, t_in, t_out, seed,
-                                                (uint32_t)b->first_game, b->step, b->step_base_now);
+#define LAUNCH_EXPLORE(S_, PL_)                                                                                                 \
+    explore_kernel<S_, PL_><<<grid, 128, 0, st>>>(b->bufs.meta, state, actions, b->n_games, ship_mask, b->cfg.dt, t_in, t_out, seed, \
+                                                  (uint32_t)b->first_game, b->step, b->step_base_now)
+    const bool wide = b->PL == ASTRO_MAX_PLANETS_WIDE;
+    if (b->S == 2) {
+        if (wide) LAUNCH_EXPLORE(2, ASTRO_MAX_PLANETS_WIDE); else LAUNCH_EXPLORE(2, ASTRO_MAX_PLANETS);
+    } else {
+        if (wide) LAUNCH_EXPLORE(1, ASTRO_MAX_PLANETS_WIDE); else LAUNCH_EXPLORE(1, ASTRO_MAX_PLANETS);
+    }
+#undef LAUNCH_EXPLORE
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
     return ASTRO_OK;
@@ -3222,10 +3300,12 @@ int astro_rollout_device(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, int
     }
     // ScriptBot / NothingBot on every ship (float32 build): the bots are evaluated INSIDE the tick kernel, from the rows a tile's
     // warp has just loaded, so the ticks of a tile run back to back within a launch — no launch, no control array between ticks
-    // (`actions` is not written).  ASTRO_FUSED_BOTS=0 switches it off.
+    // (`actions` is not written).  ASTRO_FUSED_BOTS=0 switches it off.  Batches with 8 planet slots have no such instantiation
+    // and always take the bot kernel -> tick kernel loop below.
     {
         const char* fb = getenv("ASTRO_FUSED_BOTS");
-        if (!any_policy && b->precision == 32 && !(flags & ASTRO_TICK_GENERIC_KERNEL) && !(fb && atoi(fb) == 0) && n_ticks > 0) {
+        if (!any_policy && b->precision == 32 && b->PL == ASTRO_MAX_PLANETS && !(flags & ASTRO_TICK_GENERIC_KERNEL) && !(fb && atoi(fb) == 0) &&
+            n_ticks > 0) {
             b->bot_modes_now = modes[0] | (modes[1] << 4);
             ScriptParams& q = b->script_now;
             q.radius = b->cfg.planet_radius + b->cfg.ship_radius;
@@ -3319,10 +3399,14 @@ int astro_export_games(AstroBatch* b, const int32_t* index, int32_t m, const Ast
     const AstroBuffers& u = b->bufs;
     const int grid = (m + 3) / 4;
     cudaStream_t st = (cudaStream_t)stream;
-#define LAUNCH_EXP(R, S_) \
-    export_kernel<R, S_><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, current_bullets(b), u.meta, u.episode, index, m, b->n_games, b->K, out->bullet_rows, a)
-    if (b->precision == 32) { if (b->S == 2) LAUNCH_EXP(float, 2); else LAUNCH_EXP(float, 1); }
-    else { if (b->S == 2) LAUNCH_EXP(double, 2); else LAUNCH_EXP(double, 1); }
+#define LAUNCH_EXP(R, S_, PL_) \
+    export_kernel<R, S_, PL_><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, current_bullets(b), u.meta, u.episode, index, m, b->n_games, b->K, out->bullet_rows, a)
+#define LAUNCH_EXP_PL(PL_) \
+    do { if (b->precision == 32) { if (b->S == 2) LAUNCH_EXP(float, 2, PL_); else LAUNCH_EXP(float, 1, PL_); } \
+         else { if (b->S == 2) LAUNCH_EXP(double, 2, PL_); else LAUNCH_EXP(double, 1, PL_); } } while (0)
+    if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_EXP_PL(ASTRO_MAX_PLANETS_WIDE);
+    else LAUNCH_EXP_PL(ASTRO_MAX_PLANETS);
+#undef LAUNCH_EXP_PL
 #undef LAUNCH_EXP
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
@@ -3353,10 +3437,14 @@ int astro_import_games(AstroBatch* b, const int32_t* index, int32_t m, const Ast
     void* cur = (char*)u.bullets + (size_t)b->cur * buf_bytes;
     void* other = (char*)u.bullets + (size_t)(b->cur ^ 1) * buf_bytes;
     const int grid = (b->n_games / ASTRO_TILE + 3) / 4;
-#define LAUNCH_IMP(R, S_) \
-    import_kernel<R, S_><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, cur, other, u.meta, u.episode, src, m, b->n_games, b->K, in->bullet_rows, a)
-    if (b->precision == 32) { if (b->S == 2) LAUNCH_IMP(float, 2); else LAUNCH_IMP(float, 1); }
-    else { if (b->S == 2) LAUNCH_IMP(double, 2); else LAUNCH_IMP(double, 1); }
+#define LAUNCH_IMP(R, S_, PL_) \
+    import_kernel<R, S_, PL_><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, cur, other, u.meta, u.episode, src, m, b->n_games, b->K, in->bullet_rows, a)
+#define LAUNCH_IMP_PL(PL_) \
+    do { if (b->precision == 32) { if (b->S == 2) LAUNCH_IMP(float, 2, PL_); else LAUNCH_IMP(float, 1, PL_); } \
+         else { if (b->S == 2) LAUNCH_IMP(double, 2, PL_); else LAUNCH_IMP(double, 1, PL_); } } while (0)
+    if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_IMP_PL(ASTRO_MAX_PLANETS_WIDE);
+    else LAUNCH_IMP_PL(ASTRO_MAX_PLANETS);
+#undef LAUNCH_IMP_PL
 #undef LAUNCH_IMP
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
@@ -3426,7 +3514,7 @@ int astro_step_single_host(AstroBatch* b, const AstroSingleGame* in_host, AstroS
     if (b->n_games != ASTRO_TILE) return fail(ASTRO_E_INVALID, "astro_step_single_host needs a one-tile batch (n_games = %d)", ASTRO_TILE);
     const int32_t nb = in_host->n_bullets;
     if (nb < 0 || nb > b->K) return fail(ASTRO_E_INVALID, "the game holds %d bullets, bullet_cap is %d", nb, b->K);
-    if (in_host->n_planets < 1 || in_host->n_planets > ASTRO_MAX_PLANETS) return fail(ASTRO_E_INVALID, "a game needs 1..%d planets", ASTRO_MAX_PLANETS);
+    if (in_host->n_planets < 1 || in_host->n_planets > b->PL) return fail(ASTRO_E_INVALID, "a game needs 1..%d planets", b->PL);
     if (b->n_sched_ticks <= 0) return fail(ASTRO_E_STATE, "astro_set_schedule has not been called");
     if (in_host->tick < 0 || in_host->tick >= b->n_sched_ticks) return fail(ASTRO_E_INVALID, "tick %d is not on the schedule", in_host->tick);
     for (int s = 0; s < b->S; s++) {
@@ -3482,6 +3570,9 @@ static void fresh_free(AstroBatch* b) {
 
 int astro_fresh_games_enable(AstroBatch* b, const AstroCreateConfig* cc, uint32_t config_seed, int64_t skip, int32_t quota, void* stream) {
     if (int r = check(b, true)) return r;
+    if (b->PL != ASTRO_MAX_PLANETS)
+        return fail(ASTRO_E_INVALID, "fresh-game mode is not available in batches with %d planet slots (planet_slots = %d): use a reset pool",
+                    b->PL, b->PL);
     if (!cc || cc->max_planets < 1 || cc->max_planets > ASTRO_MAX_PLANETS) return fail(ASTRO_E_INVALID, "bad create config");
     if (b->precision != 32) return fail(ASTRO_E_INVALID, "fresh-game mode needs the float32 build");
     if (quota < 1 || quota > 1024 || skip < 0) return fail(ASTRO_E_INVALID, "quota must be 1..1024, skip >= 0");

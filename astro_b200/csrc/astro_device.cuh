@@ -20,6 +20,23 @@ struct alignas(4 * sizeof(R)) Body4 {
     R x, y, dx, dy;
 };
 
+// ---- the meta word (include/astro_b200.h) of a batch with PL planet slots ---------------------
+// PL = 4 reads and writes today's fields; PL = 8 keeps np's fourth bit in bit 31 (ASTRO_META_*_WIDE).
+template <int PL>
+__host__ __device__ __forceinline__ uint32_t meta_np(uint32_t m) {
+    return PL > ASTRO_MAX_PLANETS ? ASTRO_META_NP_WIDE(m) : ASTRO_META_NP(m);
+}
+template <int PL>
+__host__ __device__ __forceinline__ uint32_t meta_tick(uint32_t m) {
+    return PL > ASTRO_MAX_PLANETS ? ASTRO_META_TICK_WIDE(m) : ASTRO_META_TICK(m);
+}
+template <int PL>
+__host__ __device__ __forceinline__ uint32_t meta_pack(uint32_t nb, uint32_t np, uint32_t fin, uint32_t tick) {
+    return PL > ASTRO_MAX_PLANETS ? ASTRO_META_PACK_WIDE(nb, np, fin, tick) : ASTRO_META_PACK(nb, np, fin, tick);
+}
+template <int PL>
+__host__ __device__ constexpr uint32_t max_ticks() { return PL > ASTRO_MAX_PLANETS ? ASTRO_MAX_TICKS_WIDE : ASTRO_MAX_TICKS; }
+
 // ---- counter-based streams (host twin: astro_b200/rng.py) -------------------------------
 __device__ __forceinline__ uint32_t mix32(uint32_t x) {
     x ^= x >> 16; x *= 0x7FEB352Du; x ^= x >> 15; x *= 0x846CA68Bu; x ^= x >> 16;
@@ -277,16 +294,16 @@ __device__ __forceinline__ int fly_to(double target, double my_b, double t, bool
 // discriminant — runs for every planet without divergence and leaves a bit mask of the planets on a collision course;
 // only those go through the atan2 / norm_angle test, in planet order (the first dangerous planet decides, script.py:69-76).
 // Quirk kept: inside _danger the parameter `b` (my bearing) is shadowed by the quadratic coefficient (script.py:54).
-template <typename R, int S>
-__device__ __forceinline__ int script_decide(const Body4<R>& mv, R mb, const Body4<R>& ev, const Body4<R> (&pl)[ASTRO_MAX_PLANETS], int np,
+template <typename R, int S, int PL>
+__device__ __forceinline__ int script_decide(const Body4<R>& mv, R mb, const Body4<R>& ev, const Body4<R> (&pl)[PL], int np,
                                              const ScriptParams& q) {
     const double my[5] = {(double)mv.x, (double)mv.y, (double)mv.dx, (double)mv.dy, (double)mb};
     unsigned cand = 0;
-    double cx0[ASTRO_MAX_PLANETS], cx1[ASTRO_MAX_PLANETS], cb[ASTRO_MAX_PLANETS], csd[ASTRO_MAX_PLANETS], cspeed[ASTRO_MAX_PLANETS];
+    double cx0[PL], cx1[PL], cb[PL], csd[PL], cspeed[PL];
     const double ra = __dadd_rn(q.radius, q.avoid_distance);
     const double ra2 = __dmul_rn(ra, ra);
 #pragma unroll
-    for (int j = 0; j < ASTRO_MAX_PLANETS; j++) {
+    for (int j = 0; j < PL; j++) {
         cx0[j] = cx1[j] = cb[j] = csd[j] = cspeed[j] = 0.0;
         if (j < np) {
             const Body4<R> v = pl[j];
@@ -314,7 +331,7 @@ __device__ __forceinline__ int script_decide(const Body4<R>& mv, R mb, const Bod
         cand &= cand - 1u;
         double x0 = cx0[0], x1 = cx1[0], b = cb[0], sd = csd[0], speed = cspeed[0];
 #pragma unroll
-        for (int k = 1; k < ASTRO_MAX_PLANETS; k++)
+        for (int k = 1; k < PL; k++)
             if (j == k) { x0 = cx0[k]; x1 = cx1[k]; b = cb[k]; sd = csd[k]; speed = cspeed[k]; }
         const double distance = __dsub_rn(-b, sd);
         const double bear = atan2(x0, x1);                                        // util.bearing(x)

@@ -19,7 +19,7 @@
 //  B. SHIPS AND PLANETS, thread-per-game from the staged copies: direction, gravity, collisions,
 //     terminal logic, spawn, integration, reset — all coalesced 128-bit accesses.
 //
-// Instantiations, tick_f32_kernel<S, STATS, MANY, BOT, FIX>:
+// Instantiations, tick_f32_kernel<S, STATS, MANY, BOT, FIX> (4 planet slots) and tick_f32_wide_kernel<S, STATS, MANY> (8):
 //   MANY  several ticks of a tile per launch (astro_tick_many): meta / ships / bearings handed from tick to tick in registers,
 //         7 staging windows and 28 one-warp CTAs per SM (the one-tick launch: 8 and 26) — this form is bound by instruction issue
 //   BOT   script.ScriptBot / NothingBot evaluated inside the tick (astro_rollout_device)
@@ -57,6 +57,14 @@ constexpr int kTickWarps = kTickThreads / 32;
 #ifndef ASTRO_TICK_MIN_BLOCKS_BOT
 #define ASTRO_TICK_MIN_BLOCKS_BOT 12    /* the instantiation with the ScriptBot inside: float64 chains, 160 registers */
 #endif
+// 8 planet slots (PL = 8): eight float4 planets, their pairs and forces live in registers, and the staged frame holds two
+// more planet pairs per game (1 KB more shared memory per warp)
+#ifndef ASTRO_TICK_MIN_BLOCKS_WIDE
+#define ASTRO_TICK_MIN_BLOCKS_WIDE 16
+#endif
+#ifndef ASTRO_TICK_MIN_BLOCKS_WIDE_MANY
+#define ASTRO_TICK_MIN_BLOCKS_WIDE_MANY 16
+#endif
 // Round 2, instruction diet of the fused form (issue-bound; ncu dynamic instruction counts in profiles/r2_ab_diet.md):
 #ifndef ASTRO_OPT_STAGE
 #define ASTRO_OPT_STAGE 1     /* several ticks per launch: staging requests unrolled and predicated, 2-3 instructions per window instead of ~14 */
@@ -67,11 +75,11 @@ constexpr int kTickWarps = kTickThreads / 32;
 
 // Per-game entries used by the bullet loop are indexed by the game's rank among the tile's games
 // that own bullets (`cid`): item -> cid comes out of one ballot per window, no lookup table.
-template <int W>
+template <int W, int PL>
 struct TileScratchT {              // per warp
     float4 bul[W * 32];            // the tile's bullet list, staged by cp.async; survivors are compacted here
-    float4 fsxy[32];               // [cid] OLD ship0.xy, ship1.xy          } what the bullet loop reads
-    float4 fpxy[2][32];            // [cid] OLD planet0.xy planet1.xy / 2,3 } (transposed pairs)
+    float4 fsxy[32];               // [cid] OLD ship0.xy, ship1.xy                } what the bullet loop reads
+    float4 fpxy[PL / 2][32];       // [cid] OLD planet0.xy planet1.xy / 2,3 / ... } (transposed pairs)
     float4 sxy[32];                // [lane] OLD ship positions  }
     float4 svel[32];               // [lane] OLD ship velocities } for the newborn bullets
     float4 dir[32];                // [lane] sin/cos of both bearings
@@ -119,16 +127,23 @@ struct ExactResult {
     float x, y;
     unsigned flags;  // bit 0 keep, bits 1-2 ship hits
 };
-__device__ __forceinline__ ExactResult bullet_exact(float bx, float by, float bdx, float bdy, float4 sxy, float4 p01,
-                                                    float4 p23, int n_ships, int np, const Consts& c) {
+// p[k] = planets 2k and 2k + 1: (x, y) of each.
+template <int PL>
+__device__ __forceinline__ ExactResult bullet_exact(float bx, float by, float bdx, float bdy, float4 sxy, const float4 (&p)[PL / 2],
+                                                    int n_ships, int np, const Consts& c) {
     unsigned ship_hits = 0;
     if (collide_exact((double)sxy.x, (double)sxy.y, (double)bx, (double)by, c.r2_sb)) ship_hits |= 1u;
     if (n_ships > 1 && collide_exact((double)sxy.z, (double)sxy.w, (double)bx, (double)by, c.r2_sb)) ship_hits |= 2u;
     bool gone = ship_hits != 0;
-    gone |= collide_exact((double)p01.x, (double)p01.y, (double)bx, (double)by, c.r2_pb);  // np >= 1
-    if (np > 1) gone |= collide_exact((double)p01.z, (double)p01.w, (double)bx, (double)by, c.r2_pb);
-    if (np > 2) gone |= collide_exact((double)p23.x, (double)p23.y, (double)bx, (double)by, c.r2_pb);
-    if (np > 3) gone |= collide_exact((double)p23.z, (double)p23.w, (double)bx, (double)by, c.r2_pb);
+    gone |= collide_exact((double)p[0].x, (double)p[0].y, (double)bx, (double)by, c.r2_pb);  // np >= 1
+    if (np > 1) gone |= collide_exact((double)p[0].z, (double)p[0].w, (double)bx, (double)by, c.r2_pb);
+    if (np > 2) gone |= collide_exact((double)p[1].x, (double)p[1].y, (double)bx, (double)by, c.r2_pb);
+    if (np > 3) gone |= collide_exact((double)p[1].z, (double)p[1].w, (double)bx, (double)by, c.r2_pb);
+#pragma unroll
+    for (int k = 2; k < PL / 2; k++) {
+        if (np > 2 * k) gone |= collide_exact((double)p[k].x, (double)p[k].y, (double)bx, (double)by, c.r2_pb);
+        if (np > 2 * k + 1) gone |= collide_exact((double)p[k].z, (double)p[k].w, (double)bx, (double)by, c.r2_pb);
+    }
     double v0 = __dadd_rn((double)bdx, c.zero_dt), v1 = __dadd_rn((double)bdy, c.zero_dt);
     double e0 = __dadd_rn((double)bx, __dmul_rn(c.dt, v0)), e1 = __dadd_rn((double)by, __dmul_rn(c.dt, v1));
     ExactResult r;
@@ -200,29 +215,34 @@ __device__ __forceinline__ f32x2 dist2_pair(float4 o, f32x2 bx, f32x2 by) {
 }
 
 // bullet_exact() for the transposed staging.
-__device__ __forceinline__ ExactResult bullet_exact_t(float4 bv, float4 sT, float4 pA, float4 pB, int n_ships, int np,
+template <int PL>
+__device__ __forceinline__ ExactResult bullet_exact_t(float4 bv, float4 sT, const float4 (&pT)[PL / 2], int n_ships, int np,
                                                       const Consts& c) {
-    return bullet_exact(bv.x, bv.y, bv.z, bv.w, make_float4(sT.x, sT.z, sT.y, sT.w), make_float4(pA.x, pA.z, pA.y, pA.w),
-                        make_float4(pB.x, pB.z, pB.y, pB.w), n_ships, np, c);
+    float4 p[PL / 2];
+#pragma unroll
+    for (int k = 0; k < PL / 2; k++) p[k] = make_float4(pT[k].x, pT[k].z, pT[k].y, pT[k].w);
+    return bullet_exact<PL>(bv.x, bv.y, bv.z, bv.w, make_float4(sT.x, sT.z, sT.y, sT.w), p, n_ships, np, c);
 }
 
 // One bullet bv = (x, y, dx, dy) against its game's staged frame (transposed pairs: both ships,
-// planets 0/1, planets 2/3).  Returns keep; bv.x / bv.y advanced; ship_hits receives bits 0/1 when
+// planets 0/1, planets 2/3, ...).  Returns keep; bv.x / bv.y advanced; ship_hits receives bits 0/1 when
 // the bullet touches ship 0/1 (always decided in float64).  Arena test: keep iff (|x'| <= 1) or
 // (|y'| <= 1)  <=>  min(|x'|, |y'|) <= 1, so only the smaller magnitude can sit in the band.
-template <int S>
-__device__ __forceinline__ bool bullet_step_t(float4& bv, float4 sT, float4 pA, float4 pB, const uint32_t* np_of,
+template <int S, int PL>
+__device__ __forceinline__ bool bullet_step_t(float4& bv, float4 sT, const float4 (&pT)[PL / 2], const uint32_t* np_of,
                                               unsigned gi, const Consts& c, unsigned& ship_hits) {
     const f32x2 bx = bc2(bv.x), by = bc2(bv.y);
     const float ds = min2(dist2_pair(sT, bx, by));  // S == 1: both halves hold ship 0
-    const float dp = fminf(min2(dist2_pair(pA, bx, by)), min2(dist2_pair(pB, bx, by)));
+    float dp = fminf(min2(dist2_pair(pT[0], bx, by)), min2(dist2_pair(pT[1], bx, by)));
+#pragma unroll
+    for (int k = 2; k < PL / 2; k++) dp = fminf(dp, min2(dist2_pair(pT[k], bx, by)));
     float x0, x1;
     upk2(fma2(bc2(c.dt_f), pk2(bv.z, bv.w), pk2(bv.x, bv.y)), x0, x1);
     const float mn = fminf(fabsf(x0), fabsf(x1));
     const bool sure = (ds >= c.r2f_sb * 1.000001f) & (fabsf(dp - c.r2f_pb) > c.r2f_pb * 1e-6f) & (fabsf(mn - 1.0f) > 4e-6f);
     bool keep = (mn <= 1.0f) & (dp >= c.r2f_pb);
     if (__builtin_expect(!sure, 0)) {
-        ExactResult r = bullet_exact_t(bv, sT, pA, pB, S, (int)(np_of[gi] >> 8), c);
+        ExactResult r = bullet_exact_t<PL>(bv, sT, pT, S, (int)(np_of[gi] >> 8), c);
         x0 = r.x;
         x1 = r.y;
         keep = r.flags & 1u;
@@ -372,7 +392,7 @@ struct TileIn {
     uint32_t ctl_raw;   // the tile's control bytes of this lane's game (S bytes), when actions are given
     uint32_t fire_word; // (several ticks per launch) the fire-schedule word of this game's tick, requested at the top
 };
-template <int S, bool FIX = false, bool WARM_PLANETS = true>
+template <int S, int PL, bool FIX = false, bool WARM_PLANETS = true>
 __device__ __forceinline__ void load_tile_in(const TickParams& p, const TickVar& v, unsigned tile, unsigned lane, TileIn& in) {
     const size_t g = (size_t)tile * 32 + lane;
     in.meta = LD_STREAM(&p.meta[g]);
@@ -381,7 +401,7 @@ __device__ __forceinline__ void load_tile_in(const TickParams& p, const TickVar&
     // The planet slots to load depend on meta (np).  Warm L2 with the tile's planet rows meanwhile:
     // the dependent loads then take an L2 round trip instead of an HBM one (measured:
     // 93.4 -> 91.4 us per 1M-game tick; sectors without a live lane are the price).
-    const float4* planets = reinterpret_cast<const float4*>(p.planets) + (size_t)tile * (ASTRO_MAX_PLANETS * 32) + lane;
+    const float4* planets = reinterpret_cast<const float4*>(p.planets) + (size_t)tile * (PL * 32) + lane;
     if (WARM_PLANETS) {
 #pragma unroll
         for (int j = 0; j < ASTRO_PREFETCH_PLANETS; j++) asm volatile("prefetch.global.L2 [%0];" ::"l"(&planets[j * 32]));
@@ -407,10 +427,10 @@ __device__ __forceinline__ void load_tile_in(const TickParams& p, const TickVar&
 // FIX = the launch's options are the production rollout's, known at compile time (launch_tick_f32 checks them): duel games,
 // packed controls given, event planes written, no reward / done arrays, auto-reset from the pool (no ring, no captured
 // step base) — the tests of those options and the address arithmetic of the absent arrays fold away.
-template <int S, bool STATS, bool MANY, bool BOT, bool FIX>
+template <int S, bool STATS, bool MANY, bool BOT, bool FIX, int PL>
 // `last` = no further tick of this tile follows in this launch: only then do meta, ships and bearings go to memory
 // (planets and the bullet list always do), and the tile's statistics (`stat_acc`, summed over the launch's ticks).
-__device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v, TileScratchT<MANY ? ASTRO_STAGE_WINDOWS_MANY : ASTRO_STAGE_WINDOWS>& t, const unsigned lane,
+__device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v, TileScratchT<MANY ? ASTRO_STAGE_WINDOWS_MANY : ASTRO_STAGE_WINDOWS, PL>& t, const unsigned lane,
                                           const unsigned tile_index, const TileIn& in, TileIn& next, const bool last,
                                           unsigned& stat_acc, const bool have_fire_word) {
     using B4 = Body4<float>;
@@ -421,7 +441,7 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
     const size_t tile = (size_t)tile_index;
     float4* ships = reinterpret_cast<float4*>(p.ships) + tile * (S * 32) + lane;
     float* ship_b = reinterpret_cast<float*>(p.ship_b) + tile * (S * 32) + lane;
-    float4* planets = reinterpret_cast<float4*>(p.planets) + tile * (ASTRO_MAX_PLANETS * 32) + lane;
+    float4* planets = reinterpret_cast<float4*>(p.planets) + tile * (PL * 32) + lane;
     // The tile's bullet list: a dense run of capacity 32 K in the buffer being read, rewritten dense
     // into the same run of the other buffer.  32-bit indexing (astro_batch_create checks
     // n_games * K < 2^31): one IMAD.WIDE per address.
@@ -462,11 +482,11 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
     const bool auto_reset = FIX || ((p.flags & ASTRO_TICK_AUTO_RESET) && (p.pool_size > 0 || p.ring != nullptr));
     const bool active = !ASTRO_META_FINISHED(meta);
     const int nb = active ? (int)ASTRO_META_NB(meta) : 0;
-    const int np = active ? (int)ASTRO_META_NP(meta) : 0;
-    const uint32_t tick = ASTRO_META_TICK(meta);
-    float4 plv[ASTRO_MAX_PLANETS];
+    const int np = active ? (int)meta_np<PL>(meta) : 0;
+    const uint32_t tick = meta_tick<PL>(meta);
+    float4 plv[PL];
 #pragma unroll
-    for (int j = 0; j < ASTRO_MAX_PLANETS; j++) {
+    for (int j = 0; j < PL; j++) {
         plv[j] = make_float4(kFar, kFar, 0.f, 0.f);
         if (j < np) plv[j] = LD_STREAM(&planets[j * 32]);
     }
@@ -476,16 +496,16 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
         // (script_decide: script.py:67-91, each ship from its own perspective) or script.NothingBot (control 2) per ship —
         // so that scripted games need no launch between ticks and run many ticks per launch like the counter-stream ones.
         if (active) {
-            Body4<float> pl4[ASTRO_MAX_PLANETS];
+            Body4<float> pl4[PL];
 #pragma unroll
-            for (int j = 0; j < ASTRO_MAX_PLANETS; j++) { pl4[j].x = plv[j].x; pl4[j].y = plv[j].y; pl4[j].dx = plv[j].z; pl4[j].dy = plv[j].w; }
+            for (int j = 0; j < PL; j++) { pl4[j].x = plv[j].x; pl4[j].y = plv[j].y; pl4[j].dx = plv[j].z; pl4[j].dy = plv[j].w; }
 #pragma unroll
             for (int s = 0; s < S; s++) {
                 if (((p.bot_modes >> (4 * s)) & 15) == ASTRO_BOT_SCRIPT) {
                     Body4<float> me, en;
                     me.x = shv[s].x; me.y = shv[s].y; me.dx = shv[s].z; me.dy = shv[s].w;
                     en.x = shv[S - 1 - s].x; en.y = shv[S - 1 - s].y; en.dx = shv[S - 1 - s].z; en.dy = shv[S - 1 - s].w;
-                    ctl[s] = script_decide<float, S>(me, sb[s], en, pl4, np, p.script);
+                    ctl[s] = script_decide<float, S, PL>(me, sb[s], en, pl4, np, p.script);
                 }
             }
         }
@@ -501,7 +521,7 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
     const bool nonempty = nb > 0;
     const unsigned ne = __ballot_sync(full, nonempty);
     const unsigned cid = __popc(ne & lt_mask);                    // this game's rank among the games with bullets
-    using Scratch = TileScratchT<kStageWindows>;
+    using Scratch = TileScratchT<kStageWindows, PL>;
 #if ASTRO_SMEM_ASM
     // every hot shared-memory access of the tick goes off this one base register (see lds128 above)
     const unsigned sbase = __shfl_sync(full, (unsigned)__cvta_generic_to_shared(&t), 0);
@@ -577,16 +597,17 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
     sts128(SOFF(svel) + lane * 16u, make_float4(shv[0].z, shv[0].w, shv[1].z, shv[1].w));
     if (nonempty) {
         sts128(SOFF(fsxy) + cid * 16u, make_float4(shv[0].x, shv[1].x, shv[0].y, shv[1].y));
-        sts128(SOFF(fpxy) + cid * 16u, make_float4(plv[0].x, plv[1].x, plv[0].y, plv[1].y));
-        sts128(SOFF(fpxy) + 512u + cid * 16u, make_float4(plv[2].x, plv[3].x, plv[2].y, plv[3].y));
+#pragma unroll
+        for (int k = 0; k < PL / 2; k++)
+            sts128(SOFF(fpxy) + (unsigned)k * 512u + cid * 16u, make_float4(plv[2 * k].x, plv[2 * k + 1].x, plv[2 * k].y, plv[2 * k + 1].y));
     }
 #else
     t.sxy[lane] = make_float4(shv[0].x, shv[1].x, shv[0].y, shv[1].y);
     t.svel[lane] = make_float4(shv[0].z, shv[0].w, shv[1].z, shv[1].w);
     if (nonempty) {
         t.fsxy[cid] = make_float4(shv[0].x, shv[1].x, shv[0].y, shv[1].y);
-        t.fpxy[0][cid] = make_float4(plv[0].x, plv[1].x, plv[0].y, plv[1].y);
-        t.fpxy[1][cid] = make_float4(plv[2].x, plv[3].x, plv[2].y, plv[3].y);
+#pragma unroll
+        for (int k = 0; k < PL / 2; k++) t.fpxy[k][cid] = make_float4(plv[2 * k].x, plv[2 * k + 1].x, plv[2 * k].y, plv[2 * k + 1].y);
     }
 #endif
 #ifdef ASTRO_TIMELINE
@@ -607,16 +628,16 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
             ST_STREAM(&ship_b[s * 32], sb[s]);
         }
 #pragma unroll
-        for (int i = 0; i < ASTRO_MAX_PLANETS; i++)
+        for (int i = 0; i < PL; i++)
             if (i < np) ST_STREAM(&planets[i * 32], plv[i]);
     }
     if (active && !freeze) {
 #else
     if (active) {
 #endif
-        f32x2 pxy[ASTRO_MAX_PLANETS];
+        f32x2 pxy[PL];
 #pragma unroll
-        for (int j = 0; j < ASTRO_MAX_PLANETS; j++) pxy[j] = pk2(plv[j].x, plv[j].y);
+        for (int j = 0; j < PL; j++) pxy[j] = pk2(plv[j].x, plv[j].y);
         float dirs[4];
         if (S == 2) np_sincos_f32x2(sb[0], sb[1], dirs[0], dirs[1], dirs[2], dirs[3]);
         else { np_sincos_f32(sb[0], dirs[0], dirs[1]); dirs[2] = dirs[0]; dirs[3] = dirs[1]; }
@@ -632,12 +653,12 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
             f32x2 acc = bc2(0.0f);
             float dmin = 3.0e38f;
 #pragma unroll
-            for (int j = 0; j < ASTRO_MAX_PLANETS; j++) dmin = fminf(dmin, grav_pair(pxy[j], sxy, acc, c));
+            for (int j = 0; j < PL; j++) dmin = fminf(dmin, grav_pair(pxy[j], sxy, acc, c));
             bool h = dmin < c.r2f_sp;
             if (__builtin_expect(fabsf(dmin - c.r2f_sp) <= c.r2f_sp * 1e-6f, 0)) {
                 h = false;
 #pragma unroll
-                for (int j = 0; j < ASTRO_MAX_PLANETS; j++)
+                for (int j = 0; j < PL; j++)
                     if (j < np)
                         h |= collide_exact((double)shv[s].x, (double)shv[s].y, (double)plv[j].x, (double)plv[j].y, c.r2_sp);
             }
@@ -655,13 +676,13 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
             if (collide(shv[0].x, shv[0].y, shv[1].x, shv[1].y, c.r2_ss, c.r2f_ss)) hits |= 3u;
         }
         // planets (core.py:289-294): pair forces are antisymmetric, the clamped self term is zero
-        f32x2 q[ASTRO_MAX_PLANETS];
+        f32x2 q[PL];
 #pragma unroll
-        for (int i = 0; i < ASTRO_MAX_PLANETS; i++) q[i] = bc2(0.0f);
+        for (int i = 0; i < PL; i++) q[i] = bc2(0.0f);
 #pragma unroll
-        for (int i = 0; i < ASTRO_MAX_PLANETS; i++) {
+        for (int i = 0; i < PL; i++) {
 #pragma unroll
-            for (int j = i + 1; j < ASTRO_MAX_PLANETS; j++) {
+            for (int j = i + 1; j < PL; j++) {
                 const f32x2 e = sub2(pxy[j], pxy[i]);
                 float s0, s1;
                 upk2(mul2(e, e), s0, s1);
@@ -671,7 +692,7 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
             }
         }
 #pragma unroll
-        for (int i = 0; i < ASTRO_MAX_PLANETS; i++)
+        for (int i = 0; i < PL; i++)
             if (i < np) ST_STREAM(&planets[i * 32], advance_body2(pxy[i], pk2(plv[i].z, plv[i].w), q[i], c));
     }
 
@@ -681,7 +702,9 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
     if (auto_reset && active && (hits || tick >= (uint32_t)p.timeout_tick)) {
         if (!has_ring) {
             const uint32_t k = pool_pick(p.seed, p.first_game + (uint32_t)g, v.step + step_base + 1u, (uint32_t)p.pool_size);
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(p.pool_rec + (size_t)k * 8));
+            const float4* const r = p.pool_rec + (size_t)k * pool_rec_float4s<PL>();
+            asm volatile("prefetch.global.L2 [%0];" ::"l"(r));
+            if (PL > ASTRO_MAX_PLANETS) asm volatile("prefetch.global.L2 [%0];" ::"l"(r + 8));   // (a 256-byte record: two lines)
         } else {
             // fresh-game mode: which record the game will get depends on who else ends this tick; the tile's next
             // record is the likely one
@@ -727,17 +750,22 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
 #if ASTRO_SMEM_ASM
                 float4 bv = lds128(bul_s + w * 512u);
                 const unsigned fr = sbase + gi * 16u;
-                const float4 sT = lds128(fr + (unsigned)offsetof(Scratch, fsxy)), pA = lds128(fr + (unsigned)offsetof(Scratch, fpxy)),
-                             pB = lds128(fr + (unsigned)offsetof(Scratch, fpxy) + 512u);
+                const float4 sT = lds128(fr + (unsigned)offsetof(Scratch, fsxy));
+                float4 pT[PL / 2];
+#pragma unroll
+                for (int k = 0; k < PL / 2; k++) pT[k] = lds128(fr + (unsigned)offsetof(Scratch, fpxy) + (unsigned)k * 512u);
 #else
                 float4 bv = t.bul[w * 32u + lane];
-                const float4 sT = t.fsxy[gi], pA = t.fpxy[0][gi], pB = t.fpxy[1][gi];
+                const float4 sT = t.fsxy[gi];
+                float4 pT[PL / 2];
+#pragma unroll
+                for (int k = 0; k < PL / 2; k++) pT[k] = t.fpxy[k][gi];
 #endif
                 unsigned sh_hits = 0;
 #ifdef ASTRO_EXPERIMENTS
-                const bool keep = freeze ? (bv.x + sT.x + pA.x + pB.x != 123456.0f) : bullet_step_t<S>(bv, sT, pA, pB, t.hits, gi, c, sh_hits);
+                const bool keep = freeze ? (bv.x + sT.x + pT[0].x + pT[1].x != 123456.0f) : bullet_step_t<S, PL>(bv, sT, pT, t.hits, gi, c, sh_hits);
 #else
-                const bool keep = bullet_step_t<S>(bv, sT, pA, pB, t.hits, gi, c, sh_hits);
+                const bool keep = bullet_step_t<S, PL>(bv, sT, pT, t.hits, gi, c, sh_hits);
 #endif
                 if (sh_hits) atomicOr(&t.hits[gi], sh_hits);
                 const unsigned kb = __ballot_sync(full, keep);   // (every lane has loaded its window item by now)
@@ -866,7 +894,7 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
                 }
                 spawned = S;
             }
-            next.meta = ASTRO_META_PACK(m, np, 0, tick + 1);
+            next.meta = meta_pack<PL>(m, np, 0, tick + 1);
             if (last) ST_STREAM(&p.meta[g], next.meta);
             m_out = m;
         }
@@ -876,13 +904,13 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
     const bool ended = (ev & ASTRO_EV_DONE_MASK) != 0;       // (a skipped game: no)
     if (auto_reset) {
         // Where the new game comes from (core.create, core.py:86-135): a 128-byte record — ships (5 floats each), planet
-        // count (word 10), planets (floats 16..31) — of the reset pool, picked by a hash of (game, stream step); or, in
+        // count (word 10), planets (floats 16..31; 8-slot batches: 256 bytes, floats 16..47) — of the reset pool, picked by a hash of (game, stream step); or, in
         // fresh-game mode, the tile's next unused record of its ring (words 11 / 12: position in the generate_configs
         // stream, seed): a warp-local count, so every record — every stream position — is consumed exactly once.  A game
         // that finds the tile's ring empty waits, frozen (tick field = ASTRO_MAX_TICKS), and asks again every tick.
         const float4* rec = nullptr;
         if (has_ring) {
-            const bool want = ended | (!active && ASTRO_META_TICK(meta) == (uint32_t)ASTRO_MAX_TICKS);
+            const bool want = ended | (!active && meta_tick<PL>(meta) == max_ticks<PL>());
             const unsigned wants = __ballot_sync(full, want);
             if (wants) {
                 const unsigned used = t.used;
@@ -892,13 +920,13 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
                 if (want && idx < (unsigned)p.quota) rec = p.ring + ((size_t)tile_index * (unsigned)p.quota + idx) * 8;
             }
         } else if (ended) {
-            rec = p.pool_rec + (size_t)pool_pick(p.seed, p.first_game + (uint32_t)g, v.step + step_base + 1u, (uint32_t)p.pool_size) * 8;
+            rec = p.pool_rec + (size_t)pool_pick(p.seed, p.first_game + (uint32_t)g, v.step + step_base + 1u, (uint32_t)p.pool_size) * pool_rec_float4s<PL>();
         }
         if (ended) atomicAdd(&p.episode[g], 1u);      // the per-slot episode counter: a fire-and-forget RED
         if (rec) {
-            float4 r[8];
+            float4 r[4 + PL];
 #pragma unroll
-            for (int j = 0; j < 8; j++) r[j] = __ldg(&rec[j]);
+            for (int j = 0; j < 4 + PL; j++) r[j] = __ldg(&rec[j]);
             const int np_new = __float_as_int(r[2].z);
             next.shv[0] = r[0];
             next.sb[0] = r[1].x;
@@ -915,14 +943,14 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
                 }
             }
 #pragma unroll
-            for (int j = 0; j < ASTRO_MAX_PLANETS; j++)
+            for (int j = 0; j < PL; j++)
                 if (j < np_new) planets[j * 32] = r[4 + j];
-            next.meta = ASTRO_META_PACK(0, np_new, 0, 0);
+            next.meta = meta_pack<PL>(0, np_new, 0, 0);
             if (last) p.meta[g] = next.meta;
             if (!FIX && p.game_pos) p.game_pos[g] = __float_as_uint(r[2].w);
         } else if (ended) {
             ev |= ASTRO_EV_AWAIT;
-            next.meta = ASTRO_META_PACK(0, np, 1, ASTRO_MAX_TICKS);
+            next.meta = meta_pack<PL>(0, np, 1, max_ticks<PL>());
             p.meta[g] = next.meta;
         }
     } else if (ended) {
@@ -930,7 +958,7 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
         // so the finished word goes to memory now, whichever tick of the launch this is (the ships were
         // stored by the physics above: without auto-reset every tick stores them) — identical to
         // separate astro_tick calls.
-        next.meta = ASTRO_META_PACK(0, np, 1, tick);
+        next.meta = meta_pack<PL>(0, np, 1, tick);
         p.meta[g] = next.meta;
     }
 
@@ -1031,7 +1059,8 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
 // (BOT: the instantiation with the ScriptBot inside — float64 arithmetic of its own, far more registers: fewer CTAs per SM)
 template <int S, bool STATS, bool MANY, bool BOT = false, bool FIX = false>
 __global__ void __launch_bounds__(kTickThreads, BOT ? ASTRO_TICK_MIN_BLOCKS_BOT : (MANY ? ASTRO_TICK_MIN_BLOCKS_MANY : ASTRO_TICK_MIN_BLOCKS)) tick_f32_kernel(const __grid_constant__ TickParams p) {
-    using TileScratch = TileScratchT<MANY ? ASTRO_STAGE_WINDOWS_MANY : ASTRO_STAGE_WINDOWS>;
+    constexpr int PL = ASTRO_MAX_PLANETS;
+    using TileScratch = TileScratchT<MANY ? ASTRO_STAGE_WINDOWS_MANY : ASTRO_STAGE_WINDOWS, PL>;
     __shared__ TileScratch s_tiles[kTickWarps];
     unsigned tile = (blockIdx.x * kTickThreads + threadIdx.x) >> 5;   // among the p.tiles tiles of this launch, from p.tile0
 #if ASTRO_PDL
@@ -1073,7 +1102,7 @@ __global__ void __launch_bounds__(kTickThreads, BOT ? ASTRO_TICK_MIN_BLOCKS_BOT 
     unsigned used0 = 0;
     const bool has_ring = !FIX && p.ring != nullptr;
     if (has_ring && lane == 0) used0 = p.tile_used[tile];
-    load_tile_in<S, FIX>(p, tick_var<S>(p, 0u), tile, lane, in);
+    load_tile_in<S, PL, FIX>(p, tick_var<S>(p, 0u), tile, lane, in);
     if (has_ring && lane == 0) scratch.used = used0;
 #pragma unroll 1
     for (unsigned k = 0; k < (MANY ? (unsigned)p.n_fused : 1u); k++) {
@@ -1085,9 +1114,9 @@ __global__ void __launch_bounds__(kTickThreads, BOT ? ASTRO_TICK_MIN_BLOCKS_BOT 
             const size_t g = (size_t)tile * 32 + lane;
             ctl_next = load_controls<S>(v.actions + p.act_stride, g, FIX || (p.flags & ASTRO_TICK_PACKED_CONTROLS) != 0);
         }
-        if (MANY) in.fire_word = p.fire_bits[min(ASTRO_META_TICK(in.meta), (uint32_t)p.n_sched_ticks - 1u) >> 5];
+        if (MANY) in.fire_word = p.fire_bits[min(meta_tick<PL>(in.meta), (uint32_t)p.n_sched_ticks - 1u) >> 5];
         // (one-warp CTAs: the scratch is s_tiles[0], every shared address a compile-time constant — no base register)
-        tick_tile<S, STATS, MANY, BOT, FIX>(p, v, scratch, lane, tile, in, next, !MANY || k + 1u == (unsigned)p.n_fused, stat_acc, MANY);
+        tick_tile<S, STATS, MANY, BOT, FIX, PL>(p, v, scratch, lane, tile, in, next, !MANY || k + 1u == (unsigned)p.n_fused, stat_acc, MANY);
         if (MANY) {
             // The next tick of this tile: meta, ships and bearings are handed on in registers (they were stored as
             // well), so it starts its prefix sums and list requests at once; only the planet rows are loaded.  The
@@ -1103,4 +1132,87 @@ __global__ void __launch_bounds__(kTickThreads, BOT ? ASTRO_TICK_MIN_BLOCKS_BOT 
         __syncwarp();
         if (lane == 0) p.tile_used[tile] = scratch.used;
     }
+}
+
+// The same shell for 8 planet slots, generic options only (no BOT / FIX forms): a kernel of its own name, so that the
+// 4-slot kernels above are compiled exactly as before.
+template <int S, bool STATS, bool MANY, bool BOT, bool FIX, int PL>
+__device__ __forceinline__ void tick_f32_body(const TickParams& p) {
+    using TileScratch = TileScratchT<MANY ? ASTRO_STAGE_WINDOWS_MANY : ASTRO_STAGE_WINDOWS, PL>;
+    __shared__ TileScratch s_tiles[kTickWarps];
+    unsigned tile = (blockIdx.x * kTickThreads + threadIdx.x) >> 5;   // among the p.tiles tiles of this launch, from p.tile0
+#if ASTRO_PDL
+    if (!MANY) {
+        asm volatile("griddepcontrol.launch_dependents;" ::: "memory");   // the next kernel's CTAs may take the slots this grid frees
+        asm volatile("griddepcontrol.wait;" ::: "memory");                // ... and the previous kernel's stores are visible from here
+    }
+#endif
+    if (tile >= (unsigned)p.tiles) return;  // whole warps: n_games % 32 == 0
+#if ASTRO_BOUSTROPHEDON
+    // Odd launches walk the tiles backwards: what the previous launch wrote last — still in the 126 MB L2 —
+    // is read first, and rewritten there before it ever went to HBM.
+    if ((!MANY || ASTRO_OPAQUE_TILE) && (p.step & 1u)) tile = (unsigned)p.tiles - 1u - tile;
+#endif
+    tile += (unsigned)p.tile0;
+#if ASTRO_OPAQUE_TILE
+    // A launch of several ticks: ptxas re-derives the tile index from %ctaid every tick (five instructions) rather than keep
+    // it; the result of a shuffle it has to keep.  (A/B at 20 ticks per launch: 52.7 -> 50.8 us per tick together with the
+    // cheaper statistics; without the backwards walk at all: 51.7.)
+    if (MANY) tile = __shfl_sync(0xffffffffu, tile, 0);
+#endif
+#if ASTRO_OPAQUE_LANE
+    // (several ticks per launch: ptxas re-reads %tid.x a dozen times per tick instead of keeping the lane id; a value that came
+    // through a shuffle it keeps)
+    const unsigned lane = MANY ? __shfl_sync(0xffffffffu, threadIdx.x & 31u, threadIdx.x & 31u) : (threadIdx.x & 31u);
+#else
+    const unsigned lane = threadIdx.x & 31u;
+#endif
+    // n_fused consecutive ticks of this tile, back to back (astro_tick_many): games do not interact, so a
+    // tile can run ahead of the others; what tick k wrote is what tick k + 1 reads — from L2, not from HBM.
+    // The rows are lane-private; the bullet list is written by some lanes and read by others: the warp
+    // barrier orders those accesses.
+    // (MANY = false: the one-tick launch, without the loop around it — the loop form costs a single tick 6 %)
+    TileIn in, next;
+    unsigned stat_acc = 0;
+    TileScratch& scratch = s_tiles[kTickWarps == 1 ? 0 : (threadIdx.x >> 5)];
+    // fresh-game mode: how many of the tile's pre-created games have been used since the last refill — requested with the
+    // tile's rows, parked in shared memory once they are all on their way (a wait here would cost a round trip)
+    unsigned used0 = 0;
+    const bool has_ring = !FIX && p.ring != nullptr;
+    if (has_ring && lane == 0) used0 = p.tile_used[tile];
+    load_tile_in<S, PL, FIX>(p, tick_var<S>(p, 0u), tile, lane, in);
+    if (has_ring && lane == 0) scratch.used = used0;
+#pragma unroll 1
+    for (unsigned k = 0; k < (MANY ? (unsigned)p.n_fused : 1u); k++) {
+        const TickVar v = tick_var<S>(p, MANY ? k : 0u);
+        // (several ticks per launch) the NEXT tick's controls are requested now — a different array every tick,
+        // straight from HBM — so that they have arrived when this tick is done
+        uint32_t ctl_next = 0;
+        if (MANY && (FIX || p.actions) && k + 1u < (unsigned)p.n_fused) {
+            const size_t g = (size_t)tile * 32 + lane;
+            ctl_next = load_controls<S>(v.actions + p.act_stride, g, FIX || (p.flags & ASTRO_TICK_PACKED_CONTROLS) != 0);
+        }
+        if (MANY) in.fire_word = p.fire_bits[min(meta_tick<PL>(in.meta), (uint32_t)p.n_sched_ticks - 1u) >> 5];
+        // (one-warp CTAs: the scratch is s_tiles[0], every shared address a compile-time constant — no base register)
+        tick_tile<S, STATS, MANY, BOT, FIX, PL>(p, v, scratch, lane, tile, in, next, !MANY || k + 1u == (unsigned)p.n_fused, stat_acc, MANY);
+        if (MANY) {
+            // The next tick of this tile: meta, ships and bearings are handed on in registers (they were stored as
+            // well), so it starts its prefix sums and list requests at once; only the planet rows are loaded.  The
+            // warp barrier orders this tick's list stores before the next tick's requests (no fence: a fence would
+            // hold the warp until its last stores are acknowledged).
+            in = next;
+            in.ctl_raw = ctl_next;
+            if (S == 1) { in.shv[1] = in.shv[0]; in.sb[1] = in.sb[0]; }
+            __syncwarp();
+        }
+    }
+    if (has_ring) {
+        __syncwarp();
+        if (lane == 0) p.tile_used[tile] = scratch.used;
+    }
+}
+
+template <int S, bool STATS, bool MANY>
+__global__ void __launch_bounds__(kTickThreads, MANY ? ASTRO_TICK_MIN_BLOCKS_WIDE_MANY : ASTRO_TICK_MIN_BLOCKS_WIDE) tick_f32_wide_kernel(const __grid_constant__ TickParams p) {
+    tick_f32_body<S, STATS, MANY, false, false, ASTRO_MAX_PLANETS_WIDE>(p);
 }

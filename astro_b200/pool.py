@@ -8,11 +8,14 @@ import numpy as np
 from . import core
 
 
-def make_pool(config, size):
-    """`size` initial states -> dict(ships [M,S,5] = x,y,dx,dy,b ; planets [M,4,4] ; np [M])."""
+def make_pool(config, size, planet_slots=None):
+    """`size` initial states -> dict(ships [M,S,5] = x,y,dx,dy,b ; planets [M,PL,4] ; np [M]), PL = planet_slots
+    (default: batched.planet_slots_for(config), 4 or 8)."""
+    from .batched import planet_slots_for
     S = 1 if config.solo else 2
+    PL = planet_slots_for(config) if planet_slots is None else int(planet_slots)
     ships = np.zeros((size, S, 5))
-    planets = np.zeros((size, 4, 4))
+    planets = np.zeros((size, PL, 4))
     n_planets = np.zeros(size, dtype=np.int32)
     for i, c in enumerate(it.islice(core.generate_configs(config), size)):
         s = core.create(c)

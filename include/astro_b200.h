@@ -22,7 +22,8 @@
  * games (one warp).  R is float (precision 32) or double (precision 64); R4 = {x, y, dx, dy}.
  *     ships    R4  [n_tiles][S][32]      ship s of game g  -> ((g/32)*S + s)*32 + g%32
  *     ship_b   R   [n_tiles][S][32]      bearing
- *     planets  R4  [n_tiles][4][32]      slots >= np are dead
+ *     planets  R4  [n_tiles][PL][32]     slots >= np are dead; PL = the batch's planet slots (4, or 8 for
+ *                                        AstroConfig.planet_slots = 8: games of up to eight planets)
  *     bullets  R4  [2][n_tiles][32*K]    TILE LISTS, two buffers.  In the current buffer
  *                                        (astro_bullet_buffer()) tile t's run holds the bullets of its
  *                                        32 games back to back, no gaps: game g's bullets are items
@@ -32,6 +33,7 @@
  *                                        dead.  Every astro_tick reads the current buffer, writes
  *                                        the tile's new list into the other one and flips.
  *     meta     u32 [n_tiles*32]          nb (bits 0-9) | np (10-12) | finished (13) | tick (14-31)
+ *                                        8-slot batches: np bit 3 in bit 31, tick in bits 14-30 (ASTRO_META_*_WIDE)
  *     episode  u32 [n_tiles*32]          games finished in this slot (a counter; bumped on reset)
  * Ships, planets and meta are accessed thread-per-game: every load/store is a fully coalesced
  * 128-bit (R=float) access across the warp.  A tile's bullets are one contiguous run in HBM (3 KB
@@ -47,12 +49,14 @@
 extern "C" {
 #endif
 
-#define ASTRO_ABI_VERSION 4   /* 4: astro_stats_peer_*, astro_stats_allreduce, astro_value_forward */
+#define ASTRO_ABI_VERSION 5   /* 5: AstroConfig.planet_slots, AstroSingleGame.planets[ASTRO_MAX_PLANETS_WIDE] */
 #define ASTRO_TILE 32
 #define ASTRO_MAX_SHIPS 2
 #define ASTRO_MAX_PLANETS 4
+#define ASTRO_MAX_PLANETS_WIDE 8 /* AstroConfig.planet_slots = 8 */
 #define ASTRO_MAX_BULLET_CAP 1023
 #define ASTRO_MAX_TICKS 262143 /* 18-bit per-game tick counter */
+#define ASTRO_MAX_TICKS_WIDE 131071 /* 17 bits in 8-slot batches */
 
 /* meta word */
 #define ASTRO_META_NB(m) ((m) & 1023u)
@@ -61,6 +65,13 @@ extern "C" {
 #define ASTRO_META_TICK(m) ((m) >> 14)
 #define ASTRO_META_PACK(nb, np, fin, tick) \
     ((uint32_t)(nb) | ((uint32_t)(np) << 10) | ((uint32_t)(fin) << 13) | ((uint32_t)(tick) << 14))
+/* meta word of an 8-slot batch: np = 8 needs a fourth bit, which sits in bit 31; nb, the low three bits of np and the
+ * finished bit stay where they are, and so does the tick's lowest bit (a tick still advances by + (1 << 14)) */
+#define ASTRO_META_NP_WIDE(m) ((((m) >> 10) & 7u) | (((m) >> 28) & 8u))
+#define ASTRO_META_TICK_WIDE(m) (((m) >> 14) & 0x1ffffu)
+#define ASTRO_META_PACK_WIDE(nb, np, fin, tick)                                                                    \
+    ((uint32_t)(nb) | (((uint32_t)(np) & 7u) << 10) | ((uint32_t)(fin) << 13) | ((uint32_t)(tick) << 14) |      \
+     (((uint32_t)(np) & 8u) << 28))
 
 /* per-game event bits written by astro_tick (u8 per game) */
 #define ASTRO_EV_HIT0 1      /* ship 0 collided   (core.py:253-255) */
@@ -109,7 +120,9 @@ typedef struct AstroConfig {
     double gravity, dt, max_time, reload_time, bullet_speed, ship_thrust, ship_rspeed, ship_radius,
         planet_mass, planet_radius;
     int32_t solo; /* 1 -> one ship per game */
-    int32_t reserved;
+    int32_t planet_slots; /* planet slots per game: 0 or 4 (ASTRO_MAX_PLANETS), or 8 (ASTRO_MAX_PLANETS_WIDE) for games of
+                             up to eight planets.  The game-major arrays of the batch (AstroResetPool, astro_create_games,
+                             AstroGameArrays) then hold that many planet rows per game. */
 } AstroConfig;
 
 /* Device pointers of the caller-owned state (layout above; bullets = both buffers, contiguous). */
@@ -123,7 +136,7 @@ typedef struct AstroBuffers {
 } AstroBuffers;
 
 /* Reset pool: M initial states built by create() (core.py:86-135) on the host, in device
- * memory, game-major: ships R [M][S][5] = x,y,dx,dy,b ; planets R [M][4][4] ; np i32 [M]. */
+ * memory, game-major: ships R [M][S][5] = x,y,dx,dy,b ; planets R [M][PL][4] ; np i32 [M]. */
 typedef struct AstroResetPool {
     const void* ships;
     const void* planets;
@@ -175,8 +188,8 @@ int astro_set_schedule(AstroBatch* b, const uint32_t* fire_bits_host, int32_t n_
 
 /* Counter-stream keys (astro_b200/rng.py): controls when actions == NULL, reset-pool picks. */
 int astro_set_stream(AstroBatch* b, uint32_t seed, int64_t first_game, uint32_t step);
-/* The pool is SNAPSHOT by this call (precision 32: repacked into one 128-byte record per entry, which the
- * tick kernel reads); call it again after changing the pool's contents.  Synchronises the device. */
+/* The pool is SNAPSHOT by this call (precision 32: repacked into one 128-byte record per entry — 256 bytes in 8-slot
+ * batches — which the tick kernel reads); call it again after changing the pool's contents.  Synchronises the device. */
 int astro_set_reset_pool(AstroBatch* b, const AstroResetPool* pool);
 
 /* core.step (core.py:215-303) for every game of the batch: one fused kernel.
@@ -229,7 +242,7 @@ int astro_reset_done(AstroBatch* b, void* stream);
 
 /* rl.ValueNetwork.get_features + to_batch (rl.py:43-99) with core.roll_ships (core.py:306-327)
  * for both perspectives: obs f32 [n_games][S][n_rows][1+5S+4] device; rows = planets then
- * bullets, the rest filled with -1; n_rows >= 4 + bullet_cap.  Finished games: all -1. */
+ * bullets, the rest filled with -1; n_rows >= PL + bullet_cap.  Finished games: all -1. */
 int astro_observe(AstroBatch* b, float* obs, int32_t n_rows, void* stream);
 
 /* The same features written ONCE: obs f32 [n_games][n_rows][1+5S+4], ship 0's perspective only.
@@ -244,8 +257,8 @@ int astro_observe_shared(AstroBatch* b, float* obs, int32_t n_rows, void* stream
  * legacy randint / rand / choice draws in the reference's order) and the reference's float32 /
  * float64 arithmetic, bit for bit.  seeds u32 [m] device (core.generate_configs, core.py:77-83, is
  * RandomState(config.seed).randint(2**30) per game: astro_b200/rng.py config_seeds).  Output in
- * the AstroResetPool layout, batch precision R: ships R [m][S][5], planets R [m][4][4] (dead slots
- * zero), n_planets i32 [m] — pass it to astro_set_reset_pool, or refresh it between rollouts so
+ * the AstroResetPool layout, batch precision R: ships R [m][S][5], planets R [m][PL][4] (dead slots
+ * zero), max_planets <= PL, n_planets i32 [m] — pass it to astro_set_reset_pool, or refresh it between rollouts so
  * that re-created games never repeat. */
 int astro_create_games(AstroBatch* b, const AstroCreateConfig* cc, const uint32_t* seeds, int32_t m, void* ships,
                        void* planets, int32_t* n_planets, void* stream);
@@ -329,7 +342,7 @@ int astro_rollout_device(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, int
 
 /* Game-major float64 view of games, the layout host-side code wants (State conversion for the drop-in core.step /
  * core.play, core.py:11-18 and :377-410; JSONL logs, core.py:413-443): row i describes one game.  DEVICE pointers.
- *   ships R [m][S][5] = x, y, dx, dy, b    planets [m][4][4] (dead slots zero)    bullets [m][k][4] (dead slots zero)
+ *   ships R [m][S][5] = x, y, dx, dy, b    planets [m][PL][4] (dead slots zero)    bullets [m][k][4] (dead slots zero)
  *   n_planets / n_bullets / tick i32 [m]   finished u8 [m]   episode u32 [m] (may be NULL) */
 typedef struct AstroGameArrays {
     double* ships;
@@ -362,7 +375,7 @@ int astro_import_games(AstroBatch* b, const int32_t* index, int32_t m, const Ast
  *   out: the new state (tick + 1), events[0] = ASTRO_EV_* of the tick, finished = 1 when the game ended */
 typedef struct AstroSingleGame {
     double ships[ASTRO_MAX_SHIPS][5];
-    double planets[ASTRO_MAX_PLANETS][4];
+    double planets[ASTRO_MAX_PLANETS_WIDE][4]; /* rows >= the batch's planet slots are ignored */
     int32_t n_planets, n_bullets, tick, reserved;
     uint32_t episode;
     uint8_t finished[4];
