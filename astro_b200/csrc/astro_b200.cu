@@ -1080,238 +1080,38 @@ __global__ void __launch_bounds__(64) fresh_fill_kernel(const __grid_constant__ 
 __global__ void fresh_fill_commit_kernel(const __grid_constant__ FreshParams f) { f.cursor[0] += (unsigned)f.n_games; }
 
 // ------------------------------------------------------------------------------------------
-// policy_kernel<R, S>: rl.ValueNetwork.forward (rl.py:140-165) on the features of rl.py:43-72,
-// fused — the observation tensor never exists.  For every game and both perspectives
-// (core.roll_ships): per live object row  h = f0(x); h = f[i](softsign(h)) x2 ; max over the rows ;
-// h = softsign(v[i](h)) x2 ; q = tanh(v0(h)) ; control = argmax q  (the greedy policy of
-// rl.QBot, rl.py:168-200).
-//
-// WARP = one game, BOTH perspectives at once; LANE = UNIT of the 32-wide layers, its rows of the
-// three per-object layers (15 + 32 + 32 weights) held in registers for the whole kernel.  The warp
-// walks the game's live rows (planets then bullets; 7.8 per game on average against 36 padded — no
-// padding work).  The two perspectives see the same objects and differ only in the order of the
-// ship columns, so the ship part of f0 is computed once per game and perspective, the object part
-// once per row for both; a row then costs 5 + 2 x (32 + 32) FMAs per lane, as two independent
-// chains.  Activations cross lanes through a 128-byte shared buffer per chain, read back as
-// broadcast LDS.128; the max-pool over rows is a register per lane — no atomics, no block barrier.
-// The head runs on the same lanes with its weights streamed from a transposed copy (coalesced,
-// L1-resident).  fp32 FMA arithmetic (CUDA cores): agrees with the PyTorch fp32 network to ~1e-6;
-// tensor-core formats (tf32 / bf16) would flip near-tied argmaxes.
+// rl.ValueNetwork (rl.py:140-165): 32-wide layers, at most kPolMaxOut outputs
 // ------------------------------------------------------------------------------------------
 constexpr int kPolW = 32;           // layer width (rl.py:144)
 constexpr int kPolMaxOut = 8;
-constexpr int kPolWarps = 4;
-constexpr int kPolGamesPerWarp = 2; // at least this many games per warp: the lane's 79 weights are loaded once for all of them
-struct PolicyWeights {              // every matrix TRANSPOSED, [in][out]: lane = unit reads it coalesced
-    float f0t[15][kPolW], f0b[kPolW];
-    float f1t[kPolW][kPolW], f1b[kPolW];
-    float f2t[kPolW][kPolW], f2b[kPolW];
-    float v1t[kPolW][kPolW], v1b[kPolW];
-    float v2t[kPolW][kPolW], v2b[kPolW];
-    float v0t[kPolW][kPolMaxOut], v0b[kPolMaxOut];
-};
-// (the weights live in device memory owned by the batch handle: every batch has its own network)
 
 // x / (1 + |x|) with the fast reciprocal (2 ulp): the network's outputs stay within ~1e-6 of PyTorch's
 __device__ __forceinline__ float softsign(float x) { return div_fast_normal(x, 1.0f + fabsf(x)); }
 
-// One 32 -> 32 layer for two independent activation vectors held in shared memory (broadcast
-// LDS.128), this lane's weight row in registers as PAIRS (w[c], w[c+1]): each FFMA2 advances the even
-// and the odd partial sum of one chain at once — the same sums, in the same order, as two scalar
-// FMAs (each half of a packed operation rounds like the scalar one).  Returns both pre-activations
-// of the lane's unit.
-__device__ __forceinline__ void layer2(const f32x2 (&w)[kPolW / 2], float bias, const float4* xa, const float4* xb, float& ya, float& yb) {
-    f32x2 a = pk2(bias, 0.f), b = pk2(bias, 0.f);
-#pragma unroll
-    for (int c = 0; c < kPolW / 4; c++) {
-        const float4 u = xa[c], v = xb[c];
-        a = fma2(w[2 * c], pk2(u.x, u.y), a);
-        b = fma2(w[2 * c], pk2(v.x, v.y), b);
-        a = fma2(w[2 * c + 1], pk2(u.z, u.w), a);
-        b = fma2(w[2 * c + 1], pk2(v.z, v.w), b);
-    }
-    float a0, a1, b0, b1;
-    upk2(a, a0, a1);
-    upk2(b, b0, b1);
-    ya = a0 + a1;
-    yb = b0 + b1;
-}
-// The same with the weights streamed from a transposed matrix wt[in][out] (head layers).
-__device__ __forceinline__ void layer2_t(const float* __restrict__ wt, int stride, int lane, float bias, const float* xa,
-                                         const float* xb, float& ya, float& yb) {
-    f32x2 a = pk2(bias, 0.f), b = pk2(bias, 0.f);
-#pragma unroll 8
-    for (int c = 0; c < kPolW; c += 2) {
-        const f32x2 w = pk2(__ldg(wt + c * stride + lane), __ldg(wt + (c + 1) * stride + lane));
-        const float2 u = *reinterpret_cast<const float2*>(xa + c), v = *reinterpret_cast<const float2*>(xb + c);
-        a = fma2(w, pk2(u.x, u.y), a);
-        b = fma2(w, pk2(v.x, v.y), b);
-    }
-    float a0, a1, b0, b1;
-    upk2(a, a0, a1);
-    upk2(b, b0, b1);
-    ya = a0 + a1;
-    yb = b0 + b1;
-}
-
-#ifndef ASTRO_POL_MIN_BLOCKS
-#define ASTRO_POL_MIN_BLOCKS 4
-#endif
-template <typename R, int S, int PL>
-__global__ void __launch_bounds__(kPolWarps * 32, ASTRO_POL_MIN_BLOCKS)
-policy_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_, const void* __restrict__ planets_,
-              const void* __restrict__ bullets_, const uint32_t* __restrict__ meta_, uint8_t* __restrict__ actions,
-              float* __restrict__ q_out, int n_games, int K, int nout, int ship_mask, const PolicyWeights* __restrict__ pol) {
-    using B4 = Body4<R>;
-    constexpr int DIN = 1 + 5 * S + 4;
-    const PolicyWeights& g_pol = *pol;
-    __shared__ float4 s_act[kPolWarps][2][kPolW / 4];   // activation exchange, one buffer per chain
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    float* actA = reinterpret_cast<float*>(s_act[warp][0]);
-    float* actB = reinterpret_cast<float*>(s_act[warp][1]);
-    // this lane's unit: its rows of the three per-object layers
-    float w0[DIN];
-    f32x2 w1[kPolW / 2], w2[kPolW / 2];   // (w[c], w[c+1]) pairs for the packed FMAs
-#pragma unroll
-    for (int c = 0; c < DIN; c++) w0[c] = g_pol.f0t[c][lane];
-#pragma unroll
-    for (int c = 0; c < kPolW; c += 2) {
-        w1[c >> 1] = pk2(g_pol.f1t[c][lane], g_pol.f1t[c + 1][lane]);
-        w2[c >> 1] = pk2(g_pol.f2t[c][lane], g_pol.f2t[c + 1][lane]);
-    }
-    const float b0 = g_pol.f0b[lane], b1 = g_pol.f1b[lane], b2 = g_pol.f2b[lane];
-    // grid-stride over games: one resident wave of CTAs (launch side), no partial last wave
-    for (int g = blockIdx.x * kPolWarps + warp; g < n_games; g += gridDim.x * kPolWarps) {
-    const size_t tile = (size_t)(g >> 5);
-    const int gl = g & 31;
-
-    const uint32_t meta = meta_[g];
-    const bool fin = ASTRO_META_FINISHED(meta);
-    const int np = fin ? 0 : (int)meta_np<PL>(meta);
-    const int rows = fin ? 0 : np + (int)ASTRO_META_NB(meta);
-    // ship features (x, y, dx, dy, norm_angle(b) / pi), ship 0 then ship 1: lane 5 s + c holds feature c of ship s
-    float feat = 0.f;
-    if (lane < 5 * S) {
-        const int s = lane / 5, c = lane % 5;
-        if (c < 4) feat = (float)reinterpret_cast<const R*>(ships_)[((size_t)tile * (S * 32) + s * 32 + gl) * 4 + c];
-        else feat = norm_angle_over_pi((double)reinterpret_cast<const R*>(ship_b_)[(size_t)tile * (S * 32) + s * 32 + gl]);
-    }
-    // the ship columns (1 .. 5S) are the same for every row: perspective A = ship order (0, 1), B = (1, 0)
-    float baseA = b0, baseB = baseA;
-#pragma unroll
-    for (int s = 0; s < S; s++)
-#pragma unroll
-        for (int c = 0; c < 5; c++) {
-            const float f = __shfl_sync(0xffffffffu, feat, 5 * s + c);
-            baseA = __fmaf_rn(w0[1 + 5 * s + c], f, baseA);
-            baseB = __fmaf_rn(w0[1 + 5 * ((s + 1) % S) + c], f, baseB);
-        }
-    const B4* pl = reinterpret_cast<const B4*>(planets_) + tile * (PL * 32) + gl;
-    const B4* bl = reinterpret_cast<const B4*>(bullets_) + tile * (size_t)(32 * K) + tile_list_offset(meta_ + tile * 32, gl, lane);
-    // lane r fetches row r's object (coalesced for the bullets); rows beyond 32 are fetched in a second batch
-    float bestA = -3.0e38f, bestB = -3.0e38f;
-    for (int r0 = 0; r0 < rows; r0 += 32) {
-        B4 mine = B4();
-        if (r0 + lane < rows) mine = (r0 + lane < np) ? pl[(r0 + lane) * 32] : bl[r0 + lane - np];
-        const int n = min(32, rows - r0);
-        // (A/B: two rows per step as four independent chains — 82.9 us against 76.4 per 16,384 games: an odd
-        // row count repeats a row, and the kernel is bound by its 16 warps per SM, not by the chains' latency)
-        for (int r = 0; r < n; r++) {
-            const float ox = __shfl_sync(0xffffffffu, (float)mine.x, r), oy = __shfl_sync(0xffffffffu, (float)mine.y, r);
-            const float ovx = __shfl_sync(0xffffffffu, (float)mine.dx, r), ovy = __shfl_sync(0xffffffffu, (float)mine.dy, r);
-            float h = r0 + r < np ? 0.0f : w0[0];      // w0[0] * flag
-            h = __fmaf_rn(w0[1 + 5 * S + 0], ox, h);
-            h = __fmaf_rn(w0[1 + 5 * S + 1], oy, h);
-            h = __fmaf_rn(w0[1 + 5 * S + 2], ovx, h);
-            h = __fmaf_rn(w0[1 + 5 * S + 3], ovy, h);
-            actA[lane] = softsign(baseA + h);
-            actB[lane] = softsign(baseB + h);
-            __syncwarp();
-            float ya, yb;
-            layer2(w1, b1, s_act[warp][0], s_act[warp][1], ya, yb);
-            __syncwarp();
-            actA[lane] = softsign(ya);
-            actB[lane] = softsign(yb);
-            __syncwarp();
-            layer2(w2, b2, s_act[warp][0], s_act[warp][1], ya, yb);
-            __syncwarp();
-            bestA = fmaxf(bestA, ya);
-            bestB = fmaxf(bestB, yb);
-        }
-    }
-    // head: v[0], v[1] (linear -> softsign), v0 -> tanh, argmax; lane = unit, both perspectives
-    actA[lane] = bestA;
-    actB[lane] = bestB;
-    __syncwarp();
-    float ya, yb;
-    layer2_t(&g_pol.v1t[0][0], kPolW, lane, g_pol.v1b[lane], actA, actB, ya, yb);
-    __syncwarp();
-    actA[lane] = softsign(ya);
-    actB[lane] = softsign(yb);
-    __syncwarp();
-    layer2_t(&g_pol.v2t[0][0], kPolW, lane, g_pol.v2b[lane], actA, actB, ya, yb);
-    __syncwarp();
-    actA[lane] = softsign(ya);
-    actB[lane] = softsign(yb);
-    __syncwarp();
-    float qa = -2.0f, qb = -2.0f;                    // lanes >= nout stay below any tanh value
-    if (lane < kPolMaxOut) {
-        layer2_t(&g_pol.v0t[0][0], kPolMaxOut, lane, g_pol.v0b[lane], actA, actB, ya, yb);
-        if (lane < nout) { qa = tanhf(ya); qb = tanhf(yb); }
-    }
-    // argmax over lanes 0 .. nout-1, first maximum like torch.argmax
-    float ma = qa, mb = qb;
-#pragma unroll
-    for (int d = 4; d > 0; d >>= 1) {
-        ma = fmaxf(ma, __shfl_xor_sync(0xffffffffu, ma, d));
-        mb = fmaxf(mb, __shfl_xor_sync(0xffffffffu, mb, d));
-    }
-    const bool live = rows > 0;
-    int ctlA = __ffs(__ballot_sync(0xffffffffu, lane < nout && qa == ma)) - 1;
-    int ctlB = __ffs(__ballot_sync(0xffffffffu, lane < nout && qb == mb)) - 1;
-    if (!live) ctlA = ctlB = 2;                      // finished game: the no-op control
-    if (lane == 0 && (ship_mask & 1)) actions[(size_t)g * S] = (uint8_t)ctlA;
-    if (S == 2 && lane == 1 && (ship_mask & 2)) actions[(size_t)g * S + 1] = (uint8_t)ctlB;
-    if (q_out && lane < nout) {
-        q_out[((size_t)g * S) * nout + lane] = live ? qa : 0.0f;
-        if (S == 2) q_out[((size_t)g * S + 1) * nout + lane] = live ? qb : 0.0f;
-    }
-    __syncwarp();
-    }  // games of this warp
-}
-
 // ------------------------------------------------------------------------------------------
-// policy_mma_kernel<R, S>: the same network on the tensor cores.  The three per-object layers are batched GEMMs
-// [row-vectors, 32] x [32, 32]: a warp takes a game's live rows eight objects at a time as ONE 16-row MMA tile — rows 0-7
-// the eight objects seen by ship 0, rows 8-15 the same objects seen by ship 1 — and runs f0, f[0], f[1] as
-// mma.sync.m16n8k8 TF32 tiles with fp32 accumulators (HMMA.1688.F32.TF32).  TF32 keeps 10 mantissa bits, which would move
-// the outputs by 1e-3 and flip near-tied argmaxes, so every product is taken as three: a = a_hi + a_lo, w = w_hi + w_lo
-// (each part exactly representable in TF32), a.w ~ a_lo.w_hi + a_hi.w_lo + a_hi.w_hi — the "3xTF32" scheme: fp32-level
-// results (the outputs stay within 2e-6 of the PyTorch fp32 network, as the CUDA-core kernel's do).
-//   * A fragments come straight from registers: a lane of quad g holds object row g, and the accumulator layout of one
-//     layer (columns 2t, 2t+1 of n-tile nt) IS the A layout of the next layer's k-step nt once the weights' input columns
-//     are permuted to match (k index t <-> unit 8 nt + 2t, t + 4 <-> 8 nt + 2t + 1) — no shuffle, no shared memory between
-//     layers.  The first layer's A fragment (15 features, K padded to 16) is built per lane from the game's ship features
-//     and ONE component of the row's object.
-//   * B fragments (weights, split into hi / lo, permuted, fragment-ordered: one LDS.128 per k-step and n-tile) are staged in
-//     shared memory once per CTA (20 KB).
-//   * max-pool: a running maximum in the accumulator layout, reduced across the quads once per game; the head (two
-//     32 x 32 layers and 32 -> nout on two vectors per game) stays on the CUDA cores, as in policy_kernel.
+// policy_mma_kernel<R, S, PL>: rl.ValueNetwork.forward (rl.py:140-165) on the features of rl.py:43-72, fused — the
+// observation tensor never exists — for every game and both perspectives (core.roll_ships), then control = argmax q (the
+// greedy policy of rl.QBot, rl.py:168-200).  The three per-object layers are batched GEMMs [row-vectors, 32] x [32, 32]:
+// a warp takes a game's live rows eight objects at a time as ONE 16-row MMA tile — rows 0-7 the eight objects seen by
+// ship 0, rows 8-15 the same objects seen by ship 1 — and runs f0, f[0], f[1] as mma.sync.m16n8k16 tiles with FP16
+// operands and fp32 accumulators (HMMA.16816.F32).  An 11-bit operand alone would move the outputs by 1e-3 and flip
+// near-tied argmaxes, so every product is taken as three: a = a_hi + a_lo, w = w_hi + w_lo (each part an FP16 number),
+// a.w ~ a_lo.w_hi + a_hi.w_lo + a_hi.w_hi — fp32-level results (the outputs stay within 2e-6 of the PyTorch fp32
+// network).  FP16's range (|x| < 65,504; lo parts below 6e-5 lose relative precision, 3e-8 absolute) is ample for this
+// network: activations sit in (-1, 1), features and pre-activations within a few units.
+//   * A fragments come straight from registers: the accumulator layout of one layer (columns 2t, 2t+1 of n-tiles 2k and
+//     2k+1) IS the A layout of the next layer's k-step k — no shuffle, no shared memory between layers.  The first
+//     layer's A fragment (15 features, K padded to 16: one k-step) is built per lane from the game's ship features and
+//     one or two components of the row's object.
+//   * B fragments (weights, split into hi / lo, fragment-ordered: one LDS.128 per k-step and n-tile) are built once by
+//     astro_policy_set_weights and staged in shared memory once per CTA (20 KB).
+//   * max-pool: a running maximum in the accumulator layout, reduced across the quads once per game; a warp pools 8
+//     games and then runs the head (two 32 x 32 layers and 32 -> nout) for all of them as one 16-row tile.
 // ------------------------------------------------------------------------------------------
 constexpr int kMmaWarps = 4;
 constexpr int kPoolStride = 36;      // floats per row of the pooled tile (32 + 4: the A-fragment loads hit 32 different banks)
-// Two forms of the MMA, selected at build time:
-//   ASTRO_POLICY_F16 = 1 (default)  mma.sync.m16n8k16 FP16 operands (HMMA.16816.F32): 16 input columns per instruction
-//   ASTRO_POLICY_F16 = 0            mma.sync.m16n8k8  TF32 operands (HMMA.1688.F32.TF32): 8 per instruction
-// Both carry 11 significant bits per operand and use the same three-product split (x = hi + lo), so the results agree to
-// fp32 level; the FP16 form halves the MMA and B-fragment-load counts — the TF32 form was bound by the tensor pipe's issue
-// interval.  FP16's range (|x| < 65,504; lo parts below 6e-5 lose relative precision, 3e-8 absolute) is ample for this
-// network: activations sit in (-1, 1), features and pre-activations within a few units.
-#ifndef ASTRO_POLICY_F16
-#define ASTRO_POLICY_F16 1
-#endif
-constexpr int kKs0 = ASTRO_POLICY_F16 ? 1 : 2;   // k-steps of the first layer (16 input columns)
-constexpr int kKs = ASTRO_POLICY_F16 ? 2 : 4;    // k-steps of a 32-wide layer
+constexpr int kKs0 = 1;              // k-steps of the first layer (16 input columns)
+constexpr int kKs = 2;               // k-steps of a 32-wide layer
 struct PolicyFragWeights {           // B fragments {b0_hi, b1_hi, b0_lo, b1_lo} per lane, built once by astro_policy_set_weights
     float4 f0[kKs0][4][32];          // [k-step][n-tile][lane]: per-object layers
     float4 f1[kKs][4][32];
@@ -1328,21 +1128,6 @@ struct PolicyFrags {                 // per CTA, in (dynamic) shared memory
     float4 red[kMmaWarps][8][4][2];  // per warp: max-pool exchange, [quad][t][half of the 16 accumulators as 2 float4]
     float sf[kMmaWarps][8][12];      // per warp: the ship features of its 8 games, ship 0 then ship 1
 };
-// x = hi + lo for the 3xTF32 scheme.  The tensor core reads only the 19 high bits of an fp32 operand (it truncates), so hi
-// is x itself — no instruction — standing for trunc(x); lo = x - trunc(x) exactly (a mask and a subtraction), and adding
-// half a TF32 ulp to lo's bit pattern makes the hardware's truncation of lo a round-to-nearest: what the pair drops is
-// below 2^-22 |x| and unbiased.  (cvt.rna.tf32.f32 runs on the XU pipe at a quarter rate: the split was half of this
-// kernel's time when it went through it.)
-__device__ __forceinline__ void split_tf32 [[maybe_unused]] (float x, uint32_t& hi, uint32_t& lo) {
-    hi = __float_as_uint(x);
-    lo = __float_as_uint(__fsub_rn(x, __uint_as_float(hi & 0xffffe000u))) + 0x1000u;
-}
-__device__ __forceinline__ void mma_tf32(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-                 : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-}
-#if ASTRO_POLICY_F16
 // two fp32 values -> the FP16 pair (hi) and the FP16 pair of what that dropped (lo); lower half = the even column
 __device__ __forceinline__ void split_f16x2(float xe, float xo, uint32_t& hi, uint32_t& lo) {
     asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(xo), "f"(xe));
@@ -1385,34 +1170,6 @@ __device__ __forceinline__ void mma_layer(float (&out)[NT][4], const float (&in)
         mma_kstep16<NT>(out, x, wf + kk * NT * 32, lane);
     }
 }
-#else
-template <int NT, bool ACT>
-__device__ __forceinline__ void mma_layer(float (&out)[NT][4], const float (&in)[4][4], const float4* __restrict__ wf, int lane);
-#endif
-// (TF32 form) one k-step of a layer for NT n-tiles: A = (x0, x1, x2, x3) in fp32, split here; B from shared memory
-template <int NT>
-__device__ __forceinline__ void mma_kstep(float (&acc)[NT][4], float x0, float x1, float x2, float x3, const float4* __restrict__ bfrag, int lane) {
-    uint32_t h0, h1, h2, h3, l0, l1, l2, l3;
-    split_tf32(x0, h0, l0); split_tf32(x1, h1, l1); split_tf32(x2, h2, l2); split_tf32(x3, h3, l3);
-#pragma unroll
-    for (int nt = 0; nt < NT; nt++) {
-        const float4 b = bfrag[nt * 32 + lane];
-        const uint32_t bh0 = __float_as_uint(b.x), bh1 = __float_as_uint(b.y), bl0 = __float_as_uint(b.z), bl1 = __float_as_uint(b.w);
-        mma_tf32(acc[nt], l0, l1, l2, l3, bh0, bh1);      // small terms first
-        mma_tf32(acc[nt], h0, h1, h2, h3, bl0, bl1);
-        mma_tf32(acc[nt], h0, h1, h2, h3, bh0, bh1);
-    }
-}
-#if !ASTRO_POLICY_F16
-template <int NT, bool ACT>
-__device__ __forceinline__ void mma_layer(float (&out)[NT][4], const float (&in)[4][4], const float4* __restrict__ wf, int lane) {
-#pragma unroll
-    for (int kk = 0; kk < 4; kk++) {     // the accumulators of n-tile kk are the A fragment of k-step kk (input columns permuted to match)
-        const float a = in[kk][0], b = in[kk][2], c = in[kk][1], d = in[kk][3];
-        mma_kstep<NT>(out, ACT ? softsign(a) : a, ACT ? softsign(b) : b, ACT ? softsign(c) : c, ACT ? softsign(d) : d, wf + kk * NT * 32, lane);
-    }
-}
-#endif
 template <int NT>
 __device__ __forceinline__ void init_bias(float (&acc)[NT][4], const float2 (*bias)[4], int t) {
 #pragma unroll
@@ -1443,15 +1200,15 @@ policy_mma_kernel(const void* __restrict__ ships_, const void* __restrict__ ship
         for (int i = threadIdx.x; i < (int)(sizeof(PolicyFragWeights) / 16); i += blockDim.x) dst[i] = src[i];
     }
     __syncthreads();
-    // ---- what this lane's four feature slots (columns t, t + 4, t + 8, t + 12) are: flag / ship feature / object component / zero
-    // (FP16 form: columns 2t, 2t + 1, 2t + 8, 2t + 9 — one k-step of 16; TF32 form: t, t + 4, t + 8, t + 12 — two of 8)
+    // ---- what this lane's four feature slots (columns 2t, 2t + 1, 2t + 8, 2t + 9: one k-step of 16) are: flag / ship
+    // feature / object component / zero
     int ship_idx[4], obj_idx[4];
     bool is_flag = false, any_obj = false;
 #pragma unroll
     for (int j = 0; j < 4; j++) {
-        const int col = ASTRO_POLICY_F16 ? 2 * t + (j & 1) + 8 * (j >> 1) : t + 4 * j;
+        const int col = 2 * t + (j & 1) + 8 * (j >> 1);
         ship_idx[j] = obj_idx[j] = -1;
-        if (col == 0) is_flag = true;                           // (slot 0 of lane t = 0 in both forms)
+        if (col == 0) is_flag = true;                           // (slot 0 of lane t = 0)
         else if (col <= 5 * S) ship_idx[j] = col - 1;           // feature (col - 1) % 5 of ship (col - 1) / 5, ship 0's perspective
         else if (col < DIN) { obj_idx[j] = col - 1 - 5 * S; any_obj = true; }
     }
@@ -1544,15 +1301,10 @@ policy_mma_kernel(const void* __restrict__ ships_, const void* __restrict__ ship
                 if (is_flag) xa[0] = xb[0] = (r < np) ? 0.0f : 1.0f;
                 float acc[4][4], nxt[4][4];
                 init_bias<4>(acc, s_w.bias[0], t);               // f0: K = 16 (15 features)
-#if ASTRO_POLICY_F16
                 {
                     const float x0[8] = {xa[0], xa[1], xb[0], xb[1], xa[2], xa[3], xb[2], xb[3]};
                     mma_kstep16<4>(acc, x0, &s_w.f0[0][0][0], lane);
                 }
-#else
-                mma_kstep<4>(acc, xa[0], xb[0], xa[1], xb[1], &s_w.f0[0][0][0], lane);
-                mma_kstep<4>(acc, xa[2], xb[2], xa[3], xb[3], &s_w.f0[1][0][0], lane);
-#endif
 #pragma unroll
                 for (int layer = 1; layer <= 2; layer++) {       // f[0], f[1]: h = W softsign(h) + b
                     const float4* wf = layer == 1 ? &s_w.f1[0][0][0] : &s_w.f2[0][0][0];
@@ -1593,7 +1345,6 @@ policy_mma_kernel(const void* __restrict__ ships_, const void* __restrict__ ship
         // ---- head for the 8 games at once: v[0], v[1] (linear -> softsign) as 16 x 32 x 32 MMA tiles, v0 as 16 x 32 x 8
         float h1[4][4], h2[4][4], q4[1][4];
         init_bias<4>(h1, s_w.bias[3], t);
-#if ASTRO_POLICY_F16
 #pragma unroll
         for (int kk = 0; kk < 2; kk++) {
             const float2 p0 = *reinterpret_cast<const float2*>(&pool[gq][16 * kk + 2 * t]), p1 = *reinterpret_cast<const float2*>(&pool[gq + 8][16 * kk + 2 * t]);
@@ -1601,11 +1352,6 @@ policy_mma_kernel(const void* __restrict__ ships_, const void* __restrict__ ship
             const float x[8] = {p0.x, p0.y, p1.x, p1.y, p2.x, p2.y, p3.x, p3.y};
             mma_kstep16<4>(h1, x, &s_w.v1[kk][0][0], lane);
         }
-#else
-#pragma unroll
-        for (int kk = 0; kk < 4; kk++)
-            mma_kstep<4>(h1, pool[gq][kk * 8 + t], pool[gq + 8][kk * 8 + t], pool[gq][kk * 8 + t + 4], pool[gq + 8][kk * 8 + t + 4], &s_w.v1[kk][0][0], lane);
-#endif
         init_bias<4>(h2, s_w.bias[4], t);
         mma_layer<4, true>(h2, h1, &s_w.v2[0][0][0], lane);
         {
@@ -1659,7 +1405,6 @@ policy_mma_kernel(const void* __restrict__ ships_, const void* __restrict__ ship
 //   longer come from a padding row: pre-activations are far below 1e9); an item without any live row takes every chunk,
 //   exactly the reference's arithmetic.
 // ------------------------------------------------------------------------------------------
-#if ASTRO_POLICY_F16
 template <int DIN>
 __global__ void __launch_bounds__(kMmaWarps * 32, ASTRO_MMA_MIN_BLOCKS)
 value_forward_kernel(const float* __restrict__ features, float* __restrict__ q_out, int n_items, int rows, int nout,
@@ -1824,7 +1569,6 @@ value_forward_kernel(const float* __restrict__ features, float* __restrict__ q_o
         __syncwarp();
     }
 }
-#endif
 
 // ------------------------------------------------------------------------------------------
 // explore_kernel: rl.EpsilonGreedy.__call__ (rl.py:10-30) for every ship — the random policy that
@@ -2210,8 +1954,7 @@ struct AstroBatch {
     int64_t first_game;
     int64_t launches;
     int32_t policy_nout;  // > 0 once astro_policy_set_weights has been called
-    PolicyWeights* d_pol; // this batch's network (astro_policy_set_weights)
-    PolicyFragWeights* d_pol_frags;   // ... as tensor-core B fragments (policy_mma_kernel)
+    PolicyFragWeights* d_pol_frags;   // this batch's network as tensor-core B fragments (astro_policy_set_weights)
     int32_t* d_src;       // astro_import_games: game -> row map
     char* d_single;       // astro_step_single_host: device staging, in record then out record
     int64_t single_bytes;
@@ -2258,9 +2001,24 @@ int check(const AstroBatch* b, bool need_bound) {
     return ASTRO_OK;
 }
 
-const void* current_bullets(const AstroBatch* b) {
+// Bullet-list buffer `which` of the two: b->cur holds the lists, the other one is where the next tick writes them.
+void* bullet_buffer(const AstroBatch* b, int which) {
     const size_t buf_bytes = (size_t)b->n_games * b->K * 4 * (b->precision == 32 ? sizeof(float) : sizeof(double));
-    return (const char*)b->bufs.bullets + (size_t)b->cur * buf_bytes;
+    return (char*)b->bufs.bullets + (size_t)which * buf_bytes;
+}
+
+template <typename T> struct TypeTag { using type = T; };
+template <int N> using IntTag = std::integral_constant<int, N>;
+
+// The batch's layout as kernel template arguments: calls f(TypeTag<R>, IntTag<S>, IntTag<PL>) for the batch's precision,
+// ships per game and planet slots, and returns what f returns.
+template <typename F>
+auto with_layout(const AstroBatch* b, F&& f) {
+    auto by_pl = [&](auto r, auto s) {
+        return b->PL == ASTRO_MAX_PLANETS_WIDE ? f(r, s, IntTag<ASTRO_MAX_PLANETS_WIDE>()) : f(r, s, IntTag<ASTRO_MAX_PLANETS>());
+    };
+    auto by_s = [&](auto r) { return b->S == 2 ? by_pl(r, IntTag<2>()) : by_pl(r, IntTag<1>()); };
+    return b->precision == 32 ? by_s(TypeTag<float>()) : by_s(TypeTag<double>());
 }
 
 void fill_params(const AstroBatch* b, TickParams& p) {
@@ -2268,9 +2026,8 @@ void fill_params(const AstroBatch* b, TickParams& p) {
     p.ships = b->bufs.ships;
     p.ship_b = b->bufs.ship_b;
     p.planets = b->bufs.planets;
-    const size_t buf_bytes = (size_t)b->n_games * b->K * 4 * (b->precision == 32 ? sizeof(float) : sizeof(double));
-    p.bullets_in = (char*)b->bufs.bullets + (size_t)b->cur * buf_bytes;
-    p.bullets_out = (char*)b->bufs.bullets + (size_t)(b->cur ^ 1) * buf_bytes;
+    p.bullets_in = bullet_buffer(b, b->cur);
+    p.bullets_out = bullet_buffer(b, b->cur ^ 1);
     p.meta = b->bufs.meta;
     p.episode = b->bufs.episode;
     p.fire_bits = b->d_fire_bits;
@@ -2501,21 +2258,13 @@ int do_ticks(AstroBatch* b, const uint8_t* actions, float* reward, uint8_t* done
             p.bot_modes = b->bot_modes_now;
             p.script = b->script_now;
         }
-        cudaError_t e;
-        if (b->PL == ASTRO_MAX_PLANETS_WIDE) {
-            constexpr int PL = ASTRO_MAX_PLANETS_WIDE;
-            if (fused)
-                e = b->S == 2 ? launch_tick_f32_wide<2>(p, st) : launch_tick_f32_wide<1>(p, st);
-            else if (b->precision == 32)
-                e = b->S == 2 ? launch_tick<float, 2, PL>(p, st) : launch_tick<float, 1, PL>(p, st);
-            else
-                e = b->S == 2 ? launch_tick<double, 2, PL>(p, st) : launch_tick<double, 1, PL>(p, st);
-        } else if (fused)
-            e = b->S == 2 ? launch_tick_f32<2>(p, st) : launch_tick_f32<1>(p, st);
-        else if (b->precision == 32)
-            e = b->S == 2 ? launch_tick<float, 2, ASTRO_MAX_PLANETS>(p, st) : launch_tick<float, 1, ASTRO_MAX_PLANETS>(p, st);
-        else
-            e = b->S == 2 ? launch_tick<double, 2, ASTRO_MAX_PLANETS>(p, st) : launch_tick<double, 1, ASTRO_MAX_PLANETS>(p, st);
+        const cudaError_t e = with_layout(b, [&](auto r, auto s, auto pl) {
+            if (fused) {                                     // (float32 batches only)
+                if constexpr (pl == ASTRO_MAX_PLANETS) return launch_tick_f32<s>(p, st);
+                else return launch_tick_f32_wide<s>(p, st);
+            }
+            return launch_tick<typename decltype(r)::type, s, pl>(p, st);
+        });
         if (e != cudaSuccess) return fail(ASTRO_E_CUDA, "tick_kernel launch: %s", cudaGetErrorString(e));
         b->launches += 1;
         k0 += kc;
@@ -2608,7 +2357,6 @@ int astro_batch_destroy(AstroBatch* b) {
     cudaFree(b->d_reward);
     cudaFree(b->d_fire_bits);
     cudaFree(b->d_pool_rec);
-    cudaFree(b->d_pol);
     cudaFree(b->d_pol_frags);
     cudaFree(b->d_src);
     cudaFree(b->d_single);
@@ -2705,11 +2453,7 @@ int astro_set_reset_pool(AstroBatch* b, const AstroResetPool* pool) {
         const float* ps = (const float*)pool->ships;
         const float* pp = (const float*)pool->planets;
         float* rec = (float*)b->d_pool_rec;
-        if (wide) {
-            if (b->S == 2) pack_pool_kernel<2, ASTRO_MAX_PLANETS_WIDE><<<grid, 128>>>(ps, pp, pool->np, rec, pool->size);
-            else pack_pool_kernel<1, ASTRO_MAX_PLANETS_WIDE><<<grid, 128>>>(ps, pp, pool->np, rec, pool->size);
-        } else if (b->S == 2) pack_pool_kernel<2, ASTRO_MAX_PLANETS><<<grid, 128>>>(ps, pp, pool->np, rec, pool->size);
-        else pack_pool_kernel<1, ASTRO_MAX_PLANETS><<<grid, 128>>>(ps, pp, pool->np, rec, pool->size);
+        with_layout(b, [&](auto, auto s, auto pl) { pack_pool_kernel<s, pl><<<grid, 128>>>(ps, pp, pool->np, rec, pool->size); });
         CUDA_TRY(cudaGetLastError());
         CUDA_TRY(cudaDeviceSynchronize());
         b->launches += 1;
@@ -2879,19 +2623,7 @@ int astro_reset_done(AstroBatch* b, void* stream) {
     fill_params(b, p);
     const int grid = (p.n_games + kTickThreads - 1) / kTickThreads;
     cudaStream_t st = (cudaStream_t)stream;
-#define LAUNCH_RESET(PL_)                                                                  \
-    do {                                                                                   \
-        if (b->precision == 32) {                                                          \
-            if (b->S == 2) reset_kernel<float, 2, PL_><<<grid, kTickThreads, 0, st>>>(p);  \
-            else reset_kernel<float, 1, PL_><<<grid, kTickThreads, 0, st>>>(p);            \
-        } else {                                                                           \
-            if (b->S == 2) reset_kernel<double, 2, PL_><<<grid, kTickThreads, 0, st>>>(p); \
-            else reset_kernel<double, 1, PL_><<<grid, kTickThreads, 0, st>>>(p);           \
-        }                                                                                  \
-    } while (0)
-    if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_RESET(ASTRO_MAX_PLANETS_WIDE);
-    else LAUNCH_RESET(ASTRO_MAX_PLANETS);
-#undef LAUNCH_RESET
+    with_layout(b, [&](auto r, auto s, auto pl) { reset_kernel<typename decltype(r)::type, s, pl><<<grid, kTickThreads, 0, st>>>(p); });
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
     return ASTRO_OK;
@@ -2910,27 +2642,18 @@ static int observe_impl(AstroBatch* b, float* obs, int32_t n_rows, bool both, vo
     const int grid = (b->n_games + kObserveWarps - 1) / kObserveWarps;
     cudaStream_t st = (cudaStream_t)stream;
     const AstroBuffers& u = b->bufs;
-    const void* cur_bullets = current_bullets(b);
-#define LAUNCH_OBS(R, S_, BOTH_, PL_)                                                                                       \
-    do {                                                                                                                    \
-        CUDA_TRY(cudaFuncSetAttribute(observe_kernel<R, S_, BOTH_, PL_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        observe_kernel<R, S_, BOTH_, PL_><<<grid, kObserveWarps * 32, smem, st>>>(u.ships, u.ship_b, u.planets, cur_bullets, u.meta, \
-                                                                                  obs, b->n_games, b->K, n_rows);             \
-    } while (0)
-#define LAUNCH_OBS_PL(PL_)                                                                                        \
-    do {                                                                                                          \
-        if (b->precision == 32) {                                                                                 \
-            if (b->S == 2) { if (both) LAUNCH_OBS(float, 2, true, PL_); else LAUNCH_OBS(float, 2, false, PL_); }   \
-            else LAUNCH_OBS(float, 1, false, PL_);                                                                \
-        } else {                                                                                                  \
-            if (b->S == 2) { if (both) LAUNCH_OBS(double, 2, true, PL_); else LAUNCH_OBS(double, 2, false, PL_); } \
-            else LAUNCH_OBS(double, 1, false, PL_);                                                               \
-        }                                                                                                         \
-    } while (0)
-    if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_OBS_PL(ASTRO_MAX_PLANETS_WIDE);
-    else LAUNCH_OBS_PL(ASTRO_MAX_PLANETS);
-#undef LAUNCH_OBS_PL
-#undef LAUNCH_OBS
+    auto launch = [&](auto kernel) {
+        CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kernel<<<grid, kObserveWarps * 32, smem, st>>>(u.ships, u.ship_b, u.planets, bullet_buffer(b, b->cur), u.meta, obs, b->n_games,
+                                                       b->K, n_rows);
+        return ASTRO_OK;
+    };
+    if (int r = with_layout(b, [&](auto tr, auto s, auto pl) {
+            using R = typename decltype(tr)::type;
+            if constexpr (s == 2) return both ? launch(observe_kernel<R, 2, true, pl>) : launch(observe_kernel<R, 2, false, pl>);
+            else return launch(observe_kernel<R, 1, false, pl>);     // (both views of a solo game are the same)
+        }))
+        return r;
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
     return ASTRO_OK;
@@ -2959,19 +2682,9 @@ int astro_script_controls(AstroBatch* b, double avoid_distance, double avoid_thr
     const int grid = (b->n_games * b->S + 127) / 128;
     cudaStream_t st = (cudaStream_t)stream;
     const AstroBuffers& u = b->bufs;
-#define LAUNCH_SCRIPT(PL_)                                                                                              \
-    do {                                                                                                                \
-        if (b->precision == 32) {                                                                                       \
-            if (b->S == 2) script_kernel<float, 2, PL_><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, u.meta, actions, q);  \
-            else script_kernel<float, 1, PL_><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, u.meta, actions, q);            \
-        } else {                                                                                                        \
-            if (b->S == 2) script_kernel<double, 2, PL_><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, u.meta, actions, q); \
-            else script_kernel<double, 1, PL_><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, u.meta, actions, q);           \
-        }                                                                                                               \
-    } while (0)
-    if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_SCRIPT(ASTRO_MAX_PLANETS_WIDE);
-    else LAUNCH_SCRIPT(ASTRO_MAX_PLANETS);
-#undef LAUNCH_SCRIPT
+    with_layout(b, [&](auto r, auto s, auto pl) {
+        script_kernel<typename decltype(r)::type, s, pl><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, u.meta, actions, q);
+    });
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
     return ASTRO_OK;
@@ -2997,19 +2710,10 @@ int astro_create_games(AstroBatch* b, const AstroCreateConfig* cc, const uint32_
     q.pad = 0;
     const int grid = (m + 63) / 64;
     cudaStream_t st = (cudaStream_t)stream;
-#define LAUNCH_CREATE(PL_)                                                                                                  \
-    do {                                                                                                                    \
-        if (b->precision == 32) {                                                                                           \
-            if (b->S == 2) create_kernel<float, 2, PL_><<<grid, 64, 0, st>>>(seeds, (float*)ships, (float*)planets, n_planets, q);   \
-            else create_kernel<float, 1, PL_><<<grid, 64, 0, st>>>(seeds, (float*)ships, (float*)planets, n_planets, q);             \
-        } else {                                                                                                            \
-            if (b->S == 2) create_kernel<double, 2, PL_><<<grid, 64, 0, st>>>(seeds, (double*)ships, (double*)planets, n_planets, q); \
-            else create_kernel<double, 1, PL_><<<grid, 64, 0, st>>>(seeds, (double*)ships, (double*)planets, n_planets, q);           \
-        }                                                                                                                   \
-    } while (0)
-    if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_CREATE(ASTRO_MAX_PLANETS_WIDE);
-    else LAUNCH_CREATE(ASTRO_MAX_PLANETS);
-#undef LAUNCH_CREATE
+    with_layout(b, [&](auto tr, auto s, auto pl) {
+        using R = typename decltype(tr)::type;
+        create_kernel<R, s, pl><<<grid, 64, 0, st>>>(seeds, (R*)ships, (R*)planets, n_planets, q);
+    });
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
     return ASTRO_OK;
@@ -3023,29 +2727,20 @@ int astro_policy_set_weights(AstroBatch* b, const float* weights_host, int32_t n
     if (!weights_host || n_floats != expect)
         return fail(ASTRO_E_INVALID, "expected %d floats (f0, f[0], f[1], v[0], v[1], v0: weight then bias each), got %d", expect, n_floats);
     CUDA_TRY(cudaSetDevice(b->device));
-    PolicyWeights* w = new (std::nothrow) PolicyWeights();
-    if (!w) return fail(ASTRO_E_NOMEM, "out of host memory");
-    memset(w, 0, sizeof(*w));
-    const float* p = weights_host;
-    for (int u = 0; u < kPolW; u++) for (int c = 0; c < din; c++) w->f0t[c][u] = *p++;
-    memcpy(w->f0b, p, sizeof(w->f0b)); p += kPolW;
-    for (int u = 0; u < kPolW; u++) for (int c = 0; c < kPolW; c++) w->f1t[c][u] = *p++;
-    memcpy(w->f1b, p, sizeof(w->f1b)); p += kPolW;
-    for (int u = 0; u < kPolW; u++) for (int c = 0; c < kPolW; c++) w->f2t[c][u] = *p++;
-    memcpy(w->f2b, p, sizeof(w->f2b)); p += kPolW;
-    for (int u = 0; u < kPolW; u++) for (int c = 0; c < kPolW; c++) w->v1t[c][u] = *p++;
-    memcpy(w->v1b, p, sizeof(w->v1b)); p += kPolW;
-    for (int u = 0; u < kPolW; u++) for (int c = 0; c < kPolW; c++) w->v2t[c][u] = *p++;
-    memcpy(w->v2b, p, sizeof(w->v2b)); p += kPolW;
-    for (int u = 0; u < nout; u++) for (int c = 0; c < kPolW; c++) w->v0t[c][u] = *p++;
-    memcpy(w->v0b, p, sizeof(float) * nout);
-    // the same weights as tensor-core B fragments for policy_mma_kernel: split into TF32 hi / lo parts (round to nearest,
-    // ties away: cvt.rna.tf32.f32), input columns in the order the A fragments arrive in (see the kernel)
+    // weights_host: every layer's weight [out][in] (nn.Linear), then its bias
+    const float* f0 = weights_host;
+    const float* f1 = f0 + kPolW * din + kPolW;
+    const float* f2 = f1 + kPolW * kPolW + kPolW;
+    const float* v1 = f2 + kPolW * kPolW + kPolW;
+    const float* v2 = v1 + kPolW * kPolW + kPolW;
+    const float* v0 = v2 + kPolW * kPolW + kPolW;
+    const float* v0b = v0 + nout * kPolW;
+    // the weights as tensor-core B fragments for policy_mma_kernel / value_forward_kernel, input columns in the order the A
+    // fragments arrive in (see the kernel)
     PolicyFragWeights* fw = new (std::nothrow) PolicyFragWeights();
-    if (!fw) { delete w; return fail(ASTRO_E_NOMEM, "out of host memory"); }
+    if (!fw) return fail(ASTRO_E_NOMEM, "out of host memory");
     memset(fw, 0, sizeof(*fw));
     {
-#if ASTRO_POLICY_F16
         // FP16 pairs: a fragment register holds input columns (k, k + 1), the even one in the low half; hi = the weight rounded
         // to FP16, lo = what that dropped, rounded to FP16
         auto pair = [](float we, float wo, uint32_t& hi, uint32_t& lo) {
@@ -3066,52 +2761,27 @@ int astro_policy_set_weights(AstroBatch* b, const float* weights_host, int32_t n
             const int g_ = l >> 2, t_ = l & 3;
             for (int nt = 0; nt < 4; nt++) {
                 const int n = nt * 8 + g_;
-                fw->f0[0][nt][l] = entry16([&](int c) { return c < din ? w->f0t[c][n] : 0.f; }, 2 * t_);
+                fw->f0[0][nt][l] = entry16([&](int c) { return c < din ? f0[n * din + c] : 0.f; }, 2 * t_);
                 for (int kk = 0; kk < 2; kk++) {
                     const int k0 = 16 * kk + 2 * t_;
-                    fw->f1[kk][nt][l] = entry16([&](int c) { return w->f1t[c][n]; }, k0);
-                    fw->f2[kk][nt][l] = entry16([&](int c) { return w->f2t[c][n]; }, k0);
-                    fw->v1[kk][nt][l] = entry16([&](int c) { return w->v1t[c][n]; }, k0);
-                    fw->v2[kk][nt][l] = entry16([&](int c) { return w->v2t[c][n]; }, k0);
+                    fw->f1[kk][nt][l] = entry16([&](int c) { return f1[n * kPolW + c]; }, k0);
+                    fw->f2[kk][nt][l] = entry16([&](int c) { return f2[n * kPolW + c]; }, k0);
+                    fw->v1[kk][nt][l] = entry16([&](int c) { return v1[n * kPolW + c]; }, k0);
+                    fw->v2[kk][nt][l] = entry16([&](int c) { return v2[n * kPolW + c]; }, k0);
                 }
             }
-            for (int kk = 0; kk < 2; kk++) fw->v0[kk][l] = entry16([&](int c) { return w->v0t[c][g_]; }, 16 * kk + 2 * t_);
+            for (int kk = 0; kk < 2; kk++) fw->v0[kk][l] = entry16([&](int c) { return g_ < nout ? v0[g_ * kPolW + c] : 0.f; }, 16 * kk + 2 * t_);
         }
-#else
-        auto rna = [](float x) { uint32_t u; memcpy(&u, &x, 4); u = (u + 0x1000u) & 0xffffe000u; float r; memcpy(&r, &u, 4); return r; };
-        auto entry = [&](float w0, float w1) { const float h0 = rna(w0), h1 = rna(w1); return make_float4(h0, h1, rna(w0 - h0), rna(w1 - h1)); };
-        for (int l = 0; l < 32; l++) {
-            const int g_ = l >> 2, t_ = l & 3;
-            for (int nt = 0; nt < 4; nt++) {
-                const int n = nt * 8 + g_;
-                for (int kk = 0; kk < 2; kk++) {                  // f0: natural K order, columns 8 kk + t, 8 kk + t + 4 (>= din: zero)
-                    const int c0 = kk * 8 + t_, c1 = c0 + 4;
-                    fw->f0[kk][nt][l] = entry(c0 < din ? w->f0t[c0][n] : 0.f, c1 < din ? w->f0t[c1][n] : 0.f);
-                }
-                for (int kk = 0; kk < 4; kk++) {
-                    const int cp = kk * 8 + 2 * t_, cn = kk * 8 + t_;     // permuted (A = accumulators) / natural (A = shared memory)
-                    fw->f1[kk][nt][l] = entry(w->f1t[cp][n], w->f1t[cp + 1][n]);
-                    fw->f2[kk][nt][l] = entry(w->f2t[cp][n], w->f2t[cp + 1][n]);
-                    fw->v1[kk][nt][l] = entry(w->v1t[cn][n], w->v1t[cn + 4][n]);
-                    fw->v2[kk][nt][l] = entry(w->v2t[cp][n], w->v2t[cp + 1][n]);
-                }
-            }
-            for (int kk = 0; kk < 4; kk++) fw->v0[kk][l] = entry(w->v0t[kk * 8 + 2 * t_][g_], w->v0t[kk * 8 + 2 * t_ + 1][g_]);
-        }
-#endif
-        const float* biases[5] = {w->f0b, w->f1b, w->f2b, w->v1b, w->v2b};
+        const float* biases[5] = {f0 + kPolW * din, f1 + kPolW * kPolW, f2 + kPolW * kPolW, v1 + kPolW * kPolW, v2 + kPolW * kPolW};
         for (int layer = 0; layer < 5; layer++)
             for (int nt = 0; nt < 4; nt++)
                 for (int t_ = 0; t_ < 4; t_++) fw->bias[layer][nt][t_] = make_float2(biases[layer][nt * 8 + 2 * t_], biases[layer][nt * 8 + 2 * t_ + 1]);
-        for (int t_ = 0; t_ < 4; t_++) fw->bias_v0[t_] = make_float2(w->v0b[2 * t_], w->v0b[2 * t_ + 1]);
+        for (int t_ = 0; t_ < 4; t_++) fw->bias_v0[t_] = make_float2(2 * t_ < nout ? v0b[2 * t_] : 0.f, 2 * t_ + 1 < nout ? v0b[2 * t_ + 1] : 0.f);
     }
-    cudaError_t e = b->d_pol ? cudaSuccess : cudaMalloc(&b->d_pol, sizeof(PolicyWeights));
-    if (e == cudaSuccess && !b->d_pol_frags) e = cudaMalloc(&b->d_pol_frags, sizeof(PolicyFragWeights));
+    cudaError_t e = b->d_pol_frags ? cudaSuccess : cudaMalloc(&b->d_pol_frags, sizeof(PolicyFragWeights));
+    // (pageable source: the copy has left `fw` when the call returns; stream-ordered before later launches)
     if (e == cudaSuccess) e = cudaMemcpy(b->d_pol_frags, fw, sizeof(*fw), cudaMemcpyHostToDevice);
     delete fw;
-    // (pageable source: the copy has left `w` when the call returns; stream-ordered before later launches)
-    if (e == cudaSuccess) e = cudaMemcpy(b->d_pol, w, sizeof(*w), cudaMemcpyHostToDevice);
-    delete w;
     if (e != cudaSuccess) return fail(ASTRO_E_CUDA, "policy weights upload: %s", cudaGetErrorString(e));
     b->policy_nout = nout;
     b->config_epoch++;
@@ -3123,46 +2793,19 @@ int astro_policy_controls(AstroBatch* b, uint8_t* actions, float* q_out, int32_t
     if (b->policy_nout <= 0) return fail(ASTRO_E_STATE, "astro_policy_set_weights has not been called");
     if (!actions) return fail(ASTRO_E_INVALID, "null actions");
     CUDA_TRY(cudaSetDevice(b->device));
-    int grid = (b->n_games + kPolWarps * kPolGamesPerWarp - 1) / (kPolWarps * kPolGamesPerWarp);
-    {   // one resident wave: 4 CTAs of 128 threads per SM (128 registers per thread)
-        int sms = 0;
-        CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device));
-        if (grid > sms * ASTRO_POL_MIN_BLOCKS) grid = sms * ASTRO_POL_MIN_BLOCKS;
-    }
     cudaStream_t st = (cudaStream_t)stream;
     const AstroBuffers& u = b->bufs;
-    // the tensor-core kernel is the default; ASTRO_POLICY_MMA=0 selects the CUDA-core kernel (A/B, tests)
-    const char* pm = getenv("ASTRO_POLICY_MMA");
-    const bool use_mma = !(pm && atoi(pm) == 0);
-    if (use_mma) {
-        int sms = 0;
-        CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device));
-        int mgrid = ((b->n_games + 7) / 8 + kMmaWarps - 1) / kMmaWarps;      // a warp takes 8 games at a time
-        if (mgrid > sms * ASTRO_MMA_MIN_BLOCKS) mgrid = sms * ASTRO_MMA_MIN_BLOCKS;
-        const int msmem = (int)sizeof(PolicyFrags);
-#define LAUNCH_MMA(R, S_, PL_) \
-    do { CUDA_TRY(cudaFuncSetAttribute(policy_mma_kernel<R, S_, PL_>, cudaFuncAttributeMaxDynamicSharedMemorySize, msmem)); \
-    policy_mma_kernel<R, S_, PL_><<<mgrid, kMmaWarps * 32, msmem, st>>>(u.ships, u.ship_b, u.planets, current_bullets(b), u.meta, actions, q_out, b->n_games, b->K, b->policy_nout, ship_mask, b->d_pol_frags); } while (0)
-#define LAUNCH_MMA_PL(PL_) \
-    do { if (b->precision == 32) { if (b->S == 2) LAUNCH_MMA(float, 2, PL_); else LAUNCH_MMA(float, 1, PL_); } \
-         else { if (b->S == 2) LAUNCH_MMA(double, 2, PL_); else LAUNCH_MMA(double, 1, PL_); } } while (0)
-        if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_MMA_PL(ASTRO_MAX_PLANETS_WIDE);
-        else LAUNCH_MMA_PL(ASTRO_MAX_PLANETS);
-#undef LAUNCH_MMA_PL
-#undef LAUNCH_MMA
-        CUDA_TRY(cudaGetLastError());
-        b->launches += 1;
-        return ASTRO_OK;
-    }
-#define LAUNCH_POL(R, S_, PL_) \
-    policy_kernel<R, S_, PL_><<<grid, kPolWarps * 32, 0, st>>>(u.ships, u.ship_b, u.planets, current_bullets(b), u.meta, actions, q_out, b->n_games, b->K, b->policy_nout, ship_mask, b->d_pol)
-#define LAUNCH_POL_PL(PL_) \
-    do { if (b->precision == 32) { if (b->S == 2) LAUNCH_POL(float, 2, PL_); else LAUNCH_POL(float, 1, PL_); } \
-         else { if (b->S == 2) LAUNCH_POL(double, 2, PL_); else LAUNCH_POL(double, 1, PL_); } } while (0)
-    if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_POL_PL(ASTRO_MAX_PLANETS_WIDE);
-    else LAUNCH_POL_PL(ASTRO_MAX_PLANETS);
-#undef LAUNCH_POL_PL
-#undef LAUNCH_POL
+    int grid = ((b->n_games + 7) / 8 + kMmaWarps - 1) / kMmaWarps;      // a warp takes 8 games at a time
+    if (grid > b->sm_count * ASTRO_MMA_MIN_BLOCKS) grid = b->sm_count * ASTRO_MMA_MIN_BLOCKS;
+    const int smem = (int)sizeof(PolicyFrags);
+    if (int r = with_layout(b, [&](auto tr, auto s, auto pl) {
+            const auto kernel = policy_mma_kernel<typename decltype(tr)::type, s, pl>;
+            CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            kernel<<<grid, kMmaWarps * 32, smem, st>>>(u.ships, u.ship_b, u.planets, bullet_buffer(b, b->cur), u.meta, actions, q_out,
+                                                       b->n_games, b->K, b->policy_nout, ship_mask, b->d_pol_frags);
+            return ASTRO_OK;
+        }))
+        return r;
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
     return ASTRO_OK;
@@ -3188,16 +2831,10 @@ int astro_explore_controls(AstroBatch* b, double t_in, double t_out, uint32_t se
     CUDA_TRY(cudaSetDevice(b->device));
     const int grid = (b->n_games * b->S + 127) / 128;
     cudaStream_t st = (cudaStream_t)stream;
-#define LAUNCH_EXPLORE(S_, PL_)                                                                                                 \
-    explore_kernel<S_, PL_><<<grid, 128, 0, st>>>(b->bufs.meta, state, actions, b->n_games, ship_mask, b->cfg.dt, t_in, t_out, seed, \
-                                                  (uint32_t)b->first_game, b->step, b->step_base_now)
-    const bool wide = b->PL == ASTRO_MAX_PLANETS_WIDE;
-    if (b->S == 2) {
-        if (wide) LAUNCH_EXPLORE(2, ASTRO_MAX_PLANETS_WIDE); else LAUNCH_EXPLORE(2, ASTRO_MAX_PLANETS);
-    } else {
-        if (wide) LAUNCH_EXPLORE(1, ASTRO_MAX_PLANETS_WIDE); else LAUNCH_EXPLORE(1, ASTRO_MAX_PLANETS);
-    }
-#undef LAUNCH_EXPLORE
+    with_layout(b, [&](auto, auto s, auto pl) {
+        explore_kernel<s, pl><<<grid, 128, 0, st>>>(b->bufs.meta, state, actions, b->n_games, ship_mask, b->cfg.dt, t_in, t_out, seed,
+                                                     (uint32_t)b->first_game, b->step, b->step_base_now);
+    });
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
     return ASTRO_OK;
@@ -3399,15 +3036,10 @@ int astro_export_games(AstroBatch* b, const int32_t* index, int32_t m, const Ast
     const AstroBuffers& u = b->bufs;
     const int grid = (m + 3) / 4;
     cudaStream_t st = (cudaStream_t)stream;
-#define LAUNCH_EXP(R, S_, PL_) \
-    export_kernel<R, S_, PL_><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, current_bullets(b), u.meta, u.episode, index, m, b->n_games, b->K, out->bullet_rows, a)
-#define LAUNCH_EXP_PL(PL_) \
-    do { if (b->precision == 32) { if (b->S == 2) LAUNCH_EXP(float, 2, PL_); else LAUNCH_EXP(float, 1, PL_); } \
-         else { if (b->S == 2) LAUNCH_EXP(double, 2, PL_); else LAUNCH_EXP(double, 1, PL_); } } while (0)
-    if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_EXP_PL(ASTRO_MAX_PLANETS_WIDE);
-    else LAUNCH_EXP_PL(ASTRO_MAX_PLANETS);
-#undef LAUNCH_EXP_PL
-#undef LAUNCH_EXP
+    with_layout(b, [&](auto r, auto s, auto pl) {
+        export_kernel<typename decltype(r)::type, s, pl><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, bullet_buffer(b, b->cur), u.meta,
+                                                                                u.episode, index, m, b->n_games, b->K, out->bullet_rows, a);
+    });
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
     return ASTRO_OK;
@@ -3433,19 +3065,13 @@ int astro_import_games(AstroBatch* b, const int32_t* index, int32_t m, const Ast
     }
     const GameArrays a = to_dev_arrays(in);
     const AstroBuffers& u = b->bufs;
-    const size_t buf_bytes = (size_t)b->n_games * b->K * 4 * (b->precision == 32 ? sizeof(float) : sizeof(double));
-    void* cur = (char*)u.bullets + (size_t)b->cur * buf_bytes;
-    void* other = (char*)u.bullets + (size_t)(b->cur ^ 1) * buf_bytes;
+    void* cur = bullet_buffer(b, b->cur);
+    void* other = bullet_buffer(b, b->cur ^ 1);
     const int grid = (b->n_games / ASTRO_TILE + 3) / 4;
-#define LAUNCH_IMP(R, S_, PL_) \
-    import_kernel<R, S_, PL_><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, cur, other, u.meta, u.episode, src, m, b->n_games, b->K, in->bullet_rows, a)
-#define LAUNCH_IMP_PL(PL_) \
-    do { if (b->precision == 32) { if (b->S == 2) LAUNCH_IMP(float, 2, PL_); else LAUNCH_IMP(float, 1, PL_); } \
-         else { if (b->S == 2) LAUNCH_IMP(double, 2, PL_); else LAUNCH_IMP(double, 1, PL_); } } while (0)
-    if (b->PL == ASTRO_MAX_PLANETS_WIDE) LAUNCH_IMP_PL(ASTRO_MAX_PLANETS_WIDE);
-    else LAUNCH_IMP_PL(ASTRO_MAX_PLANETS);
-#undef LAUNCH_IMP_PL
-#undef LAUNCH_IMP
+    with_layout(b, [&](auto r, auto s, auto pl) {
+        import_kernel<typename decltype(r)::type, s, pl><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, cur, other, u.meta, u.episode,
+                                                                                src, m, b->n_games, b->K, in->bullet_rows, a);
+    });
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
     return ASTRO_OK;
@@ -3719,7 +3345,6 @@ int astro_value_forward(AstroBatch* b, const float* features, int32_t n_items, i
     if (!features || !q_out) return fail(ASTRO_E_INVALID, "null argument");
     if (n_items < 0 || rows < 1) return fail(ASTRO_E_INVALID, "n_items >= 0 and rows >= 1");
     if (n_items == 0) return ASTRO_OK;
-#if ASTRO_POLICY_F16
     CUDA_TRY(cudaSetDevice(b->device));
     cudaStream_t st = (cudaStream_t)stream;
     int grid = ((n_items + 15) / 16 + kMmaWarps - 1) / kMmaWarps;      // a warp takes 16 items at a time
@@ -3735,10 +3360,6 @@ int astro_value_forward(AstroBatch* b, const float* features, int32_t n_items, i
     CUDA_TRY(cudaGetLastError());
     b->launches += 1;
     return ASTRO_OK;
-#else
-    (void)stream;
-    return fail(ASTRO_E_STATE, "astro_value_forward needs the FP16 tensor-core build (ASTRO_POLICY_F16=1)");
-#endif
 }
 
 int astro_stats_peer_create(AstroBatch* b, int32_t rank, int32_t world, uint8_t* handle_out) {

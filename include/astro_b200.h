@@ -429,7 +429,6 @@ int astro_stats_allreduce(AstroBatch* b, int64_t* counters_dev, int32_t clear, v
  *   ASTRO_TICK_NO_FIX=1        the generic tick instantiations instead of the ones with the rollout options fixed at compile time
  *   ASTRO_FUSED_BOTS=0         astro_rollout_device: bot kernel -> tick kernel per tick instead of the ScriptBot inside the tick
  *   ASTRO_LOOP_GRAPH=0         astro_rollout_device: plain launches instead of CUDA graphs of 16 ticks
- *   ASTRO_POLICY_MMA=0         astro_policy_controls: the CUDA-core kernel instead of the tensor-core one
  *   ASTRO_ROLLOUT_CHUNK=n      astro_rollout_host: ticks per copy / launch (default 8 with packed controls, else 4)
  *   ASTRO_HOST_SLICES=n        astro_tick_host: slices of tiles on internal streams (copies of one overlap the kernel of another)
  *   ASTRO_L2_FETCH_GRANULARITY, ASTRO_EXTRA_SMEM   experiment knobs (tools/experiments) */

@@ -410,11 +410,9 @@ def test_observe_script_and_export_import_on_eight_planet_states(precision):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize('mma', ['1', '0'])
-def test_policy_kernels_on_eight_planet_states(mma, monkeypatch):
+def test_policy_kernels_on_eight_planet_states():
     import torch
     from astro_b200 import rl
-    monkeypatch.setenv('ASTRO_POLICY_MMA', mma)
     games = _played_wide(32, N=4096 + 32, ticks=70, seed=4)
     torch.manual_seed(2)
     net = rl.ValueNetwork(solo=False, nout=6).to(games.device)
