@@ -15,7 +15,9 @@
 //     rank inside the game's segment = popc(ballot & segment mask), so the reference order
 //     (stable) is kept.  In HBM the flat list IS the storage order (one dense run per tile, see
 //     the header): a window of 32 list items is one contiguous 512-byte read, and the new list —
-//     survivors and newborn, dense again — is written to the tile's run in the other buffer.
+//     survivors and newborn, dense again — is written to the tile's run in the other buffer.  (The
+//     production rollout's fused form keeps the list in shared memory from tick to tick instead and
+//     writes it once per launch: the resident pool, section 6 of tick_tile.)
 //  B. SHIPS AND PLANETS, thread-per-game from the staged copies: direction, gravity, collisions,
 //     terminal logic, spawn, integration, reset — all coalesced 128-bit accesses.
 //
@@ -84,9 +86,12 @@ struct TileScratchT {              // per warp
     float4 svel[32];               // [lane] OLD ship velocities } for the newborn bullets
     float4 dir[32];                // [lane] sin/cos of both bearings
     uint32_t hits[32];             // [cid] bits 0-1: ship hits found by the bullet loop; bits 8+: np
-    int32_t shift[32];             // [cid] new list: item j of the compacted list moves to j + shift (kDrop: game over)
+    union {
+        int32_t shift[32];         // [cid] new list: item j of the compacted list moves to j + shift (kDrop: game over)
+        uint32_t gcount[32];       // resident pool: [lane] items the bullet loop removed, then the game's next list slot
+    };
     uint16_t gstart[34];           // [cid] first survivor of the game in the compacted list; [n] = survivors of the tile
-    uint8_t ref[W * 32];               // compacted item -> cid
+    uint8_t ref[W * 32];               // compacted item -> cid (resident pool: item -> tag, lane | generation << 5)
     uint32_t used;                     // fresh-game mode: records of the tile's ring consumed since the last refill
 };
 constexpr int kDrop = 0x40000000;
@@ -117,6 +122,15 @@ __device__ __forceinline__ unsigned lds8(unsigned a) { unsigned v; asm volatile(
 __device__ __forceinline__ void sts32(unsigned a, unsigned v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
 __device__ __forceinline__ void sts8(unsigned a, unsigned v) { asm volatile("st.shared.u8 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
 __device__ __forceinline__ void sts16(unsigned a, unsigned v) { asm volatile("st.shared.u16 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
+__device__ __forceinline__ void reds_add(unsigned a, unsigned v) { asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
+__device__ __forceinline__ void reds_or(unsigned a, unsigned v) { asm volatile("red.shared.or.b32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
+// Resident bullet pool (tick_tile, MANY && FIX): the pool size, or kNotResident when the next tick stages its list from HBM.
+constexpr unsigned kNotResident = 0xffffffffu;
+// Tag of a pool item: owning lane in bits 0-4, the game's generation in bit 5 (0xff: past the end, never live).  An item is
+// live iff its generation bit equals bit `lane` of the warp's generation mask.
+__device__ __forceinline__ bool tag_live(unsigned tag, unsigned genmask) {
+    return (tag >> 5) == (__funnelshift_r(genmask, genmask, tag) & 1u);   // (funnel shift: the amount is taken mod 32)
+}
 
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
@@ -432,9 +446,12 @@ template <int S, bool STATS, bool MANY, bool BOT, bool FIX, int PL>
 // (planets and the bullet list always do), and the tile's statistics (`stat_acc`, summed over the launch's ticks).
 __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v, TileScratchT<MANY ? ASTRO_STAGE_WINDOWS_MANY : ASTRO_STAGE_WINDOWS, PL>& t, const unsigned lane,
                                           const unsigned tile_index, const TileIn& in, TileIn& next, const bool last,
-                                          unsigned& stat_acc, const bool have_fire_word) {
+                                          unsigned& stat_acc, const bool have_fire_word, unsigned& pool, unsigned& genmask) {
     using B4 = Body4<float>;
     constexpr int kStageWindows = MANY ? ASTRO_STAGE_WINDOWS_MANY : ASTRO_STAGE_WINDOWS;
+    // `pool` / `genmask` (warp-uniform, kept by the caller from tick to tick): the resident bullet pool of section 6
+    constexpr bool RES = ASTRO_SMEM_ASM && MANY && FIX && !BOT;
+    const bool resident = RES && pool != kNotResident;
     const unsigned full = 0xffffffffu;
     const int g = (int)(tile_index * 32u + lane);
     const Consts& c = p.c;
@@ -521,12 +538,18 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
     const bool nonempty = nb > 0;
     const unsigned ne = __ballot_sync(full, nonempty);
     const unsigned cid = __popc(ne & lt_mask);                    // this game's rank among the games with bullets
+    // a tile whose list does not fit the staging buffer (more than kStageWindows * 32 bullets, rare) takes several rounds
+    const bool multi = !resident && total > (unsigned)kStageWindows * 32u;
+    // the resident pool's per-game rows are indexed by lane (every lane writes its own), except in a tick of several rounds
+    const bool by_lane = RES && !multi;
+    const unsigned fi = by_lane ? lane : cid;
     using Scratch = TileScratchT<kStageWindows, PL>;
 #if ASTRO_SMEM_ASM
     // every hot shared-memory access of the tick goes off this one base register (see lds128 above)
     const unsigned sbase = __shfl_sync(full, (unsigned)__cvta_generic_to_shared(&t), 0);
 #define SOFF(field) (sbase + (unsigned)offsetof(Scratch, field))
-    if (nonempty) sts32(SOFF(hits) + cid * 4u, (unsigned)np << 8);
+    if (by_lane || nonempty) sts32(SOFF(hits) + fi * 4u, (unsigned)np << 8);
+    if (RES) sts32(SOFF(gcount) + lane * 4u, 0u);
 #else
     if (nonempty) t.hits[cid] = (unsigned)np << 8;
 #endif
@@ -576,15 +599,26 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
         }
         cp_async_commit();
     };
-    stage_round(0u);
-    unsigned incl = (unsigned)nb;
+    unsigned my_excl = 0;   // (the resident pool stages nothing and needs no prefix sum)
+    if (!resident) {
+        stage_round(0u);
+        unsigned incl = (unsigned)nb;
 #pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-        unsigned v = __shfl_up_sync(full, incl, d);
-        if ((int)lane >= d) incl += v;
+        for (int d = 1; d < 32; d <<= 1) {
+            unsigned v = __shfl_up_sync(full, incl, d);
+            if ((int)lane >= d) incl += v;
+        }
+        my_excl = incl - (unsigned)nb;
     }
-    const unsigned my_excl = incl - (unsigned)nb;
     const unsigned start_key = nonempty ? my_excl : 0x80000000u;  // empty games never "start"
+#if ASTRO_SMEM_ASM
+    if (RES && !resident && !multi) {
+        // the staged list becomes the pool: every item tagged with its game's lane (generation 0), the tail never live
+        genmask = 0u;
+        for (unsigned i = 0; i < (unsigned)nb; i++) sts8(SOFF(ref) + my_excl + i, lane);
+        if ((total & 31u) != 0u && lane >= (total & 31u)) sts8(SOFF(ref) + (total & ~31u) + lane, 0xffu);
+    }
+#endif
     TL(2);
 
     // ================= 3. ships and planets while the bullets fly ===============================
@@ -595,11 +629,11 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
 #if ASTRO_SMEM_ASM
     sts128(SOFF(sxy) + lane * 16u, make_float4(shv[0].x, shv[1].x, shv[0].y, shv[1].y));
     sts128(SOFF(svel) + lane * 16u, make_float4(shv[0].z, shv[0].w, shv[1].z, shv[1].w));
-    if (nonempty) {
-        sts128(SOFF(fsxy) + cid * 16u, make_float4(shv[0].x, shv[1].x, shv[0].y, shv[1].y));
+    if (by_lane || nonempty) {
+        sts128(SOFF(fsxy) + fi * 16u, make_float4(shv[0].x, shv[1].x, shv[0].y, shv[1].y));
 #pragma unroll
         for (int k = 0; k < PL / 2; k++)
-            sts128(SOFF(fpxy) + (unsigned)k * 512u + cid * 16u, make_float4(plv[2 * k].x, plv[2 * k + 1].x, plv[2 * k].y, plv[2 * k + 1].y));
+            sts128(SOFF(fpxy) + (unsigned)k * 512u + fi * 16u, make_float4(plv[2 * k].x, plv[2 * k + 1].x, plv[2 * k].y, plv[2 * k + 1].y));
     }
 #else
     t.sxy[lane] = make_float4(shv[0].x, shv[1].x, shv[0].y, shv[1].y);
@@ -720,7 +754,6 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
     // buffer (`multi`: more than kStageWindows * 32 bullets, rare) compacts into the list it is
     // reading instead — writes only land on items already consumed — and copies from there.
     unsigned carry = 0, c0 = 0;
-    const bool multi = total > (unsigned)kStageWindows * 32u;
 
     TL(4);  // physics done, new ship / planet state stored
     // (two copies of the loops, one per value of `multi`: the common one — a single round, survivors into shared memory —
@@ -792,15 +825,57 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
             }
         }
     };
+#if ASTRO_SMEM_ASM
+    if (by_lane) {
+        // The resident pool (section 6): item j's game comes from its tag; an item of a game that ended on the previous
+        // tick (generation bit out of date) or past the end is dropped and counted nowhere.  The game's live items that
+        // go (culled or hit a ship) are counted per game: survivors = nb - removed.
+        cp_async_wait_all();
+        __syncwarp();
+        TL(5);
+        const unsigned n_win = ((resident ? pool : total) + 31u) >> 5;
+#pragma unroll 1
+        for (unsigned w = 0; w < n_win; w++) {
+            const unsigned tag = lds8(SOFF(ref) + w * 32u + lane);
+            float4 bv = lds128(bul_s + w * 512u);
+            const unsigned gl = tag & 31u;
+            const bool live = tag_live(tag, genmask);
+            const unsigned fr = sbase + gl * 16u;
+            const float4 sT = lds128(fr + (unsigned)offsetof(Scratch, fsxy));
+            float4 pT[PL / 2];
+#pragma unroll
+            for (int k = 0; k < PL / 2; k++) pT[k] = lds128(fr + (unsigned)offsetof(Scratch, fpxy) + (unsigned)k * 512u);
+            unsigned sh_hits = 0;
+#ifdef ASTRO_EXPERIMENTS
+            bool keep = freeze ? (bv.x + sT.x + pT[0].x + pT[1].x != 123456.0f) : bullet_step_t<S, PL>(bv, sT, pT, t.hits, gl, c, sh_hits);
+#else
+            bool keep = bullet_step_t<S, PL>(bv, sT, pT, t.hits, gl, c, sh_hits);
+#endif
+            if (live && !keep) {   // (a ship hit is never kept)
+                reds_add(SOFF(gcount) + gl * 4u, 1u);
+                if (sh_hits) reds_or(SOFF(hits) + gl * 4u, sh_hits);
+            }
+            keep = keep && live;
+            const unsigned kb = __ballot_sync(full, keep);   // (every lane has loaded its window item by now)
+            const unsigned pos = carry + __popc(kb & lt_mask);
+            if (keep) {
+                sts128(SOFF(bul) + pos * 16u, bv);
+                sts8(SOFF(ref) + pos, tag);
+            }
+            carry += __popc(kb);
+        }
+    } else
+#endif
     if (total != 0u) {
         if (__builtin_expect(multi, 0)) bullet_rounds(std::true_type{});
         else bullet_rounds(std::false_type{});
     }
 #if ASTRO_SMEM_ASM
-    if (lane == 0) sts16(SOFF(gstart) + (unsigned)__popc(ne) * 2u, carry);
+    if (!by_lane && lane == 0) sts16(SOFF(gstart) + (unsigned)__popc(ne) * 2u, carry);
     __syncwarp();
     // first survivor of this lane's game in the compacted list, and one past its last
-    const unsigned g_first = nonempty ? lds16(SOFF(gstart) + cid * 2u) : 0u, g_end = nonempty ? lds16(SOFF(gstart) + cid * 2u + 2u) : 0u;
+    const bool in_gstart = !by_lane && nonempty;
+    const unsigned g_first = in_gstart ? lds16(SOFF(gstart) + cid * 2u) : 0u, g_end = in_gstart ? lds16(SOFF(gstart) + cid * 2u + 2u) : 0u;
 #else
     if (lane == 0) t.gstart[__popc(ne)] = (uint16_t)carry;
     __syncwarp();
@@ -821,6 +896,12 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
         ev = ASTRO_EV_SKIPPED;
     } else {
         int m = 0;   // survivors of this game
+#if ASTRO_SMEM_ASM
+        if (by_lane) {
+            m = nb - (int)lds32(SOFF(gcount) + lane * 4u);
+            hits |= lds32(SOFF(hits) + lane * 4u) & 3u;
+        } else
+#endif
         if (nonempty) {
             m = (int)(g_end - g_first);
 #if ASTRO_SMEM_ASM
@@ -962,56 +1043,122 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
         p.meta[g] = next.meta;
     }
 
-    // ================= 6. the new list: survivors and newborn, dense, into the other buffer =========
-    // Game order, the game's survivors (reference order) then its newborn.  The compacted list in
-    // shared memory is already that, except for the survivors of games that just ended (dropped)
-    // and the newborn (inserted after their game): when the tile has neither, the compacted list
-    // is copied out as it is; otherwise every survivor moves by its game's shift.  Either way a
-    // step stores (nearly) contiguous 512 bytes.
+    // ================= 6. the new list: survivors and newborn =======================================
+    // In HBM: dense, into the other buffer, in game order, the game's survivors (reference order) then
+    // its newborn.  The compacted list in shared memory is already that, except for the survivors of
+    // games that just ended (dropped) and the newborn (inserted after their game): when the tile has
+    // neither, the compacted list is copied out as it is; otherwise every survivor moves by its game's
+    // shift.  Either way a step stores (nearly) contiguous 512 bytes.
+    // The production rollout's fused form (RES) keeps the list in shared memory instead, as a resident
+    // pool, and writes the dense list once per launch (below).
     const unsigned n_surv = carry;
-    const bool moves = __ballot_sync(full, (ev & ASTRO_EV_DONE_MASK) != 0 || n_born != 0) != 0;
-    if (!moves && !multi) {
-#pragma unroll 1
 #if ASTRO_SMEM_ASM
-        for (unsigned j = lane; j < n_surv; j += 32u) ST_STREAM(&list_out[j], lds128(SOFF(bul) + j * 16u));
-#else
-        for (unsigned j = lane; j < n_surv; j += 32u) ST_STREAM(&list_out[j], t.bul[j]);
-#endif
-    } else {
-        unsigned oincl = (unsigned)m_out;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            unsigned v = __shfl_up_sync(full, oincl, d);
-            if ((int)lane >= d) oincl += v;
-        }
-        const unsigned oexcl = oincl - (unsigned)m_out;
-        if (n_born > 0) ST_STREAM(&list_out[oexcl + surv], born[0]);
-        if (n_born > 1) ST_STREAM(&list_out[oexcl + surv + 1u], born[1]);
+    if (RES) {
+        // The resident pool: the compacted survivors stay in `bul`, each with its tag in `ref`, the newborn are appended
+        // after them, and a game that ended flips its generation bit — its items die in the next tick's loop.  Nothing
+        // goes to HBM: inside the launch only this warp reads the tile's list, so the pool need not be dense nor in game
+        // order.  Each game's items stay in reference order among themselves (stable compaction, newborn after the
+        // survivors).  The canonical list — dense, game order — is written once, on the launch's last tick, or when
+        // survivors and newborn would not fit the staging buffer; the next tick then stages from HBM again.
+        genmask ^= __ballot_sync(full, (ev & ASTRO_EV_DONE_MASK) != 0);
+        bool write_out = true;
         if (!multi) {
-#if ASTRO_SMEM_ASM
-            if (nonempty) sts32(SOFF(shift) + cid * 4u, (unsigned)((ev & ASTRO_EV_DONE_MASK) ? kDrop : (int)oexcl - (int)g_first));
-#else
-            if (nonempty) t.shift[cid] = (ev & ASTRO_EV_DONE_MASK) ? kDrop : (int)oexcl - (int)g_first;
-#endif
-            __syncwarp();
-            // (byte offsets from the two shared arrays and the list base: 9 instructions per step)
-            const char* const bul_b = reinterpret_cast<const char*>(t.bul);
-            char* const out_b = reinterpret_cast<char*>(list_out);
-#pragma unroll 1
-            for (unsigned j = lane; j < n_surv; j += 32u) {
-#if ASTRO_SMEM_ASM
-                const int sh = (int)lds32(SOFF(shift) + lds8(SOFF(ref) + j) * 4u);
-                const float4 bv = lds128(SOFF(bul) + j * 16u);
-#else
-                const int sh = t.shift[t.ref[j]];
-                const float4 bv = *reinterpret_cast<const float4*>(bul_b + j * 16u);
-#endif
-                if (sh != kDrop) ST_STREAM(reinterpret_cast<float4*>(out_b + (size_t)((j + (unsigned)sh) * 16u)), bv);
+            const unsigned b1 = __ballot_sync(full, n_born >= 1u), b2 = __ballot_sync(full, n_born >= 2u);
+            const unsigned n_new = n_surv + (unsigned)(__popc(b1) + __popc(b2));
+            if (!last && n_new <= (unsigned)kStageWindows * 32u) {
+                write_out = false;
+                const unsigned at = n_surv + (unsigned)(__popc(b1 & lt_mask) + __popc(b2 & lt_mask));
+                const unsigned tag = lane | (((genmask >> lane) & 1u) << 5);
+                if (n_born > 0) { sts128(SOFF(bul) + at * 16u, born[0]); sts8(SOFF(ref) + at, tag); }
+                if (n_born > 1) { sts128(SOFF(bul) + at * 16u + 16u, born[1]); sts8(SOFF(ref) + at + 1u, tag); }
+                if ((n_new & 31u) != 0u && lane >= (n_new & 31u)) {
+                    sts128(SOFF(bul) + ((n_new & ~31u) + lane) * 16u, make_float4(4.0f, 4.0f, 0.0f, 0.0f));   // (certainly culled)
+                    sts8(SOFF(ref) + (n_new & ~31u) + lane, 0xffu);
+                }
+                pool = n_new;
             }
+        }
+        if (write_out) {
+            pool = kNotResident;
+            unsigned oincl = (unsigned)m_out;
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) {
+                unsigned v = __shfl_up_sync(full, oincl, d);
+                if ((int)lane >= d) oincl += v;
+            }
+            const unsigned oexcl = oincl - (unsigned)m_out;
+            if (n_born > 0) ST_STREAM(&list_out[oexcl + surv], born[0]);
+            if (n_born > 1) ST_STREAM(&list_out[oexcl + surv + 1u], born[1]);
+            if (!multi) {
+                // a stable counting sort by game: item -> first(game) + rank among the game's earlier live items
+                sts32(SOFF(gcount) + lane * 4u, oexcl);
+                __syncwarp();
+#pragma unroll 1
+                for (unsigned j0 = 0; j0 < n_surv; j0 += 32u) {
+                    const unsigned j = j0 + lane, tag = lds8(SOFF(ref) + j), gl = tag & 31u;
+                    const bool live = j < n_surv && tag_live(tag, genmask);     // (games that ended on this tick: dropped)
+                    const unsigned grp = __match_any_sync(full, live ? gl : 32u + lane);
+                    unsigned at = 0;
+                    if (live) {
+                        at = lds32(SOFF(gcount) + gl * 4u);
+                        ST_STREAM(&list_out[at + (unsigned)__popc(grp & lt_mask)], lds128(SOFF(bul) + j * 16u));
+                    }
+                    __syncwarp();
+                    if (live && (grp >> lane) == 1u) sts32(SOFF(gcount) + gl * 4u, at + (unsigned)__popc(grp));
+                    __syncwarp();
+                }
+            } else {
+                // (rare) the survivors sit compacted in the list that was read: every lane copies its game's run
+                for (unsigned k = 0; k < surv; k++) list_out[oexcl + k] = list_in[g_first + k];
+            }
+        }
+    } else
+#endif
+    {
+        const bool moves = __ballot_sync(full, (ev & ASTRO_EV_DONE_MASK) != 0 || n_born != 0) != 0;
+        if (!moves && !multi) {
+#pragma unroll 1
+#if ASTRO_SMEM_ASM
+            for (unsigned j = lane; j < n_surv; j += 32u) ST_STREAM(&list_out[j], lds128(SOFF(bul) + j * 16u));
+#else
+            for (unsigned j = lane; j < n_surv; j += 32u) ST_STREAM(&list_out[j], t.bul[j]);
+#endif
         } else {
-            // (rare) the survivors sit compacted in the list that was read: every lane copies its game's run
-            const unsigned from = g_first;
-            for (unsigned k = 0; k < surv; k++) list_out[oexcl + k] = list_in[from + k];
+            unsigned oincl = (unsigned)m_out;
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) {
+                unsigned v = __shfl_up_sync(full, oincl, d);
+                if ((int)lane >= d) oincl += v;
+            }
+            const unsigned oexcl = oincl - (unsigned)m_out;
+            if (n_born > 0) ST_STREAM(&list_out[oexcl + surv], born[0]);
+            if (n_born > 1) ST_STREAM(&list_out[oexcl + surv + 1u], born[1]);
+            if (!multi) {
+#if ASTRO_SMEM_ASM
+                if (nonempty) sts32(SOFF(shift) + cid * 4u, (unsigned)((ev & ASTRO_EV_DONE_MASK) ? kDrop : (int)oexcl - (int)g_first));
+#else
+                if (nonempty) t.shift[cid] = (ev & ASTRO_EV_DONE_MASK) ? kDrop : (int)oexcl - (int)g_first;
+#endif
+                __syncwarp();
+                // (byte offsets from the two shared arrays and the list base: 9 instructions per step)
+                const char* const bul_b = reinterpret_cast<const char*>(t.bul);
+                char* const out_b = reinterpret_cast<char*>(list_out);
+#pragma unroll 1
+                for (unsigned j = lane; j < n_surv; j += 32u) {
+#if ASTRO_SMEM_ASM
+                    const int sh = (int)lds32(SOFF(shift) + lds8(SOFF(ref) + j) * 4u);
+                    const float4 bv = lds128(SOFF(bul) + j * 16u);
+#else
+                    const int sh = t.shift[t.ref[j]];
+                    const float4 bv = *reinterpret_cast<const float4*>(bul_b + j * 16u);
+#endif
+                    if (sh != kDrop) ST_STREAM(reinterpret_cast<float4*>(out_b + (size_t)((j + (unsigned)sh) * 16u)), bv);
+                }
+            } else {
+                // (rare) the survivors sit compacted in the list that was read: every lane copies its game's run
+                const unsigned from = g_first;
+                for (unsigned k = 0; k < surv; k++) list_out[oexcl + k] = list_in[from + k];
+            }
         }
     }
     if (!FIX && v.reward) {
@@ -1096,6 +1243,7 @@ __global__ void __launch_bounds__(kTickThreads, BOT ? ASTRO_TICK_MIN_BLOCKS_BOT 
     // (MANY = false: the one-tick launch, without the loop around it — the loop form costs a single tick 6 %)
     TileIn in, next;
     unsigned stat_acc = 0;
+    unsigned pool = kNotResident, genmask = 0u;   // (the resident bullet pool of tick_tile, section 6: MANY && FIX only)
     TileScratch& scratch = s_tiles[kTickWarps == 1 ? 0 : (threadIdx.x >> 5)];
     // fresh-game mode: how many of the tile's pre-created games have been used since the last refill — requested with the
     // tile's rows, parked in shared memory once they are all on their way (a wait here would cost a round trip)
@@ -1116,7 +1264,7 @@ __global__ void __launch_bounds__(kTickThreads, BOT ? ASTRO_TICK_MIN_BLOCKS_BOT 
         }
         if (MANY) in.fire_word = p.fire_bits[min(meta_tick<PL>(in.meta), (uint32_t)p.n_sched_ticks - 1u) >> 5];
         // (one-warp CTAs: the scratch is s_tiles[0], every shared address a compile-time constant — no base register)
-        tick_tile<S, STATS, MANY, BOT, FIX, PL>(p, v, scratch, lane, tile, in, next, !MANY || k + 1u == (unsigned)p.n_fused, stat_acc, MANY);
+        tick_tile<S, STATS, MANY, BOT, FIX, PL>(p, v, scratch, lane, tile, in, next, !MANY || k + 1u == (unsigned)p.n_fused, stat_acc, MANY, pool, genmask);
         if (MANY) {
             // The next tick of this tile: meta, ships and bearings are handed on in registers (they were stored as
             // well), so it starts its prefix sums and list requests at once; only the planet rows are loaded.  The
@@ -1174,6 +1322,7 @@ __device__ __forceinline__ void tick_f32_body(const TickParams& p) {
     // (MANY = false: the one-tick launch, without the loop around it — the loop form costs a single tick 6 %)
     TileIn in, next;
     unsigned stat_acc = 0;
+    unsigned pool = kNotResident, genmask = 0u;   // (the resident bullet pool of tick_tile, section 6: MANY && FIX only)
     TileScratch& scratch = s_tiles[kTickWarps == 1 ? 0 : (threadIdx.x >> 5)];
     // fresh-game mode: how many of the tile's pre-created games have been used since the last refill — requested with the
     // tile's rows, parked in shared memory once they are all on their way (a wait here would cost a round trip)
@@ -1194,7 +1343,7 @@ __device__ __forceinline__ void tick_f32_body(const TickParams& p) {
         }
         if (MANY) in.fire_word = p.fire_bits[min(meta_tick<PL>(in.meta), (uint32_t)p.n_sched_ticks - 1u) >> 5];
         // (one-warp CTAs: the scratch is s_tiles[0], every shared address a compile-time constant — no base register)
-        tick_tile<S, STATS, MANY, BOT, FIX, PL>(p, v, scratch, lane, tile, in, next, !MANY || k + 1u == (unsigned)p.n_fused, stat_acc, MANY);
+        tick_tile<S, STATS, MANY, BOT, FIX, PL>(p, v, scratch, lane, tile, in, next, !MANY || k + 1u == (unsigned)p.n_fused, stat_acc, MANY, pool, genmask);
         if (MANY) {
             // The next tick of this tile: meta, ships and bearings are handed on in registers (they were stored as
             // well), so it starts its prefix sums and list requests at once; only the planet rows are loaded.  The
