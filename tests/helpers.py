@@ -62,3 +62,68 @@ def start_from_pool(games, pool, seed, first_game):
     n = games.n
     pick = rng.pool_pick(seed, first_game + np.arange(n), np.zeros(n, dtype=np.uint32), pool['ships'].shape[0])
     return pick
+
+
+def stress_fill(K, seed):
+    """A start(games) that fills every game's bullet pool: random bullets (a share parked exactly at the arena bound),
+    half the games at the cap K, every 8th game a full pool parked in a quiet corner (nothing despawns: overflow on
+    fire ticks), tick counters spread over the first fire ticks."""
+    def fill(games):
+        r = np.random.RandomState(seed)
+        n = games.n
+        arr = games.get_arrays()
+        bl = np.concatenate([r.uniform(-1.3, 1.3, (n, K, 2)), r.uniform(-2.0, 2.0, (n, K, 2))], axis=2)
+        # a share of bullets parked exactly at / next to the arena bound and inside planets
+        edge = r.rand(n, K) < 0.05
+        bl[..., 0][edge] = np.where(r.rand(int(edge.sum())) < 0.5, 1.0, -1.0)
+        nb = r.randint(0, K + 1, n)
+        nb[r.rand(n) < 0.5] = K
+        # every 8th game: a full pool parked in a quiet corner (nothing despawns) -> overflow on fire ticks
+        quiet = np.arange(n) % 8 == 0
+        q = int(quiet.sum())
+        bl[quiet] = np.concatenate([0.95 + r.uniform(-0.01, 0.01, (q, K, 1)), r.uniform(-0.01, 0.01, (q, K, 1)),
+                                    np.zeros((q, K, 2))], axis=2)
+        nb[quiet] = K
+        ticks = r.randint(0, 40, n)       # spread over fire ticks (14, 29)
+        games.set_arrays(arr['ships'], arr['planets'], arr['n_planets'], bl, nb, ticks)
+    return fill
+
+
+# ---- the production rollout's options: packed controls in, event planes out, auto-reset -------------------------
+
+def tile_sums(nb):
+    """Bullets per 32-game tile."""
+    return np.bincount(np.arange(nb.shape[0]) // 32, weights=nb)
+
+
+def run_launches(g, packed, launches, tile_totals=None, stats=True):
+    """Ticks of `packed` (uint8 cuda [T, n_pad]) in astro_tick_many launches of the given lengths, with event planes
+    and auto-reset; returns the event planes of every tick.  tile_totals: list receiving each tile's bullet count after
+    every launch."""
+    import torch
+    T = packed.shape[0]
+    assert sum(launches) == T
+    planes = torch.zeros(g.planes_shape(T), dtype=torch.int32, device='cuda')
+    k = 0
+    for n in launches:
+        g.step_many(n, packed[k:k + n], events=planes[k:k + n], auto_reset=True, stats=stats, packed=True, planes=True)
+        k += n
+        if tile_totals is not None:
+            tile_totals.append(tile_sums(g.get_arrays()['n_bullets']))
+    torch.cuda.synchronize()
+    return planes.cpu().numpy()
+
+
+def check_same(a_games, b_games, ev_a, ev_b):
+    """Two batches hold the same state element for element (every bullet list in order), the same events and the same
+    statistics."""
+    a, b = a_games.get_arrays(), b_games.get_arrays()
+    assert a.keys() == b.keys()
+    for key in a:
+        if key != 'bullets':
+            assert np.array_equal(a[key], b[key]), key
+    nb = b['n_bullets']
+    live = np.arange(a['bullets'].shape[1])[None, :] < nb[:, None]
+    assert np.array_equal(a['bullets'][live], b['bullets'][live])        # every list, item for item, in order
+    assert np.array_equal(ev_a, ev_b)
+    assert a_games.stats() == b_games.stats()

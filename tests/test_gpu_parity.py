@@ -300,26 +300,7 @@ def test_f32_free_running_statistics_match_the_f64_build():
 
 # ------------------------------------------------------------------ config #3: 65,536 games, full pools
 
-def _stress_fill(K, seed):
-    def fill(games):
-        r = np.random.RandomState(seed)
-        n = games.n
-        arr = games.get_arrays()
-        bl = np.concatenate([r.uniform(-1.3, 1.3, (n, K, 2)), r.uniform(-2.0, 2.0, (n, K, 2))], axis=2)
-        # a share of bullets parked exactly at / next to the arena bound and inside planets
-        edge = r.rand(n, K) < 0.05
-        bl[..., 0][edge] = np.where(r.rand(int(edge.sum())) < 0.5, 1.0, -1.0)
-        nb = r.randint(0, K + 1, n)
-        nb[r.rand(n) < 0.5] = K
-        # every 8th game: a full pool parked in a quiet corner (nothing despawns) -> overflow on fire ticks
-        quiet = np.arange(n) % 8 == 0
-        q = int(quiet.sum())
-        bl[quiet] = np.concatenate([0.95 + r.uniform(-0.01, 0.01, (q, K, 1)), r.uniform(-0.01, 0.01, (q, K, 1)),
-                                    np.zeros((q, K, 2))], axis=2)
-        nb[quiet] = K
-        ticks = r.randint(0, 40, n)       # spread over fire ticks (14, 29)
-        games.set_arrays(arr['ships'], arr['planets'], arr['n_planets'], bl, nb, ticks)
-    return fill
+_stress_fill = H.stress_fill
 
 
 @pytest.mark.parametrize('K', [400, 32])

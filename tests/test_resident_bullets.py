@@ -9,6 +9,7 @@ import pytest
 from astro_b200 import core
 from astro_b200.pool import make_pool
 from astro_b200.schedule import Schedule
+from tests import helpers as H
 
 pytestmark = pytest.mark.gpu
 
@@ -38,38 +39,7 @@ def _controls(g, T, seed):
     return g.pack_controls(acts).cuda()
 
 
-def _run(g, packed, launches, tile_totals=None):
-    """Ticks of `packed` in launches of the given lengths; event planes of every tick.  tile_totals: list receiving each
-    tile's bullet count after every launch."""
-    import torch
-    T = packed.shape[0]
-    assert sum(launches) == T
-    planes = torch.zeros(g.planes_shape(T), dtype=torch.int32, device='cuda')
-    k = 0
-    for n in launches:
-        g.step_many(n, packed[k:k + n], events=planes[k:k + n], auto_reset=True, packed=True, planes=True)
-        k += n
-        if tile_totals is not None:
-            tile_totals.append(_tile_sums(g.get_arrays()['n_bullets']))
-    torch.cuda.synchronize()
-    return planes.cpu().numpy()
-
-
-def _check_same(fused, single, ev_fused, ev_single):
-    a, b = fused.get_arrays(), single.get_arrays()
-    assert a.keys() == b.keys()
-    for key in a:
-        if key != 'bullets':
-            assert np.array_equal(a[key], b[key]), key
-    nb = b['n_bullets']
-    live = np.arange(a['bullets'].shape[1])[None, :] < nb[:, None]
-    assert np.array_equal(a['bullets'][live], b['bullets'][live])        # every list, item for item, in order
-    assert np.array_equal(ev_fused, ev_single)
-    assert fused.stats() == single.stats()
-
-
-def _tile_sums(nb):
-    return np.bincount(np.arange(nb.shape[0]) // 32, weights=nb)
+_run, _check_same, _tile_sums = H.run_launches, H.check_same, H.tile_sums
 
 
 def _compare(K, launches, seed=0, **kw):
