@@ -631,20 +631,37 @@ class BatchedGames:
 
     # ---- whole game loops on the device -------------------------------------------------------------
     def rollout_device(self, n_ticks, bots=('stream', 'stream'), auto_reset=True, stats=True, avoid_distance=0.1,
-                       avoid_threshold=0.45):
+                       avoid_threshold=0.45, record=None):
         """`n_ticks` of the play loop (core.play, core.py:377-410; rl.train's games, rl.py:350-374) for
         every game without the host between ticks.  bots: one of 'stream' (counter-stream random
         controls, both ships), 'script' (script.ScriptBot), 'policy' (greedy network loaded with
         set_policy), 'explore' (that network with rl.EpsilonGreedy laid over it: set_exploration), 'nothing'
-        (script.NothingBot) per ship.  Outcomes accumulate in stats()."""
+        (script.NothingBot) per ship.  Outcomes accumulate in stats().
+        record: a RecordRing (record_ring()) that receives every tick's controls, events and — if it holds them — the
+        observations (astro_rollout_device_record); the results are the same as without it."""
         if isinstance(bots, str):
             bots = (bots,) * self.S
         modes = [nat.BOT_MODES[b] for b in bots] + [0]
         flags = (nat.TICK_AUTO_RESET if auto_reset else 0) | (0 if stats else nat.TICK_NO_STATS) | self.tick_flags
-        nat.check(nat.lib().astro_rollout_device(self._h, int(n_ticks), modes[0], modes[1], float(avoid_distance),
-                                                 float(avoid_threshold), self._actions.data_ptr(), self._events.data_ptr(),
-                                                 flags, self._stream()))
-        self.step_index += int(n_ticks)
+        n = int(n_ticks)
+        if record is None:
+            nat.check(nat.lib().astro_rollout_device(self._h, n, modes[0], modes[1], float(avoid_distance),
+                                                     float(avoid_threshold), self._actions.data_ptr(), self._events.data_ptr(),
+                                                     flags, self._stream()))
+        else:
+            if (record.n_pad, record.S) != (self.n_pad, self.S) or record.device != self.device:
+                raise ValueError('the ring was made for another batch layout (record_ring of this batch)')
+            nat.check(nat.lib().astro_rollout_device_record(self._h, n, modes[0], modes[1], float(avoid_distance),
+                                                            float(avoid_threshold), self._actions.data_ptr(), C.byref(record._ring),
+                                                            flags, self._stream()))
+            record._recorded(self.step_index, n)
+        self.step_index += n
+
+    def record_ring(self, ticks, observations=True, n_rows=None):
+        """A RecordRing of `ticks` rows for rollout_device(..., record=ring): per tick the controls, events and (observations=True)
+        ship 0's observation of the state before the tick (n_rows as observe(); default the smallest multiple of 4 that holds
+        the planet slots and bullet_cap).  A rollout_device call records at most ticks - 1 ticks."""
+        return RecordRing(self, ticks, observations, n_rows)
 
     # ---- n-step replay ingestion ---------------------------------------------------------------------
     def nstep_experiences(self, events, carry=None, n_steps=100, discount=0.995):
@@ -717,3 +734,100 @@ class BatchedGames:
     @property
     def launches(self):
         return int(nat.lib().astro_launch_count(self._h))
+
+
+class RecordRing:
+    """The per-tick log of device rollouts (AstroRecordRing, astro_rollout_device_record) — what rl.QBotTrainer keeps per bot to
+    build its Experiences (rl.py:212-228) — as cuda tensors, row = stream step % ticks:
+      controls      uint8 [ticks, n_pad, S]                the control each ship flew on that tick
+      events        uint8 [ticks, n_pad]                   that tick's ASTRO_EV_* byte (what step() returns as events)
+      observations  float32 [ticks, n_pad, n_rows, D]      ship 0's observation (observe(shared=True)) of the state before the
+                    or None                                tick; a rollout call also records the state after its last tick
+    Rows of stream steps first .. end - 1 hold an unbroken history (a rollout that does not continue where the last one ended
+    starts a new one)."""
+
+    def __init__(self, games, ticks, observations=True, n_rows=None):
+        torch = _torch()
+        R = int(ticks)
+        if R < 2:
+            raise ValueError('a ring needs at least 2 rows')
+        self.ticks, self.n_pad, self.S, self.D, self.device = R, games.n_pad, games.S, games.D, games.device
+        self.n_rows = -(-(games.PL + games.K) // 4) * 4 if n_rows is None else int(n_rows)
+        self.controls = torch.zeros((R, self.n_pad, self.S), dtype=torch.uint8, device=self.device)
+        self.events = torch.zeros((R, self.n_pad), dtype=torch.uint8, device=self.device)
+        self.observations = (torch.zeros((R, self.n_pad, self.n_rows, self.D), dtype=torch.float32, device=self.device)
+                             if observations else None)
+        self._ring = nat.AstroRecordRing(R, self.n_rows, self.controls.data_ptr(), self.events.data_ptr(),
+                                         None if self.observations is None else self.observations.data_ptr())
+        self.first = self.end = None
+
+    def _recorded(self, s0, n):
+        if self.end != s0:
+            self.first = s0
+        self.end = s0 + n
+        # row end % R now holds the observation of step `end`: the controls / events of step end - R are gone with it
+        self.first = max(self.first, self.end + 1 - self.ticks)
+
+    def _rows(self, t0, n):
+        """Ring rows of stream steps t0 .. t0 + n - 1 as an index tensor."""
+        torch = _torch()
+        return (torch.arange(t0, t0 + n, device=self.device) % self.ticks)
+
+    def window_events(self, n_ticks):
+        """The events of the last `n_ticks` recorded ticks, contiguous uint8 [n_ticks, n_pad]: the `events` input of
+        BatchedGames.nstep_experiences (a view when the window does not wrap around the ring)."""
+        T = int(n_ticks)
+        if self.end is None or T > self.end - self.first:
+            raise ValueError('the ring holds %d recorded ticks, not %d' % (0 if self.end is None else self.end - self.first, T))
+        a = (self.end - T) % self.ticks
+        if a + T <= self.ticks:
+            return self.events[a:a + T]
+        return self.events[self._rows(self.end - T, T)]
+
+    def _view_of(self, rows, game, ship):
+        """Observation rows [E, n_rows, D] of (ring row, game) seen by `ship`: ship 1 sees ship 0's block with the two ship column
+        groups exchanged (core.roll_ships, core.py:306-327; equal to observe(shared=False)[:, 1])."""
+        torch = _torch()
+        x = self.observations[rows, game]
+        if self.S == 2:
+            swap = torch.tensor([0, 6, 7, 8, 9, 10, 1, 2, 3, 4, 5, 11, 12, 13, 14], device=self.device)
+            x = torch.where((ship == 1)[:, None, None], x[..., swap], x)
+        return x
+
+    def experiences(self, reward, discount, nxt, n_steps):
+        """The Experiences (rl.py:212-228) of one nstep_experiences call over the last window of this ring
+        (nstep_experiences(ring.window_events(T), ...)): one entry per (state, action) pair it flushed, as cuda tensors
+          features       float32 [E, n_rows, D]  the bot's own view of the pair's state (ship 1: column groups exchanged)
+          action         uint8 [E]               the control it flew
+          reward, discount float32 [E]           the n-step reward and discount
+          next_features  float32 [E, n_rows, D]  the bot's view of the new state; all -1 (a finished game) when terminal
+          terminal       bool [E]                the new state is None (the game ended)
+          game, ship     int64 [E]
+          tick           int64 [E]               the stream step of the pair's tick
+        Pairs carried from earlier windows refer to their ticks, so the ring must hold n_steps ticks before the window as well
+        as the window and the state after it: ticks >= n_steps + T + 1."""
+        torch = _torch()
+        if self.observations is None:
+            raise ValueError('experiences need a ring that records observations')
+        n_steps = int(n_steps)
+        T = int(nxt.shape[0]) - n_steps
+        if tuple(nxt.shape) != (n_steps + T, self.n_pad, self.S) or T < 0:
+            raise ValueError('nxt must be [n_steps + T, %d, %d] as nstep_experiences returns it' % (self.n_pad, self.S))
+        if self.ticks < n_steps + T + 1:
+            raise ValueError('a ring of %d rows cannot hold the %d ticks before a window of %d ticks, the window and the state '
+                             'after it: it needs ticks >= n_steps + T + 1 = %d' % (self.ticks, n_steps, T, n_steps + T + 1))
+        if self.end is None or T > self.end - self.first:
+            raise ValueError('the ring does not hold the last %d ticks' % T)
+        s0 = self.end - T
+        row, game, ship = (nxt >= -1).nonzero(as_tuple=True)
+        tick = s0 + row - n_steps
+        if tick.numel() and int(tick.min()) < self.first:
+            raise ValueError('a carried pair refers to stream step %d, before the ring\'s history (from %d)' % (int(tick.min()), self.first))
+        at = tick % self.ticks
+        nx = nxt[row, game, ship]
+        terminal = nx == -1
+        next_features = self._view_of((s0 + nx.clamp(min=0)) % self.ticks, game, ship)
+        next_features = torch.where(terminal[:, None, None], torch.full_like(next_features, -1.0), next_features)
+        return dict(features=self._view_of(at, game, ship), action=self.controls[at, game, ship],
+                    reward=reward[row, game, ship], discount=discount[row, game, ship], next_features=next_features,
+                    terminal=terminal, game=game, ship=ship, tick=tick)

@@ -73,6 +73,11 @@ struct TickParams {
     int32_t bot_modes, pad2_;         // bots evaluated inside the tick (tick_f32_kernel<..., BOT>): ASTRO_BOT_* of ship s in bits 4s..4s+3
     ScriptParams script;
     Consts c;
+    // astro_rollout_device_record (tick_f32 kernels, non-FIX forms): the tick at stream step s stores its controls and event
+    // byte into row s % rec_ticks.  Appended last so that no other parameter moves.
+    uint8_t* rec_controls;            // u8 [rec_ticks][n_games][S], or NULL together with rec_events
+    uint8_t* rec_events;              // u8 [rec_ticks][n_games]
+    uint32_t rec_ticks, pad3_;
 };
 
 
@@ -637,7 +642,7 @@ template <typename R, int S, bool BOTH, int PL>
 __global__ void __launch_bounds__(kObserveWarps * 32)
 observe_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_, const void* __restrict__ planets_,
                const void* __restrict__ bullets_, const uint32_t* __restrict__ meta_, float* __restrict__ obs,
-               int n_games, int K, int n_rows) {
+               int n_games, int K, int n_rows, uint32_t ring_ticks, uint32_t step, const uint32_t* __restrict__ step_base) {
     using B4 = Body4<R>;
     constexpr int D = 1 + 5 * S + 4;
     constexpr int P = (BOTH && S == 2) ? 2 : 1;
@@ -700,6 +705,9 @@ observe_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_
     __syncwarp();
     if (lane == 0) {
         float* out = obs + (size_t)g * P * per;
+        // astro_rollout_device_record: obs is a ring of ring_ticks blocks, the block of stream step s in row s % ring_ticks
+        // (inside a captured chunk of the bot loop the stream step is *step_base + step)
+        if (ring_ticks) out += (size_t)((step + (step_base ? *step_base : 0u)) % ring_ticks) * n_games * P * per;
         asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(out),
                      "r"((unsigned)__cvta_generic_to_shared(rows)), "r"((unsigned)(P * per * 4))
                      : "memory");
@@ -1888,6 +1896,7 @@ struct LoopGraph {        // a captured chunk of the bot loop (astro_rollout_dev
     double avoid_distance, avoid_threshold;
     uint8_t* actions;
     uint8_t* events;
+    AstroRecordRing rec;  // the recording ring the chunk writes (its row is read from the device step word, not captured)
     int64_t epoch;
     int32_t launches;     // kernels of one replay
 };
@@ -1939,6 +1948,7 @@ struct AstroBatch {
     cudaEvent_t loop_in, loop_out;
     int64_t config_epoch;         // bumped by every call that changes what a captured chunk depends on
     int32_t bot_modes_now;        // != 0 while astro_rollout_device runs ticks whose bots are evaluated inside the tick kernel
+    AstroRecordRing rec_now;      // astro_rollout_device_record: the ring of the running call (events == NULL: none)
     ScriptParams script_now;
     // fresh-game mode (astro_fresh_games_enable): per-tile rings of pre-created games fed from the generate_configs stream
     FreshState* fresh;
@@ -2053,6 +2063,11 @@ void fill_params(const AstroBatch* b, TickParams& p) {
     p.step_base = b->step_base_now;
     p.first_game = (uint32_t)b->first_game;
     p.c = b->c;
+    if (b->rec_now.events) {
+        p.rec_controls = b->rec_now.controls;
+        p.rec_events = b->rec_now.events;
+        p.rec_ticks = (uint32_t)b->rec_now.ticks;
+    }
 }
 
 template <typename R, int S, int PL>
@@ -2074,7 +2089,7 @@ cudaError_t launch_tick_f32(const TickParams& p, cudaStream_t st) {
     // from the pool — have instantiations of their own (tick_f32.cuh, FIX) in which those options are compile-time constants:
     // 56.4 against 60.8 us per tick at 20 ticks per launch (same box).  ASTRO_TICK_NO_FIX=1: the generic instantiations (A/B).
     static const bool no_fix = getenv("ASTRO_TICK_NO_FIX") && atoi(getenv("ASTRO_TICK_NO_FIX")) != 0;
-    const bool fix = S == 2 && !no_fix && !p.bot_modes && p.actions && p.events && !p.reward && !p.done && !p.ring && !p.step_base && !p.game_pos && p.pool_size > 0 &&
+    const bool fix = S == 2 && !no_fix && !p.bot_modes && p.actions && p.events && !p.reward && !p.done && !p.ring && !p.step_base && !p.game_pos && !p.rec_events && p.pool_size > 0 &&
                      (p.flags & (ASTRO_TICK_PACKED_CONTROLS | ASTRO_TICK_EVENT_PLANES | ASTRO_TICK_AUTO_RESET)) ==
                          (ASTRO_TICK_PACKED_CONTROLS | ASTRO_TICK_EVENT_PLANES | ASTRO_TICK_AUTO_RESET) && !(p.flags & 1024);
     if (p.bot_modes) {              // bots inside the tick: the many-tick form, whatever n_fused
@@ -2629,23 +2644,31 @@ int astro_reset_done(AstroBatch* b, void* stream) {
     return ASTRO_OK;
 }
 
-static int observe_impl(AstroBatch* b, float* obs, int32_t n_rows, bool both, void* stream) {
-    if (int r = check(b, true)) return r;
+static int observe_args(const AstroBatch* b, const float* obs, int32_t n_rows, bool both) {
     if (!obs) return fail(ASTRO_E_INVALID, "null obs");
     const int D = 1 + 5 * b->S + 4;
     if (n_rows < b->PL + b->K) return fail(ASTRO_E_INVALID, "n_rows %d < %d planet slots + bullet_cap %d", n_rows, b->PL, b->K);
     if ((n_rows * D) % 4) return fail(ASTRO_E_INVALID, "n_rows * %d must be a multiple of 4", D);
     if ((uintptr_t)obs & 15) return fail(ASTRO_E_INVALID, "obs must be 16-byte aligned");
+    if ((size_t)kObserveWarps * observe_warp_floats(n_rows, D, b->S, (both && b->S == 2) ? 2 : 1) * sizeof(float) > 200 * 1024)
+        return fail(ASTRO_E_INVALID, "n_rows %d too large for the staging buffer", n_rows);
+    return ASTRO_OK;
+}
+
+// ring_ticks > 0: obs is a recording ring (AstroRecordRing.observations) and the block goes to the row of the current stream step
+static int observe_impl(AstroBatch* b, float* obs, int32_t n_rows, bool both, void* stream, uint32_t ring_ticks = 0) {
+    if (int r = check(b, true)) return r;
+    if (int r = observe_args(b, obs, n_rows, both)) return r;
     CUDA_TRY(cudaSetDevice(b->device));
+    const int D = 1 + 5 * b->S + 4;
     const size_t smem = (size_t)kObserveWarps * observe_warp_floats(n_rows, D, b->S, (both && b->S == 2) ? 2 : 1) * sizeof(float);
-    if (smem > 200 * 1024) return fail(ASTRO_E_INVALID, "n_rows %d too large for the staging buffer", n_rows);
     const int grid = (b->n_games + kObserveWarps - 1) / kObserveWarps;
     cudaStream_t st = (cudaStream_t)stream;
     const AstroBuffers& u = b->bufs;
     auto launch = [&](auto kernel) {
         CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         kernel<<<grid, kObserveWarps * 32, smem, st>>>(u.ships, u.ship_b, u.planets, bullet_buffer(b, b->cur), u.meta, obs, b->n_games,
-                                                       b->K, n_rows);
+                                                       b->K, n_rows, ring_ticks, b->step, b->step_base_now);
         return ASTRO_OK;
     };
     if (int r = with_layout(b, [&](auto tr, auto s, auto pl) {
@@ -2866,7 +2889,9 @@ static int rollout_chunks(AstroBatch* b, int n_chunks, const int* modes, double 
         for (int i = 0; i < 2; i++) {
             LoopGraph& q = b->loop_graph[i];
             if (q.exec && q.epoch == b->config_epoch && q.cur == b->cur && q.flags == flags && q.modes[0] == modes[0] && q.modes[1] == modes[1] &&
-                q.avoid_distance == avoid_distance && q.avoid_threshold == avoid_threshold && q.actions == actions && q.events == events)
+                q.avoid_distance == avoid_distance && q.avoid_threshold == avoid_threshold && q.actions == actions && q.events == events &&
+                q.rec.ticks == b->rec_now.ticks && q.rec.n_rows == b->rec_now.n_rows && q.rec.controls == b->rec_now.controls &&
+                q.rec.events == b->rec_now.events && q.rec.observations == b->rec_now.observations)
                 g = &q;
         }
         if (!g) {
@@ -2896,6 +2921,7 @@ static int rollout_chunks(AstroBatch* b, int n_chunks, const int* modes, double 
             if (ei != cudaSuccess) { g->exec = nullptr; return fail(ASTRO_E_CUDA, "bot-loop graph: %s", cudaGetErrorString(ei)); }
             g->epoch = b->config_epoch; g->cur = b->cur; g->flags = flags; g->modes[0] = modes[0]; g->modes[1] = modes[1];
             g->avoid_distance = avoid_distance; g->avoid_threshold = avoid_threshold; g->actions = actions; g->events = events;
+            g->rec = b->rec_now;
         }
         CUDA_TRY(cudaGraphLaunch(g->exec, ls));
         b->step += (uint32_t)kLoopChunk;
@@ -2908,8 +2934,9 @@ static int rollout_chunks(AstroBatch* b, int n_chunks, const int* modes, double 
     return ASTRO_OK;
 }
 
-int astro_rollout_device(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, int32_t ship1_mode, double avoid_distance,
-                         double avoid_threshold, uint8_t* actions, uint8_t* events, int32_t flags, void* stream) {
+// astro_rollout_device, recording into b->rec_now when its events array is set (astro_rollout_device_record)
+static int rollout_device(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, int32_t ship1_mode, double avoid_distance,
+                          double avoid_threshold, uint8_t* actions, uint8_t* events, int32_t flags, void* stream) {
     if (int r = check(b, true)) return r;
     if (n_ticks < 0) return fail(ASTRO_E_INVALID, "n_ticks < 0");
     const int modes[2] = {ship0_mode, b->S == 2 ? ship1_mode : ship0_mode};
@@ -2930,7 +2957,10 @@ int astro_rollout_device(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, int
     cudaStream_t st = (cudaStream_t)stream;
     CUDA_TRY(cudaSetDevice(b->device));
     if (any_idle) CUDA_TRY(cudaMemsetAsync(actions, 2, (size_t)b->n_games * b->S, st));  // script.NothingBot: control 2
-    if (all_stream) {
+    // Recording: the tick kernel stores each tick's controls and events itself, so the two fast paths below keep their launches;
+    // observations are taken by observe_kernel before every tick, which needs the per-tick loop at the end.
+    float* const rec_obs = b->rec_now.observations;
+    if (all_stream && !rec_obs) {
         // no bot between the ticks: the ticks of a tile run back to back inside the launches; `events` keeps the last tick's
         if (n_ticks > 1) if (int r = do_ticks(b, nullptr, nullptr, nullptr, nullptr, flags, st, n_ticks - 1)) return r;
         return n_ticks > 0 ? do_ticks(b, nullptr, nullptr, nullptr, events, flags, st, 1) : ASTRO_OK;
@@ -2941,8 +2971,8 @@ int astro_rollout_device(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, int
     // and always take the bot kernel -> tick kernel loop below.
     {
         const char* fb = getenv("ASTRO_FUSED_BOTS");
-        if (!any_policy && b->precision == 32 && b->PL == ASTRO_MAX_PLANETS && !(flags & ASTRO_TICK_GENERIC_KERNEL) && !(fb && atoi(fb) == 0) &&
-            n_ticks > 0) {
+        if (!any_policy && !rec_obs && b->precision == 32 && b->PL == ASTRO_MAX_PLANETS && !(flags & ASTRO_TICK_GENERIC_KERNEL) &&
+            !(fb && atoi(fb) == 0) && n_ticks > 0) {
             b->bot_modes_now = modes[0] | (modes[1] << 4);
             ScriptParams& q = b->script_now;
             q.radius = b->cfg.planet_radius + b->cfg.ship_radius;
@@ -2976,7 +3006,38 @@ int astro_rollout_device(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, int
     for (int k = k_done; k < n_ticks; k++) {
         if (int r = rollout_one_tick(b, modes, avoid_distance, avoid_threshold, actions, events, flags, st)) return r;
     }
+    // the state after the last tick: the new state of the pairs that flush on it
+    if (rec_obs) return observe_impl(b, rec_obs, b->rec_now.n_rows, false, stream, (uint32_t)b->rec_now.ticks);
     return ASTRO_OK;
+}
+
+int astro_rollout_device(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, int32_t ship1_mode, double avoid_distance,
+                         double avoid_threshold, uint8_t* actions, uint8_t* events, int32_t flags, void* stream) {
+    return rollout_device(b, n_ticks, ship0_mode, ship1_mode, avoid_distance, avoid_threshold, actions, events, flags, stream);
+}
+
+int astro_rollout_device_record(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, int32_t ship1_mode, double avoid_distance,
+                                double avoid_threshold, uint8_t* actions, const AstroRecordRing* ring, int32_t flags,
+                                void* stream) {
+    if (int r = check(b, true)) return r;
+    if (ring) {
+        if (b->precision != 32)
+            return fail(ASTRO_E_INVALID, "recording needs a float32 batch: the ring is written by the float32 tick kernel (precision %d)",
+                        b->precision);
+        if (flags & ASTRO_TICK_GENERIC_KERNEL)
+            return fail(ASTRO_E_INVALID, "recording needs the float32 tick kernel: ASTRO_TICK_GENERIC_KERNEL runs the template kernel, which does not record");
+        if (!ring->controls || !ring->events) return fail(ASTRO_E_INVALID, "the ring's controls and events arrays are required");
+        if (b->S == 2 && ((uintptr_t)ring->controls & 1)) return fail(ASTRO_E_INVALID, "the ring's controls must be 2-byte aligned");
+        if (ring->ticks < 2 || n_ticks >= ring->ticks)
+            return fail(ASTRO_E_INVALID, "n_ticks %d needs a ring of at least n_ticks + 1 rows (ticks = %d): the state after the last "
+                        "tick is recorded too", n_ticks, ring->ticks);
+        if (ring->observations)
+            if (int r = observe_args(b, ring->observations, ring->n_rows, false)) return r;
+        b->rec_now = *ring;
+    }
+    const int rc = rollout_device(b, n_ticks, ship0_mode, ship1_mode, avoid_distance, avoid_threshold, actions, nullptr, flags, stream);
+    b->rec_now = AstroRecordRing{};
+    return rc;
 }
 
 // (the body of one tick of astro_rollout_device with bots, on stream st)
@@ -2990,7 +3051,9 @@ static int rollout_one_tick(AstroBatch* b, const int* modes, double avoid_distan
         any_explore |= modes[k] == ASTRO_BOT_EXPLORE;
         any_idle |= modes[k] == ASTRO_BOT_NOTHING;
     }
-    const bool all_stream = false;
+    const bool all_stream = modes[0] == ASTRO_BOT_STREAM;   // (the counter stream drives every ship or none)
+    if (b->rec_now.observations)                            // the recording ring: the state the bots are about to see
+        if (int r = observe_impl(b, b->rec_now.observations, b->rec_now.n_rows, false, stream, (uint32_t)b->rec_now.ticks)) return r;
     {
         // a script bot writes every ship's control, the policy then overwrites the ships it drives
         if (any_script)

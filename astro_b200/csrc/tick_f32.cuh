@@ -26,7 +26,9 @@
 //         7 staging windows and 28 one-warp CTAs per SM (the one-tick launch: 8 and 26) — this form is bound by instruction issue
 //   BOT   script.ScriptBot / NothingBot evaluated inside the tick (astro_rollout_device)
 //   FIX   the production rollout's options fixed at compile time: packed controls given, event planes written, no reward / done
-//         arrays, auto-reset from the pool.  launch_tick_f32 (astro_b200.cu) picks it when the launch's options match.
+//         arrays, auto-reset from the pool, no recording ring.  launch_tick_f32 (astro_b200.cu) picks it when the launch's
+//         options match.  Every other form stores each tick's controls and event byte into the recording ring of
+//         astro_rollout_device_record when one is given (TickParams::rec_*).
 // What the issue-bound form paid for, and no longer does (profiles/r2_ab_diet.md): option tests and the address arithmetic of
 // absent arrays (FIX); a test and a round loop around the common bullet loop (duplicated per value of `multi`); values ptxas
 // re-derived instead of keeping — the shared-memory base behind every rare float64 block, the tile index, the lane id — which now
@@ -446,7 +448,8 @@ template <int S, bool STATS, bool MANY, bool BOT, bool FIX, int PL>
 // (planets and the bullet list always do), and the tile's statistics (`stat_acc`, summed over the launch's ticks).
 __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v, TileScratchT<MANY ? ASTRO_STAGE_WINDOWS_MANY : ASTRO_STAGE_WINDOWS, PL>& t, const unsigned lane,
                                           const unsigned tile_index, const TileIn& in, TileIn& next, const bool last,
-                                          unsigned& stat_acc, const bool have_fire_word, unsigned& pool, unsigned& genmask) {
+                                          unsigned& stat_acc, const bool have_fire_word, unsigned& pool, unsigned& genmask,
+                                          const unsigned rec_row) {
     using B4 = Body4<float>;
     constexpr int kStageWindows = MANY ? ASTRO_STAGE_WINDOWS_MANY : ASTRO_STAGE_WINDOWS;
     // `pool` / `genmask` (warp-uniform, kept by the caller from tick to tick): the resident bullet pool of section 6
@@ -487,9 +490,11 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
             if (ctl[1] > 5) ctl[1] = 2;
         }
     } else if (!BOT) {
+        // (the stream step: in a captured chunk of astro_rollout_device's loop — the counter stream with a recording ring of
+        // observations — it is relative to the device step word)
         uint32_t h0 = game_key(p.seed, p.first_game + (uint32_t)g);
-        ctl[0] = action_from_key(h0, v.step, 0u);
-        ctl[1] = S == 2 ? action_from_key(h0, v.step, 1u) : ctl[0];
+        ctl[0] = action_from_key(h0, v.step + step_base, 0u);
+        ctl[1] = S == 2 ? action_from_key(h0, v.step + step_base, 1u) : ctl[0];
     } else {
         ctl[0] = ctl[1] = 2;      // (bots decide below, once the planets are here)
     }
@@ -526,6 +531,14 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
                 }
             }
         }
+    }
+    // The recording ring (astro_rollout_device_record): whatever the source of this tick's controls — the actions array, the
+    // counter stream or the bots above — they are final here.  Row = the tick's stream step mod the ring's rows.
+    const bool recording = !FIX && p.rec_events != nullptr;
+    if (recording) {
+        const size_t at = (size_t)rec_row * (unsigned)p.n_games + (unsigned)g;
+        if (S == 2) ST_STREAM(reinterpret_cast<unsigned short*>(p.rec_controls) + at, (unsigned short)(ctl[0] | (ctl[1] << 8)));
+        else ST_STREAM(p.rec_controls + at, (unsigned char)ctl[0]);
     }
 
     // ================= 2. flat bullet list of the tile; stage it with cp.async =================
@@ -1178,6 +1191,7 @@ __device__ __forceinline__ void tick_tile(const TickParams& p, const TickVar& v,
         }
     }
     if (!FIX && v.done) v.done[g] = (uint8_t)((ev & (ASTRO_EV_DONE_MASK | ASTRO_EV_SKIPPED)) ? 1 : 0);
+    if (recording) ST_STREAM(&p.rec_events[(size_t)rec_row * (unsigned)p.n_games + (unsigned)g], (uint8_t)ev);
 
     if (STATS) {
         // warp totals -> this warp's private slot row in HBM (no block barrier, no contention);
@@ -1252,6 +1266,9 @@ __global__ void __launch_bounds__(kTickThreads, BOT ? ASTRO_TICK_MIN_BLOCKS_BOT 
     if (has_ring && lane == 0) used0 = p.tile_used[tile];
     load_tile_in<S, PL, FIX>(p, tick_var<S>(p, 0u), tile, lane, in);
     if (has_ring && lane == 0) scratch.used = used0;
+    // the recording ring's row of this launch's first tick (then one row further per tick, wrapping)
+    unsigned rec_row = 0;
+    if (!FIX && p.rec_events) rec_row = (p.step + (p.step_base ? *p.step_base : 0u)) % p.rec_ticks;
 #pragma unroll 1
     for (unsigned k = 0; k < (MANY ? (unsigned)p.n_fused : 1u); k++) {
         const TickVar v = tick_var<S>(p, MANY ? k : 0u);
@@ -1264,8 +1281,9 @@ __global__ void __launch_bounds__(kTickThreads, BOT ? ASTRO_TICK_MIN_BLOCKS_BOT 
         }
         if (MANY) in.fire_word = p.fire_bits[min(meta_tick<PL>(in.meta), (uint32_t)p.n_sched_ticks - 1u) >> 5];
         // (one-warp CTAs: the scratch is s_tiles[0], every shared address a compile-time constant — no base register)
-        tick_tile<S, STATS, MANY, BOT, FIX, PL>(p, v, scratch, lane, tile, in, next, !MANY || k + 1u == (unsigned)p.n_fused, stat_acc, MANY, pool, genmask);
+        tick_tile<S, STATS, MANY, BOT, FIX, PL>(p, v, scratch, lane, tile, in, next, !MANY || k + 1u == (unsigned)p.n_fused, stat_acc, MANY, pool, genmask, rec_row);
         if (MANY) {
+            if (++rec_row == p.rec_ticks) rec_row = 0;
             // The next tick of this tile: meta, ships and bearings are handed on in registers (they were stored as
             // well), so it starts its prefix sums and list requests at once; only the planet rows are loaded.  The
             // warp barrier orders this tick's list stores before the next tick's requests (no fence: a fence would
@@ -1331,6 +1349,9 @@ __device__ __forceinline__ void tick_f32_body(const TickParams& p) {
     if (has_ring && lane == 0) used0 = p.tile_used[tile];
     load_tile_in<S, PL, FIX>(p, tick_var<S>(p, 0u), tile, lane, in);
     if (has_ring && lane == 0) scratch.used = used0;
+    // the recording ring's row of this launch's first tick (then one row further per tick, wrapping)
+    unsigned rec_row = 0;
+    if (!FIX && p.rec_events) rec_row = (p.step + (p.step_base ? *p.step_base : 0u)) % p.rec_ticks;
 #pragma unroll 1
     for (unsigned k = 0; k < (MANY ? (unsigned)p.n_fused : 1u); k++) {
         const TickVar v = tick_var<S>(p, MANY ? k : 0u);
@@ -1343,8 +1364,9 @@ __device__ __forceinline__ void tick_f32_body(const TickParams& p) {
         }
         if (MANY) in.fire_word = p.fire_bits[min(meta_tick<PL>(in.meta), (uint32_t)p.n_sched_ticks - 1u) >> 5];
         // (one-warp CTAs: the scratch is s_tiles[0], every shared address a compile-time constant — no base register)
-        tick_tile<S, STATS, MANY, BOT, FIX, PL>(p, v, scratch, lane, tile, in, next, !MANY || k + 1u == (unsigned)p.n_fused, stat_acc, MANY, pool, genmask);
+        tick_tile<S, STATS, MANY, BOT, FIX, PL>(p, v, scratch, lane, tile, in, next, !MANY || k + 1u == (unsigned)p.n_fused, stat_acc, MANY, pool, genmask, rec_row);
         if (MANY) {
+            if (++rec_row == p.rec_ticks) rec_row = 0;
             // The next tick of this tile: meta, ships and bearings are handed on in registers (they were stored as
             // well), so it starts its prefix sums and list requests at once; only the planet rows are loaded.  The
             // warp barrier orders this tick's list stores before the next tick's requests (no fence: a fence would

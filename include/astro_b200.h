@@ -340,6 +340,29 @@ int astro_set_exploration(AstroBatch* b, double t_in, double t_out, uint32_t see
 int astro_rollout_device(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, int32_t ship1_mode, double avoid_distance,
                          double avoid_threshold, uint8_t* actions, uint8_t* events, int32_t flags, void* stream);
 
+/* A per-tick recording ring for astro_rollout_device_record: what every game's ships flew, what came of it and (optionally)
+ * what ship 0 saw, for each tick of a rollout — the log that rl.QBotTrainer keeps per bot (Experience, rl.py:212-228) and
+ * that astro_nstep_experiences turns into n-step replay pairs.  Device pointers, caller-owned; row r of every array holds
+ * the tick run at stream step s with s % ticks == r. */
+typedef struct AstroRecordRing {
+    int32_t ticks;        /* R rows; the tick run at stream step s is recorded in row s % R */
+    int32_t n_rows;       /* observation rows per game (as astro_observe_shared); ignored when observations is NULL */
+    uint8_t* controls;    /* u8 [R][n_games][S]: the control each ship flew on that tick (required) */
+    uint8_t* events;      /* u8 [R][n_games]: that tick's ASTRO_EV_* byte, exactly what astro_tick writes (required) */
+    float* observations;  /* f32 [R][n_games][n_rows][1+5S+4] or NULL: ship 0's view of the state BEFORE the tick */
+} AstroRecordRing;
+/* astro_rollout_device (same arguments but `events`, same results: recording changes no state and no counter) that also
+ * records every tick into `ring` (NULL: astro_rollout_device without events).  A call of n_ticks from stream
+ * step s0 fills rows s0 .. s0 + n_ticks - 1 (mod R) and, with observations, writes the observation of the state after its
+ * last tick into row (s0 + n_ticks) % R, so that the new state of every pair a window yields is in the ring: n_ticks <= R - 1.
+ * Float32 batches only (not precision 64, not ASTRO_TICK_GENERIC_KERNEL); observations 16-byte aligned, n_rows >= the
+ * planet slots + bullet_cap.  Controls and events are stored by the tick kernel itself, so the counter stream keeps its
+ * many-tick launches and ScriptBot / NothingBot games keep the bots inside the tick; with observations every tick is
+ * observe -> bots -> tick. */
+int astro_rollout_device_record(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, int32_t ship1_mode, double avoid_distance,
+                                double avoid_threshold, uint8_t* actions, const AstroRecordRing* ring, int32_t flags,
+                                void* stream);
+
 /* Game-major float64 view of games, the layout host-side code wants (State conversion for the drop-in core.step /
  * core.play, core.py:11-18 and :377-410; JSONL logs, core.py:413-443): row i describes one game.  DEVICE pointers.
  *   ships R [m][S][5] = x, y, dx, dy, b    planets [m][PL][4] (dead slots zero)    bullets [m][k][4] (dead slots zero)
@@ -387,9 +410,10 @@ int astro_step_single_host(AstroBatch* b, const AstroSingleGame* in_host, AstroS
 
 /* The n-step replay ingestion of rl.QBotTrainer.reward (rl.py:303-328) for every bot (game, ship) over a window of n_ticks
  * logged ticks: which (state, action) pairs are flushed into the replay buffer when, with which discounted reward, discount
- * and new state — from the ticks' event bytes alone (the actions and observations of the ticks stay where the caller
- * logged them; an Experience is identified by its tick).  Device pointers:
- *   events     u8 [n_ticks][n_games]            the ticks' ASTRO_EV_* bytes (astro_tick_many / astro_rollout_*)
+ * and new state — from the ticks' event bytes alone (an Experience is identified by its tick; the actions and observations
+ * of the ticks are in the AstroRecordRing that astro_rollout_device_record filled, or wherever the caller logged them).
+ * Device pointers:
+ *   events     u8 [n_ticks][n_games]            the ticks' ASTRO_EV_* bytes (astro_tick_many / astro_rollout_*, a ring's rows)
  *   carry      i32 [n_games][S]  in/out         pairs a bot still holds (before the window / after it); zero-initialised
  *   out_reward / out_discount f32, out_next i32 [n_steps + n_ticks][n_games][S]: row n_steps + t = the pair of tick t, rows
  *              below n_steps = the ticks before the window (carried pairs that flush now).  reward = r * d and discount =
