@@ -2,6 +2,9 @@
 import itertools as it
 import json
 import os
+import re
+import shutil
+import subprocess
 
 import numpy as np
 
@@ -127,3 +130,34 @@ def check_same(a_games, b_games, ev_a, ev_b):
     assert np.array_equal(a['bullets'][live], b['bullets'][live])        # every list, item for item, in order
     assert np.array_equal(ev_a, ev_b)
     assert a_games.stats() == b_games.stats()
+
+
+# ---- which kernels a library holds and which a call launches -------------------------------------------------------
+
+def library_kernel_names():
+    """The demangled names of every kernel of the built library (cuobjdump -symbols, then cu++filt: the spelling
+    `tick_kernel<double, (int)1, (bool)0, (int)8>(...)`).  Skips the calling test when the tools are missing."""
+    import pytest
+    from astro_b200 import _native as nat
+    cuobjdump = shutil.which('cuobjdump') or '/usr/local/cuda/bin/cuobjdump'
+    cufilt = shutil.which('cu++filt') or '/usr/local/cuda/bin/cu++filt'
+    if not (os.path.exists(cuobjdump) and os.path.exists(cufilt)):
+        pytest.skip('cuobjdump / cu++filt not available')
+    syms = subprocess.run([cuobjdump, '-symbols', nat.LIB_PATH], capture_output=True, text=True, check=True).stdout
+    names = re.findall(r'STO_ENTRY\s+(\S+)', syms)
+    plain = subprocess.run([cufilt], input='\n'.join(names) + '\n', capture_output=True, text=True, check=True).stdout
+    return [n for n in plain.split('\n') if n]
+
+
+def launched(fn, form_of):
+    """Runs fn() under torch.profiler with CUDA activity; returns its result and the set of form_of(name) over the kernels
+    it launched (CUPTI's spelling: `tick_f32_kernel<2, true, false, false, true>(...)`), Nones left out."""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        result = fn()
+        torch.cuda.synchronize()
+    names = [e.key for e in prof.key_averages()]
+    assert names, 'the profiler returned no kernel records'
+    return result, {f for f in map(form_of, names) if f is not None}

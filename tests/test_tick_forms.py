@@ -13,8 +13,6 @@ exactly the tick forms it is about.
 - Solo games with bullets in flight and parked around the ship."""
 import os
 import re
-import shutil
-import subprocess
 
 import numpy as np
 import pytest
@@ -91,14 +89,7 @@ LEDGER = _ledger()
 
 
 def _tick_forms_of_library():
-    cuobjdump = shutil.which('cuobjdump') or '/usr/local/cuda/bin/cuobjdump'
-    cufilt = shutil.which('cu++filt') or '/usr/local/cuda/bin/cu++filt'
-    if not (os.path.exists(cuobjdump) and os.path.exists(cufilt)):
-        pytest.skip('cuobjdump / cu++filt not available')
-    syms = subprocess.run([cuobjdump, '-symbols', nat.LIB_PATH], capture_output=True, text=True, check=True).stdout
-    names = re.findall(r'STO_ENTRY\s+(\S+)', syms)
-    plain = subprocess.run([cufilt], input='\n'.join(names) + '\n', capture_output=True, text=True, check=True).stdout
-    forms = [form_of(n) for n in plain.split('\n')]
+    forms = [form_of(n) for n in H.library_kernel_names()]
     return [f for f in forms if f is not None]
 
 
@@ -128,15 +119,7 @@ def test_library_tick_forms_equal_the_ledger():
 
 def _launched(fn):
     """Runs fn() under torch.profiler with CUDA activity; returns its result and the tick forms launched."""
-    import torch
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        result = fn()
-        torch.cuda.synchronize()
-    names = [e.key for e in prof.key_averages()]
-    assert names, 'the profiler returned no kernel records'
-    return result, {f for f in map(form_of, names) if f is not None}
+    return H.launched(fn, form_of)
 
 
 def _expect(forms, fn):
