@@ -31,7 +31,7 @@ EXPORTS = ('astro_abi_version', 'astro_last_error', 'astro_batch_create', 'astro
            'astro_tick_host_begin', 'astro_tick_host_end', 'astro_fresh_games_enable', 'astro_fresh_games_reset_all',
            'astro_fresh_games_refill', 'astro_fresh_games_positions', 'astro_config_seeds', 'astro_nstep_experiences', 'astro_export_games', 'astro_import_games', 'astro_single_game_bytes', 'astro_step_single_host',
            'astro_stats_peer_create', 'astro_stats_peer_open', 'astro_stats_allreduce', 'astro_value_forward',
-           'astro_rollout_device_record')
+           'astro_rollout_device_record', 'astro_rollout_device_follow')
 
 
 class AstroConfig(C.Structure):
@@ -64,6 +64,11 @@ class AstroGameArrays(C.Structure):
 class AstroRecordRing(C.Structure):
     _fields_ = [('ticks', C.c_int32), ('n_rows', C.c_int32), ('controls', C.c_void_p), ('events', C.c_void_p),
                 ('observations', C.c_void_p)]
+
+
+class AstroFollowRing(C.Structure):
+    _fields_ = [('m', C.c_int32), ('reserved', C.c_int32), ('index', C.c_void_p), ('ships', C.c_void_p), ('planets', C.c_void_p),
+                ('bullets', C.c_void_p), ('info', C.c_void_p)]
 
 
 class AstroSingleGame(C.Structure):
@@ -129,6 +134,8 @@ def lib():
     L.astro_policy_controls.argtypes = [vp, vp, vp, i32, vp]
     L.astro_rollout_device.argtypes = [vp, i32, i32, i32, C.c_double, C.c_double, vp, vp, i32, vp]
     L.astro_rollout_device_record.argtypes = [vp, i32, i32, i32, C.c_double, C.c_double, vp, C.POINTER(AstroRecordRing), i32, vp]
+    L.astro_rollout_device_follow.argtypes = [vp, i32, i32, i32, C.c_double, C.c_double, vp, C.POINTER(AstroRecordRing),
+                                              C.POINTER(AstroFollowRing), i32, vp]
     L.astro_create_games.argtypes = [vp, C.POINTER(AstroCreateConfig), vp, i32, vp, vp, vp, vp]
     L.astro_script_controls.argtypes = [vp, C.c_double, C.c_double, vp, vp]
     L.astro_export_games.argtypes = [vp, vp, i32, C.POINTER(AstroGameArrays), vp]

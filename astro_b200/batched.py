@@ -264,14 +264,18 @@ class BatchedGames:
     def get_states(self, indices):
         """Reference `State`s (or None for finished games) of the listed games only — the read path of
         logs.GameRecorder and of the drop-in core.play."""
-        a = self.get_arrays(np.asarray(indices, dtype=np.int64).reshape(-1))
+        return self.states_of(self.get_arrays(np.asarray(indices, dtype=np.int64).reshape(-1)))
+
+    def states_of(self, a):
+        """Game-major host arrays (get_arrays' keys ships, planets, bullets, n_planets, n_bullets, tick, finished) as reference
+        `State`s with float64 arrays, reload and t from this batch's schedule; None for finished games."""
         out = []
         for j in range(a['tick'].shape[0]):
             if a['finished'][j]:
                 out.append(None)
                 continue
             nb, npl, tick = int(a['n_bullets'][j]), int(a['n_planets'][j]), int(a['tick'][j])
-            sh, pl, bl = a['ships'][j], a['planets'][j], a['bullets'][j]
+            sh, pl, bl = (np.asarray(a[k][j], dtype=np.float64) for k in ('ships', 'planets', 'bullets'))
             out.append(core.State(
                 ships=core.Bodies(x=sh[:, 0:2].copy(), dx=sh[:, 2:4].copy(), b=sh[:, 4].copy()),
                 planets=core.Bodies(x=pl[:npl, 0:2].copy(), dx=pl[:npl, 2:4].copy(), b=None),
@@ -638,7 +642,8 @@ class BatchedGames:
         set_policy), 'explore' (that network with rl.EpsilonGreedy laid over it: set_exploration), 'nothing'
         (script.NothingBot) per ship.  Outcomes accumulate in stats().
         record: a RecordRing (record_ring()) that receives every tick's controls, events and — if it holds them — the
-        observations (astro_rollout_device_record); the results are the same as without it."""
+        observations (astro_rollout_device_record) and the followed games' states (astro_rollout_device_follow); the results
+        are the same as without it."""
         if isinstance(bots, str):
             bots = (bots,) * self.S
         modes = [nat.BOT_MODES[b] for b in bots] + [0]
@@ -651,17 +656,27 @@ class BatchedGames:
         else:
             if (record.n_pad, record.S) != (self.n_pad, self.S) or record.device != self.device:
                 raise ValueError('the ring was made for another batch layout (record_ring of this batch)')
-            nat.check(nat.lib().astro_rollout_device_record(self._h, n, modes[0], modes[1], float(avoid_distance),
-                                                            float(avoid_threshold), self._actions.data_ptr(), C.byref(record._ring),
-                                                            flags, self._stream()))
+            if record.follow is not None and (record.PL, record.K) != (self.PL, self.K):
+                raise ValueError('the ring follows games of another batch layout (planet slots, bullet_cap)')
+            if record.follow is None:
+                nat.check(nat.lib().astro_rollout_device_record(self._h, n, modes[0], modes[1], float(avoid_distance),
+                                                                float(avoid_threshold), self._actions.data_ptr(),
+                                                                C.byref(record._ring), flags, self._stream()))
+            else:
+                nat.check(nat.lib().astro_rollout_device_follow(self._h, n, modes[0], modes[1], float(avoid_distance),
+                                                                float(avoid_threshold), self._actions.data_ptr(),
+                                                                C.byref(record._ring), C.byref(record._follow), flags,
+                                                                self._stream()))
             record._recorded(self.step_index, n)
         self.step_index += n
 
-    def record_ring(self, ticks, observations=True, n_rows=None):
+    def record_ring(self, ticks, observations=True, n_rows=None, follow=None):
         """A RecordRing of `ticks` rows for rollout_device(..., record=ring): per tick the controls, events and (observations=True)
         ship 0's observation of the state before the tick (n_rows as observe(); default the smallest multiple of 4 that holds
-        the planet slots and bullet_cap).  A rollout_device call records at most ticks - 1 ticks."""
-        return RecordRing(self, ticks, observations, n_rows)
+        the planet slots and bullet_cap), and, with `follow` (a list of distinct game indices), those games' states before
+        the tick (RecordRing.follow_states; logs.GameRecorder.rollout).  A rollout_device call records at most ticks - 1
+        ticks."""
+        return RecordRing(self, ticks, observations, n_rows, follow)
 
     # ---- n-step replay ingestion ---------------------------------------------------------------------
     def nstep_experiences(self, events, carry=None, n_steps=100, discount=0.995):
@@ -743,15 +758,23 @@ class RecordRing:
       events        uint8 [ticks, n_pad]                   that tick's ASTRO_EV_* byte (what step() returns as events)
       observations  float32 [ticks, n_pad, n_rows, D]      ship 0's observation (observe(shared=True)) of the state before the
                     or None                                tick; a rollout call also records the state after its last tick
+    and, for a ring that follows games (follow = the list of their indices, m of them; else None), their states before the
+    tick (and after a call's last tick), in the layout of export_arrays but float32 (exact):
+      follow_ships    float32 [ticks, m, S, 5]      x, y, dx, dy, b
+      follow_planets  float32 [ticks, m, PL, 4]     slots past the game's planets are zero
+      follow_bullets  float32 [ticks, m, K, 4]      rows past the game's bullets are zero (K = bullet_cap)
+      follow_info     int32 [ticks, m, 4]           n_planets, n_bullets, tick (index into the batch's schedule), finished
     Rows of stream steps first .. end - 1 hold an unbroken history (a rollout that does not continue where the last one ended
     starts a new one)."""
 
-    def __init__(self, games, ticks, observations=True, n_rows=None):
+    def __init__(self, games, ticks, observations=True, n_rows=None, follow=None):
         torch = _torch()
         R = int(ticks)
         if R < 2:
             raise ValueError('a ring needs at least 2 rows')
+        self._games = games
         self.ticks, self.n_pad, self.S, self.D, self.device = R, games.n_pad, games.S, games.D, games.device
+        self.PL, self.K = games.PL, games.K
         self.n_rows = -(-(games.PL + games.K) // 4) * 4 if n_rows is None else int(n_rows)
         self.controls = torch.zeros((R, self.n_pad, self.S), dtype=torch.uint8, device=self.device)
         self.events = torch.zeros((R, self.n_pad), dtype=torch.uint8, device=self.device)
@@ -759,6 +782,22 @@ class RecordRing:
                              if observations else None)
         self._ring = nat.AstroRecordRing(R, self.n_rows, self.controls.data_ptr(), self.events.data_ptr(),
                                          None if self.observations is None else self.observations.data_ptr())
+        self.follow = None
+        if follow is not None:
+            self.follow = [int(i) for i in follow]
+            m = len(self.follow)
+            if m == 0 or len(set(self.follow)) != m:
+                raise ValueError('follow must list one or more distinct games')
+            if min(self.follow) < 0 or max(self.follow) >= games.n:
+                raise IndexError('followed game out of range 0..%d' % (games.n - 1))
+            self._follow_index = torch.tensor(self.follow, dtype=torch.int32, device=self.device)
+            self.follow_ships = torch.zeros((R, m, self.S, 5), dtype=torch.float32, device=self.device)
+            self.follow_planets = torch.zeros((R, m, games.PL, 4), dtype=torch.float32, device=self.device)
+            self.follow_bullets = torch.zeros((R, m, games.K, 4), dtype=torch.float32, device=self.device)
+            self.follow_info = torch.zeros((R, m, 4), dtype=torch.int32, device=self.device)
+            self._follow = nat.AstroFollowRing(m, 0, self._follow_index.data_ptr(), self.follow_ships.data_ptr(),
+                                               self.follow_planets.data_ptr(),
+                                               self.follow_bullets.data_ptr() if games.K else None, self.follow_info.data_ptr())
         self.first = self.end = None
 
     def _recorded(self, s0, n):
@@ -767,6 +806,22 @@ class RecordRing:
         self.end = s0 + n
         # row end % R now holds the observation of step `end`: the controls / events of step end - R are gone with it
         self.first = max(self.first, self.end + 1 - self.ticks)
+
+    def follow_states(self, step):
+        """The reference `State`s (float64 arrays; None for a finished game) of the followed games before the tick at stream
+        step `step` (the state after a call's last tick at step = its end), in the order of `follow`: what get_states(follow)
+        returned at that point of the rollout."""
+        if self.follow is None:
+            raise ValueError('this ring follows no games (record_ring(..., follow=[...]))')
+        s = int(step)
+        if self.end is None or not self.first <= s <= self.end:
+            raise ValueError('the ring holds the states of stream steps %s, not %d'
+                             % ('none' if self.end is None else '%d..%d' % (self.first, self.end), s))
+        r = s % self.ticks
+        info = self.follow_info[r].cpu().numpy()
+        return self._games.states_of(dict(ships=self.follow_ships[r].cpu().numpy(), planets=self.follow_planets[r].cpu().numpy(),
+                                          bullets=self.follow_bullets[r].cpu().numpy(), n_planets=info[:, 0],
+                                          n_bullets=info[:, 1], tick=info[:, 2], finished=info[:, 3]))
 
     def _rows(self, t0, n):
         """Ring rows of stream steps t0 .. t0 + n - 1 as an index tensor."""

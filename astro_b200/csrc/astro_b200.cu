@@ -1688,6 +1688,63 @@ __global__ void __launch_bounds__(128) export_kernel(const void* __restrict__ sh
     }
 }
 
+// follow_kernel: export_kernel's gather for the few games a log follows through a device rollout
+// (astro_rollout_device_follow), written in float32 — exact, the batch is float32 — into row
+// (step + *step_base) % ring_ticks of an AstroFollowRing, so that a captured chunk of the bot loop
+// writes the row of the stream step it replays.  Warp = one followed slot.  An index outside
+// 0..n_games-1 writes a zero row with finished = 1 and tick = -1.
+template <int S, int PL>
+__global__ void __launch_bounds__(128) follow_kernel(const void* __restrict__ ships_, const void* __restrict__ ship_b_,
+                                                     const void* __restrict__ planets_, const void* __restrict__ bullets_,
+                                                     const uint32_t* __restrict__ meta_, const int32_t* __restrict__ index, int m,
+                                                     int n_games, int K, uint32_t ring_ticks, uint32_t step,
+                                                     const uint32_t* __restrict__ step_base, float* __restrict__ o_ships,
+                                                     float* __restrict__ o_planets, float* __restrict__ o_bullets,
+                                                     int32_t* __restrict__ o_info) {
+    using B4 = Body4<float>;
+    const int slot = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (slot >= m) return;
+    const size_t at = (size_t)((step + (step_base ? *step_base : 0u)) % ring_ticks) * m + slot;
+    const int g = index[slot];
+    const bool valid = g >= 0 && g < n_games;
+    const size_t tile = valid ? (size_t)(g >> 5) : 0;
+    const int gl = g & 31;
+    const uint32_t meta = valid ? meta_[g] : 0u;
+    const bool fin = !valid || ASTRO_META_FINISHED(meta);
+    const int np = valid ? (int)meta_np<PL>(meta) : 0, nb = fin ? 0 : (int)ASTRO_META_NB(meta);
+    if (lane < S) {
+        B4 v = B4();
+        float b = 0.0f;
+        if (valid) {
+            v = reinterpret_cast<const B4*>(ships_)[tile * (S * 32) + lane * 32 + gl];
+            b = reinterpret_cast<const float*>(ship_b_)[tile * (S * 32) + lane * 32 + gl];
+        }
+        float* o = o_ships + (at * S + lane) * 5;
+        o[0] = v.x; o[1] = v.y; o[2] = v.dx; o[3] = v.dy; o[4] = b;
+    }
+    if (lane < PL) {
+        B4 v = B4();
+        if (lane < np) v = reinterpret_cast<const B4*>(planets_)[tile * (PL * 32) + lane * 32 + gl];
+        float* o = o_planets + (at * PL + lane) * 4;
+        o[0] = v.x; o[1] = v.y; o[2] = v.dx; o[3] = v.dy;
+    }
+    const unsigned first = valid ? tile_list_offset(meta_ + tile * 32, gl, lane) : 0u;
+    const B4* run = reinterpret_cast<const B4*>(bullets_) + tile * (size_t)(32 * K) + first;
+    for (int k = lane; k < K; k += 32) {
+        B4 v = B4();
+        if (k < nb) v = run[k];
+        float* o = o_bullets + (at * K + k) * 4;
+        o[0] = v.x; o[1] = v.y; o[2] = v.dx; o[3] = v.dy;
+    }
+    if (lane == 0) {
+        int32_t* o = o_info + at * 4;
+        o[0] = np;
+        o[1] = nb;
+        o[2] = valid ? (int32_t)meta_tick<PL>(meta) : -1;
+        o[3] = fin ? 1 : 0;
+    }
+}
+
 __global__ void import_map_kernel(const int32_t* __restrict__ index, int m, int n_games, int32_t* __restrict__ src) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= m) return;
@@ -1897,6 +1954,7 @@ struct LoopGraph {        // a captured chunk of the bot loop (astro_rollout_dev
     uint8_t* actions;
     uint8_t* events;
     AstroRecordRing rec;  // the recording ring the chunk writes (its row is read from the device step word, not captured)
+    AstroFollowRing follow;  // the follow ring the chunk writes (m == 0: none), likewise
     int64_t epoch;
     int32_t launches;     // kernels of one replay
 };
@@ -1949,6 +2007,7 @@ struct AstroBatch {
     int64_t config_epoch;         // bumped by every call that changes what a captured chunk depends on
     int32_t bot_modes_now;        // != 0 while astro_rollout_device runs ticks whose bots are evaluated inside the tick kernel
     AstroRecordRing rec_now;      // astro_rollout_device_record: the ring of the running call (events == NULL: none)
+    AstroFollowRing follow_now;   // astro_rollout_device_follow: the follow ring of the running call (m == 0: none)
     ScriptParams script_now;
     // fresh-game mode (astro_fresh_games_enable): per-tile rings of pre-created games fed from the generate_configs stream
     FreshState* fresh;
@@ -2866,6 +2925,21 @@ int astro_explore_controls(AstroBatch* b, double t_in, double t_out, uint32_t se
 static int rollout_one_tick(AstroBatch* b, const int* modes, double avoid_distance, double avoid_threshold, uint8_t* actions, uint8_t* events,
                             int32_t flags, cudaStream_t st);
 
+// astro_rollout_device_follow: the followed games' state into the follow ring's row of the current stream step
+static int follow_impl(AstroBatch* b, cudaStream_t st) {
+    const AstroFollowRing& f = b->follow_now;
+    const AstroBuffers& u = b->bufs;
+    const int grid = (f.m + 3) / 4;
+    with_layout(b, [&](auto, auto s, auto pl) {
+        follow_kernel<s, pl><<<grid, 128, 0, st>>>(u.ships, u.ship_b, u.planets, bullet_buffer(b, b->cur), u.meta, f.index, f.m,
+                                                   b->n_games, b->K, (uint32_t)b->rec_now.ticks, b->step, b->step_base_now,
+                                                   f.ships, f.planets, f.bullets, f.info);
+    });
+    CUDA_TRY(cudaGetLastError());
+    b->launches += 1;
+    return ASTRO_OK;
+}
+
 static int rollout_chunks(AstroBatch* b, int n_chunks, const int* modes, double avoid_distance, double avoid_threshold, uint8_t* actions,
                           uint8_t* events, int32_t flags, cudaStream_t st) {
     if (!b->d_step_base) {
@@ -2891,7 +2965,10 @@ static int rollout_chunks(AstroBatch* b, int n_chunks, const int* modes, double 
             if (q.exec && q.epoch == b->config_epoch && q.cur == b->cur && q.flags == flags && q.modes[0] == modes[0] && q.modes[1] == modes[1] &&
                 q.avoid_distance == avoid_distance && q.avoid_threshold == avoid_threshold && q.actions == actions && q.events == events &&
                 q.rec.ticks == b->rec_now.ticks && q.rec.n_rows == b->rec_now.n_rows && q.rec.controls == b->rec_now.controls &&
-                q.rec.events == b->rec_now.events && q.rec.observations == b->rec_now.observations)
+                q.rec.events == b->rec_now.events && q.rec.observations == b->rec_now.observations &&
+                q.follow.m == b->follow_now.m && q.follow.index == b->follow_now.index && q.follow.ships == b->follow_now.ships &&
+                q.follow.planets == b->follow_now.planets && q.follow.bullets == b->follow_now.bullets &&
+                q.follow.info == b->follow_now.info)
                 g = &q;
         }
         if (!g) {
@@ -2922,6 +2999,7 @@ static int rollout_chunks(AstroBatch* b, int n_chunks, const int* modes, double 
             g->epoch = b->config_epoch; g->cur = b->cur; g->flags = flags; g->modes[0] = modes[0]; g->modes[1] = modes[1];
             g->avoid_distance = avoid_distance; g->avoid_threshold = avoid_threshold; g->actions = actions; g->events = events;
             g->rec = b->rec_now;
+            g->follow = b->follow_now;
         }
         CUDA_TRY(cudaGraphLaunch(g->exec, ls));
         b->step += (uint32_t)kLoopChunk;
@@ -2958,9 +3036,11 @@ static int rollout_device(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, in
     CUDA_TRY(cudaSetDevice(b->device));
     if (any_idle) CUDA_TRY(cudaMemsetAsync(actions, 2, (size_t)b->n_games * b->S, st));  // script.NothingBot: control 2
     // Recording: the tick kernel stores each tick's controls and events itself, so the two fast paths below keep their launches;
-    // observations are taken by observe_kernel before every tick, which needs the per-tick loop at the end.
+    // observations (observe_kernel) and followed games' states (follow_kernel) are taken before every tick, which needs the
+    // per-tick loop at the end.
     float* const rec_obs = b->rec_now.observations;
-    if (all_stream && !rec_obs) {
+    const bool per_tick = rec_obs || b->follow_now.m > 0;
+    if (all_stream && !per_tick) {
         // no bot between the ticks: the ticks of a tile run back to back inside the launches; `events` keeps the last tick's
         if (n_ticks > 1) if (int r = do_ticks(b, nullptr, nullptr, nullptr, nullptr, flags, st, n_ticks - 1)) return r;
         return n_ticks > 0 ? do_ticks(b, nullptr, nullptr, nullptr, events, flags, st, 1) : ASTRO_OK;
@@ -2971,7 +3051,7 @@ static int rollout_device(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, in
     // and always take the bot kernel -> tick kernel loop below.
     {
         const char* fb = getenv("ASTRO_FUSED_BOTS");
-        if (!any_policy && !rec_obs && b->precision == 32 && b->PL == ASTRO_MAX_PLANETS && !(flags & ASTRO_TICK_GENERIC_KERNEL) &&
+        if (!any_policy && !per_tick && b->precision == 32 && b->PL == ASTRO_MAX_PLANETS && !(flags & ASTRO_TICK_GENERIC_KERNEL) &&
             !(fb && atoi(fb) == 0) && n_ticks > 0) {
             b->bot_modes_now = modes[0] | (modes[1] << 4);
             ScriptParams& q = b->script_now;
@@ -3006,7 +3086,9 @@ static int rollout_device(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, in
     for (int k = k_done; k < n_ticks; k++) {
         if (int r = rollout_one_tick(b, modes, avoid_distance, avoid_threshold, actions, events, flags, st)) return r;
     }
-    // the state after the last tick: the new state of the pairs that flush on it
+    // the state after the last tick: the new state of the pairs that flush on it, and the last state of a followed game's log
+    if (b->follow_now.m > 0)
+        if (int r = follow_impl(b, st)) return r;
     if (rec_obs) return observe_impl(b, rec_obs, b->rec_now.n_rows, false, stream, (uint32_t)b->rec_now.ticks);
     return ASTRO_OK;
 }
@@ -3040,6 +3122,25 @@ int astro_rollout_device_record(AstroBatch* b, int32_t n_ticks, int32_t ship0_mo
     return rc;
 }
 
+int astro_rollout_device_follow(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, int32_t ship1_mode, double avoid_distance,
+                                double avoid_threshold, uint8_t* actions, const AstroRecordRing* ring, const AstroFollowRing* follow,
+                                int32_t flags, void* stream) {
+    if (int r = check(b, true)) return r;
+    if (!follow) return fail(ASTRO_E_INVALID, "the follow ring is required (astro_rollout_device_record records without one)");
+    if (!ring) return fail(ASTRO_E_INVALID, "following games needs the recording ring: its ticks set the follow ring's rows");
+    if (follow->m < 1) return fail(ASTRO_E_INVALID, "the follow ring must follow at least one game (m = %d)", follow->m);
+    if (!follow->index || !follow->ships || !follow->planets || !follow->info || (b->K > 0 && !follow->bullets))
+        return fail(ASTRO_E_INVALID, "the follow ring's index, ships, planets, bullets and info arrays are required");
+    if (((uintptr_t)follow->index | (uintptr_t)follow->ships | (uintptr_t)follow->planets | (uintptr_t)follow->bullets |
+         (uintptr_t)follow->info) & 3)
+        return fail(ASTRO_E_INVALID, "the follow ring's arrays must be 4-byte aligned");
+    b->follow_now = *follow;
+    const int rc = astro_rollout_device_record(b, n_ticks, ship0_mode, ship1_mode, avoid_distance, avoid_threshold, actions, ring,
+                                               flags, stream);
+    b->follow_now = AstroFollowRing{};
+    return rc;
+}
+
 // (the body of one tick of astro_rollout_device with bots, on stream st)
 static int rollout_one_tick(AstroBatch* b, const int* modes, double avoid_distance, double avoid_threshold, uint8_t* actions, uint8_t* events,
                      int32_t flags, cudaStream_t st) {
@@ -3052,6 +3153,8 @@ static int rollout_one_tick(AstroBatch* b, const int* modes, double avoid_distan
         any_idle |= modes[k] == ASTRO_BOT_NOTHING;
     }
     const bool all_stream = modes[0] == ASTRO_BOT_STREAM;   // (the counter stream drives every ship or none)
+    if (b->follow_now.m > 0)                                // the follow ring: the followed games' state before the tick
+        if (int r = follow_impl(b, st)) return r;
     if (b->rec_now.observations)                            // the recording ring: the state the bots are about to see
         if (int r = observe_impl(b, b->rec_now.observations, b->rec_now.n_rows, false, stream, (uint32_t)b->rec_now.ticks)) return r;
     {

@@ -363,6 +363,30 @@ int astro_rollout_device_record(AstroBatch* b, int32_t n_ticks, int32_t ship0_mo
                                 double avoid_threshold, uint8_t* actions, const AstroRecordRing* ring, int32_t flags,
                                 void* stream);
 
+/* The state of a few followed games at every tick of a recorded rollout: with the recording ring's controls and events, the
+ * game logs of those games (core.Tick, core.py:377-410).  Device pointers, caller-owned; row r of every array (R = the
+ * AstroRecordRing's ticks) holds the state BEFORE the tick run at stream step s with s % R == r, in the layout of
+ * AstroGameArrays but float32 (exact: the batch is float32). */
+typedef struct AstroFollowRing {
+    int32_t m;              /* followed games (>= 1) */
+    int32_t reserved;
+    const int32_t* index;   /* i32 [m] device: the batch game of each followed slot */
+    float* ships;           /* f32 [R][m][S][5]    R = the AstroRecordRing's ticks */
+    float* planets;         /* f32 [R][m][PL][4] */
+    float* bullets;         /* f32 [R][m][bullet_cap][4] */
+    int32_t* info;          /* i32 [R][m][4]: n_planets, n_bullets, tick, finished */
+} AstroFollowRing;
+/* astro_rollout_device_record (same arguments, checks and results; `ring` is required) that also writes the followed games'
+ * state into `follow`: before every tick at stream step s into row s % R, and after the call's last tick into row
+ * (s0 + n_ticks) % R.  Planet slots past n_planets and bullet rows past n_bullets are zero; a finished game writes
+ * finished = 1, n_bullets = 0 (as astro_export_games), an index outside 0..n_games-1 finished = 1 and tick = -1.
+ * One small kernel before every tick: following games gives up the many-tick launches of the counter stream and the
+ * in-tick ScriptBot / NothingBot, every tick is follow -> (observe) -> bots -> tick.  The arrays must be 4-byte aligned;
+ * bullets may be NULL when bullet_cap is 0. */
+int astro_rollout_device_follow(AstroBatch* b, int32_t n_ticks, int32_t ship0_mode, int32_t ship1_mode, double avoid_distance,
+                                double avoid_threshold, uint8_t* actions, const AstroRecordRing* ring, const AstroFollowRing* follow,
+                                int32_t flags, void* stream);
+
 /* Game-major float64 view of games, the layout host-side code wants (State conversion for the drop-in core.step /
  * core.play, core.py:11-18 and :377-410; JSONL logs, core.py:413-443): row i describes one game.  DEVICE pointers.
  *   ships R [m][S][5] = x, y, dx, dy, b    planets [m][PL][4] (dead slots zero)    bullets [m][k][4] (dead slots zero)
