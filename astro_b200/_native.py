@@ -30,7 +30,7 @@ EXPORTS = ('astro_abi_version', 'astro_last_error', 'astro_batch_create', 'astro
            'astro_policy_controls', 'astro_rollout_device', 'astro_bullet_buffer', 'astro_set_bullet_buffer', 'astro_tick_many', 'astro_explore_controls', 'astro_set_exploration',
            'astro_tick_host_begin', 'astro_tick_host_end', 'astro_fresh_games_enable', 'astro_fresh_games_reset_all',
            'astro_fresh_games_refill', 'astro_fresh_games_positions', 'astro_config_seeds', 'astro_nstep_experiences', 'astro_export_games', 'astro_import_games', 'astro_single_game_bytes', 'astro_step_single_host',
-           'astro_stats_peer_create', 'astro_stats_peer_open', 'astro_stats_allreduce', 'astro_value_forward',
+           'astro_stats_peer_create', 'astro_stats_peer_open', 'astro_stats_allreduce', 'astro_value_forward', 'astro_value_forward_views',
            'astro_rollout_device_record', 'astro_rollout_device_follow')
 
 
@@ -126,6 +126,7 @@ def lib():
     L.astro_observe.argtypes = [vp, vp, i32, vp]
     L.astro_stats.argtypes = [vp, vp, i32, vp]
     L.astro_value_forward.argtypes = [vp, vp, i32, i32, vp, vp]
+    L.astro_value_forward_views.argtypes = [vp, vp, i32, i32, vp, vp, i32, vp, vp]
     L.astro_stats_peer_create.argtypes = [vp, i32, i32, vp]
     L.astro_stats_peer_open.argtypes = [vp, vp]
     L.astro_stats_allreduce.argtypes = [vp, vp, i32, vp]

@@ -598,6 +598,31 @@ class BatchedGames:
         nat.check(nat.lib().astro_value_forward(self._h, x.data_ptr(), n, rows, out.data_ptr(), self._stream()))
         return out
 
+    def value_forward_views(self, features, index, view=None):
+        """value_forward on gathered views of a perspective-0 feature batch (astro_value_forward_views): output e is the loaded
+        network on item index[e] of features (float32 cuda [M, rows, D]) as ship view[e] sees it — ship 1's view exchanges
+        the two ship column groups, as observe() does.  index: int64 [E] on the same device, -1 = an item of all -1 (a
+        finished game); other values outside 0 .. M - 1 give NaN rows.  view: uint8 [E] or None (ship 0; solo batches take
+        none).  Returns float32 [E, nout]."""
+        torch = _torch()
+        if not (features.is_cuda and features.dtype == torch.float32 and features.dim() == 3 and features.shape[-1] == self.D):
+            raise ValueError('value_forward_views needs a float32 cuda tensor [M, rows, %d]' % self.D)
+        if not (index.dtype == torch.int64 and index.dim() == 1 and index.device == features.device):
+            raise ValueError('index must be an int64 tensor [E] on the features\' device')
+        if view is not None and not (self.S == 2 and view.dtype == torch.uint8 and view.shape == index.shape
+                                     and view.device == features.device):
+            raise ValueError('view must be a uint8 tensor shaped like index on the features\' device (duel features only)')
+        x, index = features.contiguous(), index.contiguous()
+        view = None if view is None else view.contiguous()
+        M, rows, E = (int(v) for v in (x.shape[0], x.shape[1], index.shape[0]))
+        if max(M, E) >= 1 << 31:
+            raise ValueError('more than 2^31 - 1 items or outputs')
+        out = torch.empty((E, self.policy_nout), dtype=torch.float32, device=x.device)
+        nat.check(nat.lib().astro_value_forward_views(self._h, x.data_ptr() if M else None, M, rows, index.data_ptr(),
+                                                      None if view is None else view.data_ptr(), E, out.data_ptr(),
+                                                      self._stream()))
+        return out
+
     def policy_controls(self, out=None, q_out=None, ships=None):
         """Greedy controls argmax_a Q(s, a) of the loaded network for every ship of every game, each
         from its own perspective (rl.QBot, rl.py:168-200) — features and network fused in one
@@ -862,6 +887,35 @@ class RecordRing:
         Pairs carried from earlier windows refer to their ticks, so the ring must hold n_steps ticks before the window as well
         as the window and the state after it: ticks >= n_steps + T + 1."""
         torch = _torch()
+        row, game, ship, tick, at, nx_at, terminal = self._pairs(nxt, n_steps)
+        next_features = self._view_of(nx_at, game, ship)
+        next_features = torch.where(terminal[:, None, None], torch.full_like(next_features, -1.0), next_features)
+        return dict(features=self._view_of(at, game, ship), action=self.controls[at, game, ship],
+                    reward=reward[row, game, ship], discount=discount[row, game, ship], next_features=next_features,
+                    terminal=terminal, game=game, ship=ship, tick=tick)
+
+    def experience_values(self, net, reward, discount, nxt, n_steps):
+        """experiences() with the network evaluated on the pairs in place of their feature tensors: the same pairs in the same
+        order, the same checks and the same action / reward / discount / terminal / game / ship / tick entries, and
+          q       float32 [E, nout]  net on the pair's state as its ship sees it
+          next_q  float32 [E, nout]  net on the new state as its ship sees it; net on an all -1 item when terminal
+        both from one `net.forward_views` call on the ring's observations (ship 1's view and the terminal item made as the
+        network reads them), so nothing of E x n_rows x D is gathered: what the bootstrap term max_a Q(s', a) and the
+        prediction Q(s, a) of rl.QBotTrainer's update (rl.py:280-295) need from a window."""
+        torch = _torch()
+        row, game, ship, tick, at, nx_at, terminal = self._pairs(nxt, n_steps)
+        x = self.observations.view(self.ticks * self.n_pad, self.n_rows, self.D)
+        index = torch.cat((at * self.n_pad + game, torch.where(terminal, -1, nx_at.long() * self.n_pad + game)))
+        view = torch.cat((ship, ship)).to(torch.uint8) if self.S == 2 else None
+        q = net.forward_views(x, index, view)
+        E = int(row.shape[0])
+        return dict(q=q[:E], action=self.controls[at, game, ship], reward=reward[row, game, ship],
+                    discount=discount[row, game, ship], next_q=q[E:], terminal=terminal, game=game, ship=ship, tick=tick)
+
+    def _pairs(self, nxt, n_steps):
+        """The pairs of experiences(): (row, game, ship) into nstep_experiences' outputs, their stream step, the ring rows of
+        their tick and of their new state (for a terminal pair, which has none, the row of the window's first step: callers
+        replace it by all -1 features or index -1), and the terminal flags."""
         if self.observations is None:
             raise ValueError('experiences need a ring that records observations')
         n_steps = int(n_steps)
@@ -878,11 +932,5 @@ class RecordRing:
         tick = s0 + row - n_steps
         if tick.numel() and int(tick.min()) < self.first:
             raise ValueError('a carried pair refers to stream step %d, before the ring\'s history (from %d)' % (int(tick.min()), self.first))
-        at = tick % self.ticks
         nx = nxt[row, game, ship]
-        terminal = nx == -1
-        next_features = self._view_of((s0 + nx.clamp(min=0)) % self.ticks, game, ship)
-        next_features = torch.where(terminal[:, None, None], torch.full_like(next_features, -1.0), next_features)
-        return dict(features=self._view_of(at, game, ship), action=self.controls[at, game, ship],
-                    reward=reward[row, game, ship], discount=discount[row, game, ship], next_features=next_features,
-                    terminal=terminal, game=game, ship=ship, tick=tick)
+        return row, game, ship, tick, tick % self.ticks, (s0 + nx.clamp(min=0)) % self.ticks, nx == -1

@@ -1412,11 +1412,24 @@ policy_mma_kernel(const void* __restrict__ ships_, const void* __restrict__ ship
 //   A chunk of 8 rows that is padding for both items is skipped once each item has shown a live row (its maximum can no
 //   longer come from a padding row: pre-activations are far below 1e9); an item without any live row takes every chunk,
 //   exactly the reference's arithmetic.
+//   Gathered views (astro_value_forward_views): output e is the network on item index[e] (index NULL: item e) as ship
+//   view[e] sees it (view NULL: ship 0; DIN 15 only).  Ship 1's view is ship 0's with the ship column groups exchanged, so
+//   a lane reads its column c from column swap(c) of the item; MMA rows are independent, so an output equals the same item
+//   view materialised and passed through the plain path, bit for bit.  index -1 is an item whose every entry is -1 (the
+//   new state of a terminal pair), made without a memory read; any other index outside 0 .. n_items - 1 is never read and
+//   its outputs are NaN.
 // ------------------------------------------------------------------------------------------
-template <int DIN>
-__global__ void __launch_bounds__(kMmaWarps * 32, ASTRO_MMA_MIN_BLOCKS)
-value_forward_kernel(const float* __restrict__ features, float* __restrict__ q_out, int n_items, int rows, int nout,
-                     const PolicyFragWeights* __restrict__ frags) {
+//   The body is compiled twice, with and without the gathered views (VIEWS): the plain path keeps the instructions it had
+//   before the views existed (one body serving both cost it 9 %), but the two share the kernel's register allocation:
+//   ptxas gives <15> 128 registers (114 before; 128 is the cap of __launch_bounds__(128, 4)) and <10> 116, no spills — the
+//   plain path has no register headroom left.  The plain body reads item e for output e without a range check: its callers
+//   keep n_out <= n_items (astro_value_forward passes n_out = n_items, astro_value_forward_views refuses n_out > n_items
+//   without an index).
+template <int DIN, bool VIEWS>
+__device__ __forceinline__ void
+value_forward_body(const float* __restrict__ features, float* __restrict__ q_out, int n_items, int rows, int nout,
+                   const PolicyFragWeights* __restrict__ frags, const int64_t* __restrict__ index, const uint8_t* __restrict__ view,
+                   int n_out) {
     extern __shared__ float4 s_dyn[];
     PolicyFrags& s_all = *reinterpret_cast<PolicyFrags*>(s_dyn);
     const PolicyFragWeights& s_w = s_all.w;
@@ -1428,19 +1441,28 @@ value_forward_kernel(const float* __restrict__ features, float* __restrict__ q_o
         for (int i = threadIdx.x; i < (int)(sizeof(PolicyFragWeights) / 16); i += blockDim.x) dst[i] = src[i];
     }
     __syncthreads();
-    int col[4];                                   // this lane's feature columns: 2t, 2t + 1, 2t + 8, 2t + 9 (>= DIN: zero)
-#pragma unroll
-    for (int j = 0; j < 4; j++) col[j] = 2 * t + (j & 1) + 8 * (j >> 1);
+    int col[4], col1[4];                          // this lane's feature columns: 2t, 2t + 1, 2t + 8, 2t + 9 (>= DIN: zero)
+#pragma unroll                                    // col1: where ship 1's view of the item holds them
+    for (int j = 0; j < 4; j++) {
+        col[j] = 2 * t + (j & 1) + 8 * (j >> 1);
+        col1[j] = (col[j] >= 1 && col[j] <= 5) ? col[j] + 5 : (col[j] >= 6 && col[j] <= 10) ? col[j] - 5 : col[j];
+    }
     float (*pool)[kPoolStride] = s_all.pool[warp];
-    const int n_groups = (n_items + 15) >> 4;
+    const int n_groups = (n_out + 15) >> 4;
     const size_t item_stride = (size_t)rows * DIN;
     for (int grp = blockIdx.x * kMmaWarps + warp; grp < n_groups; grp += gridDim.x * kMmaWarps) {
+        uint32_t bad = 0;                         // bit j8 / 8 + j8: that output's index is out of range (NaN)
 #pragma unroll 1
         for (int j8 = 0; j8 < 8; j8++) {
-            const int ia = grp * 16 + j8, ib = ia + 8;
-            const bool has_a = ia < n_items, has_b = ib < n_items;       // (warp-uniform)
-            const float* fa = features + (size_t)(has_a ? ia : 0) * item_stride;
-            const float* fb = features + (size_t)(has_b ? ib : 0) * item_stride;
+            const int ea = grp * 16 + j8, eb = ea + 8;                   // the outputs (warp-uniform from here on)
+            const bool out_a = ea < n_out, out_b = eb < n_out;
+            const long long sa = out_a ? (VIEWS && index ? index[ea] : ea) : 0, sb = out_b ? (VIEWS && index ? index[eb] : eb) : 0;
+            const bool has_a = out_a && (!VIEWS || (sa >= -1 && sa < n_items)), has_b = out_b && (!VIEWS || (sb >= -1 && sb < n_items));
+            const bool rd_a = has_a && (!VIEWS || sa >= 0), rd_b = has_b && (!VIEWS || sb >= 0);   // (index -1: all -1, not read)
+            bad |= (out_a && !has_a ? 1u << j8 : 0u) | (out_b && !has_b ? 1u << (8 + j8) : 0u);
+            const bool v1_a = VIEWS && DIN == 15 && view && out_a && view[ea], v1_b = VIEWS && DIN == 15 && view && out_b && view[eb];
+            const float* fa = features + (size_t)(rd_a ? sa : 0) * item_stride;
+            const float* fb = features + (size_t)(rd_b ? sb : 0) * item_stride;
             float best[4][4];
 #pragma unroll
             for (int nt = 0; nt < 4; nt++)
@@ -1453,12 +1475,12 @@ value_forward_kernel(const float* __restrict__ features, float* __restrict__ q_o
                 // the type flags first (column 0: lanes t == 0), handed to the quad
                 float flag_a = -1.f, flag_b = -1.f;
                 if (t == 0 && in_range) {
-                    if (has_a) flag_a = fa[(size_t)r * DIN];
-                    if (has_b) flag_b = fb[(size_t)r * DIN];
+                    if (rd_a) flag_a = fa[(size_t)r * DIN];
+                    if (rd_b) flag_b = fb[(size_t)r * DIN];
                 }
                 flag_a = __shfl_sync(0xffffffffu, flag_a, lane & ~3);
                 flag_b = __shfl_sync(0xffffffffu, flag_b, lane & ~3);
-                const bool live_a = in_range && has_a && !(flag_a < 0.f), live_b = in_range && has_b && !(flag_b < 0.f);
+                const bool live_a = in_range && rd_a && !(flag_a < 0.f), live_b = in_range && rd_b && !(flag_b < 0.f);
                 const bool any_live = __ballot_sync(0xffffffffu, live_a | live_b) != 0u;
                 if (!any_live && seen_a && seen_b) continue;             // padding only, and nobody's maximum can be there
                 seen_a |= __ballot_sync(0xffffffffu, live_a) != 0u;
@@ -1468,8 +1490,8 @@ value_forward_kernel(const float* __restrict__ features, float* __restrict__ q_o
                 for (int j = 0; j < 4; j++) {
                     xa[j] = xb[j] = 0.f;
                     if (col[j] < DIN && in_range) {
-                        if (has_a) xa[j] = (col[j] == 0) ? flag_a : fa[(size_t)r * DIN + col[j]];
-                        if (has_b) xb[j] = (col[j] == 0) ? flag_b : fb[(size_t)r * DIN + col[j]];
+                        if (has_a) xa[j] = (col[j] == 0) ? flag_a : rd_a ? fa[(size_t)r * DIN + (v1_a ? col1[j] : col[j])] : -1.f;
+                        if (has_b) xb[j] = (col[j] == 0) ? flag_b : rd_b ? fb[(size_t)r * DIN + (v1_b ? col1[j] : col[j])] : -1.f;
                     }
                 }
                 float acc[4][4], nxt[4][4];
@@ -1565,17 +1587,27 @@ value_forward_kernel(const float* __restrict__ features, float* __restrict__ q_o
             q4[0][0] = b2.x; q4[0][1] = b2.y; q4[0][2] = b2.x; q4[0][3] = b2.y;
         }
         mma_layer<1, true>(q4, h2, &s_w.v0[0][0], lane);
-        // this lane: outputs 2t, 2t + 1 of item grp * 16 + gq (entries 0-1) and of item grp * 16 + 8 + gq (entries 2-3)
+        // this lane: outputs 2t, 2t + 1 of output grp * 16 + gq (entries 0-1) and of output grp * 16 + 8 + gq (entries 2-3)
+        const float nan = __int_as_float(0x7fc00000);
 #pragma unroll
         for (int e = 0; e < 2; e++) {
             if (2 * t + e < nout) {
-                const int ia = grp * 16 + gq, ib = ia + 8;
-                if (ia < n_items) q_out[(size_t)ia * nout + 2 * t + e] = tanhf(q4[0][e]);
-                if (ib < n_items) q_out[(size_t)ib * nout + 2 * t + e] = tanhf(q4[0][2 + e]);
+                const int oa = grp * 16 + gq, ob = oa + 8;
+                if (oa < n_out) q_out[(size_t)oa * nout + 2 * t + e] = (bad >> gq) & 1u ? nan : tanhf(q4[0][e]);
+                if (ob < n_out) q_out[(size_t)ob * nout + 2 * t + e] = (bad >> (8 + gq)) & 1u ? nan : tanhf(q4[0][2 + e]);
             }
         }
         __syncwarp();
     }
+}
+
+template <int DIN>
+__global__ void __launch_bounds__(kMmaWarps * 32, ASTRO_MMA_MIN_BLOCKS)
+value_forward_kernel(const float* __restrict__ features, float* __restrict__ q_out, int n_items, int rows, int nout,
+                     const PolicyFragWeights* __restrict__ frags, const int64_t* __restrict__ index,
+                     const uint8_t* __restrict__ view, int n_out) {
+    if (index || view) value_forward_body<DIN, true>(features, q_out, n_items, rows, nout, frags, index, view, n_out);
+    else value_forward_body<DIN, false>(features, q_out, n_items, rows, nout, frags, nullptr, nullptr, n_out);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -3505,27 +3537,46 @@ int astro_stats(AstroBatch* b, int64_t* counters_dev, int32_t clear, void* strea
     return ASTRO_OK;
 }
 
+static int value_forward_launch(AstroBatch* b, const float* features, int32_t n_items, int32_t rows, const int64_t* index,
+                                const uint8_t* view, int32_t n_out, float* q_out, cudaStream_t st) {
+    CUDA_TRY(cudaSetDevice(b->device));
+    int grid = ((n_out + 15) / 16 + kMmaWarps - 1) / kMmaWarps;        // a warp takes 16 outputs at a time
+    if (grid > b->sm_count * ASTRO_MMA_MIN_BLOCKS) grid = b->sm_count * ASTRO_MMA_MIN_BLOCKS;
+    const int smem = (int)sizeof(PolicyFrags);
+    if (b->S == 2) {
+        CUDA_TRY(cudaFuncSetAttribute(value_forward_kernel<15>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        value_forward_kernel<15><<<grid, kMmaWarps * 32, smem, st>>>(features, q_out, n_items, rows, b->policy_nout, b->d_pol_frags,
+                                                                     index, view, n_out);
+    } else {
+        CUDA_TRY(cudaFuncSetAttribute(value_forward_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        value_forward_kernel<10><<<grid, kMmaWarps * 32, smem, st>>>(features, q_out, n_items, rows, b->policy_nout, b->d_pol_frags,
+                                                                     index, nullptr, n_out);
+    }
+    CUDA_TRY(cudaGetLastError());
+    b->launches += 1;
+    return ASTRO_OK;
+}
+
 int astro_value_forward(AstroBatch* b, const float* features, int32_t n_items, int32_t rows, float* q_out, void* stream) {
     if (int r = check(b, false)) return r;
     if (b->policy_nout <= 0 || !b->d_pol_frags) return fail(ASTRO_E_STATE, "astro_policy_set_weights has not been called");
     if (!features || !q_out) return fail(ASTRO_E_INVALID, "null argument");
     if (n_items < 0 || rows < 1) return fail(ASTRO_E_INVALID, "n_items >= 0 and rows >= 1");
     if (n_items == 0) return ASTRO_OK;
-    CUDA_TRY(cudaSetDevice(b->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    int grid = ((n_items + 15) / 16 + kMmaWarps - 1) / kMmaWarps;      // a warp takes 16 items at a time
-    if (grid > b->sm_count * ASTRO_MMA_MIN_BLOCKS) grid = b->sm_count * ASTRO_MMA_MIN_BLOCKS;
-    const int smem = (int)sizeof(PolicyFrags);
-    if (b->S == 2) {
-        CUDA_TRY(cudaFuncSetAttribute(value_forward_kernel<15>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        value_forward_kernel<15><<<grid, kMmaWarps * 32, smem, st>>>(features, q_out, n_items, rows, b->policy_nout, b->d_pol_frags);
-    } else {
-        CUDA_TRY(cudaFuncSetAttribute(value_forward_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        value_forward_kernel<10><<<grid, kMmaWarps * 32, smem, st>>>(features, q_out, n_items, rows, b->policy_nout, b->d_pol_frags);
-    }
-    CUDA_TRY(cudaGetLastError());
-    b->launches += 1;
-    return ASTRO_OK;
+    return value_forward_launch(b, features, n_items, rows, nullptr, nullptr, n_items, q_out, (cudaStream_t)stream);
+}
+
+int astro_value_forward_views(AstroBatch* b, const float* features, int32_t n_items, int32_t rows, const int64_t* index,
+                              const uint8_t* view, int32_t n_out, float* q_out, void* stream) {
+    // the arguments first (they need no batch), then the batch
+    if (n_items < 0 || n_out < 0 || rows < 1) return fail(ASTRO_E_INVALID, "n_items >= 0, n_out >= 0 and rows >= 1");
+    if (!index && n_out > n_items) return fail(ASTRO_E_INVALID, "without an index, output e is item e: n_out <= n_items");
+    if ((n_items > 0 && !features) || (n_out > 0 && !q_out)) return fail(ASTRO_E_INVALID, "null features or q_out");
+    if (int r = check(b, false)) return r;
+    if (b->policy_nout <= 0 || !b->d_pol_frags) return fail(ASTRO_E_STATE, "astro_policy_set_weights has not been called");
+    if (view && b->S != 2) return fail(ASTRO_E_INVALID, "a view array needs duel features (din 15)");
+    if (n_out == 0) return ASTRO_OK;
+    return value_forward_launch(b, features, n_items, rows, index, view, n_out, q_out, (cudaStream_t)stream);
 }
 
 int astro_stats_peer_create(AstroBatch* b, int32_t rank, int32_t world, uint8_t* handle_out) {

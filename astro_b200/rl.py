@@ -19,6 +19,8 @@ from . import core
 from .batched import BatchedGames
 
 _CACHE = {}
+_BOTH = {}
+_SWAP = [0, 6, 7, 8, 9, 10, 1, 2, 3, 4, 5, 11, 12, 13, 14]     # ship 1's feature columns in ship 0's view (core.roll_ships)
 
 def _games(solo, n, cap, device=None):
     n_pad = max(32, -(-n // 32) * 32)
@@ -28,6 +30,15 @@ def _games(solo, n, cap, device=None):
         cfg = core.SOLO_CONFIG if solo else core.DEFAULT_CONFIG
         g = _CACHE[key] = BatchedGames(cfg, n_pad, bullet_cap=cap, precision=64, **({} if device is None else dict(device=device)))
     return g
+
+def _both_views(n, device):
+    """forward_views' (index, view) of forward_both on n items: every item as ship 0, then as ship 1.  One pair per device,
+    for the largest n asked so far; smaller n take its first 2n entries."""
+    iv = _BOTH.get(device)
+    if iv is None or iv[0].shape[0] < 2 * n:
+        iv = _BOTH[device] = (torch.arange(n, device=device).repeat_interleave(2),
+                              torch.arange(2 * n, device=device).remainder(2).to(torch.uint8))
+    return iv[0][:2 * n], iv[1][:2 * n]
 
 class ValueNetwork(torch.nn.Module):
     """The reference's Q-network (rl.py:32-165) with the feature extraction on the GPU.
@@ -103,10 +114,21 @@ class ValueNetwork(torch.nn.Module):
         Ship 1's features are ship 0's with the ship column groups exchanged (core.roll_ships,
         core.py:306-327 + rl.py:62-70); exchanging the matching COLUMNS of the first layer's weight
         gives the same pre-activations without a second observation tensor
-        (`BatchedGames.observe(shared=True)`)."""
+        (`BatchedGames.observe(shared=True)`).  Under the conditions of `forward`'s kernel this is
+        forward_views of every item as ship 0 and as ship 1 (value_forward_kernel reads ship 1's
+        columns in place): bit for bit forward() of the two-view tensor observe() gives."""
         if x.shape[-1] != 15:
             raise ValueError('forward_both needs duel features [..., N, 15]')
-        swap = torch.tensor([0, 6, 7, 8, 9, 10, 1, 2, 3, 4, 5, 11, 12, 13, 14], device=x.device)
+        g = self._fused(x)
+        if g is not None:
+            flat = x.reshape(-1, x.shape[-2], 15)
+            index, view = _both_views(flat.shape[0], x.device)
+            return g.value_forward_views(flat, index, view).view(tuple(x.shape[:-2]) + (2, -1))
+        return self.forward_both_torch(x)
+
+    def forward_both_torch(self, x):
+        """forward_both layer by layer in PyTorch (training, CPU tensors, float64 features)."""
+        swap = torch.tensor(_SWAP, device=x.device)
         w = torch.cat((self.f0.weight, self.f0.weight[:, swap]), dim=0)           # [64, 15]
         b = torch.cat((self.f0.bias, self.f0.bias), dim=0)
         h = torch.nn.functional.linear(x, w, b)                                    # [..., N, 64]
@@ -117,6 +139,43 @@ class ValueNetwork(torch.nn.Module):
         for layer in self.v:
             h = self.activation(layer(h))
         return torch.tanh(self.v0(h))
+
+    def forward_views(self, x, index, view=None):
+        """The network on gathered views of ONE perspective-0 feature batch x [M, N, D] -> [E, nout]: output e is forward()
+        of item index[e] as ship view[e] sees it (ship 1: the ship column groups exchanged, as forward_both), index -1 an
+        item whose every entry is -1 (a finished game: the new state of a terminal pair).  index: int64 [E] on x's device;
+        view: uint8 [E] (0 = ship 0, otherwise ship 1) or None (ship 0; solo features, D = 10, take none).
+
+        Under the conditions of `forward`'s kernel (cuda float32, no autograd) this is one value_forward_kernel launch that
+        reads each row where the view has it, so no [E, N, D] tensor is made; otherwise the gather, the column exchange and
+        forward_torch in PyTorch, with the same values.  Raises ValueError before any launch on a dtype or shape that does
+        not fit, or an index outside -1 .. M - 1 (one reduction over index)."""
+        D = self.f0.in_features
+        if not (x.dim() == 3 and x.shape[-1] == D and x.shape[-2] >= 1 and x.is_floating_point()):
+            raise ValueError('forward_views needs a feature batch [M, N, %d] (N >= 1)' % D)
+        if not (isinstance(index, torch.Tensor) and index.dtype == torch.int64 and index.dim() == 1 and index.device == x.device):
+            raise ValueError('index must be an int64 tensor [E] on the features\' device')
+        if view is not None and not (D == 15 and isinstance(view, torch.Tensor) and view.dtype == torch.uint8
+                                     and view.shape == index.shape and view.device == x.device):
+            raise ValueError('view must be a uint8 tensor shaped like index on the features\' device (duel features only)')
+        if index.numel():
+            lo, hi = (int(v) for v in torch.aminmax(index))
+            if lo < -1 or hi >= x.shape[0]:
+                raise ValueError('index values %d .. %d outside -1 .. %d' % (lo, hi, x.shape[0] - 1))
+        g = self._fused(x)
+        if g is not None:
+            return g.value_forward_views(x, index, view)
+        return self.forward_torch(self._gather_views(x, index, view))
+
+    @staticmethod
+    def _gather_views(x, index, view):
+        """The [E, N, D] tensor forward_views evaluates: x[index], all -1 where index is -1, the ship column groups
+        exchanged where view is set."""
+        items = x[index.clamp(min=0)] if x.shape[0] else x.new_full((index.shape[0],) + tuple(x.shape[1:]), -1.0)
+        items = torch.where((index < 0)[:, None, None], torch.full_like(items, -1.0), items)
+        if view is not None:
+            items = torch.where((view != 0)[:, None, None], items[..., torch.tensor(_SWAP, device=x.device)], items)
+        return items
 
     def evaluate(self, state):
         dev = next(self.parameters()).device

@@ -459,6 +459,21 @@ int astro_stats(AstroBatch* b, int64_t* counters_dev, int32_t clear, void* strea
  * Tensor-core kernel (FP16 three-product split, fp32 accumulation): within 2e-6 of the PyTorch fp32 network. */
 int astro_value_forward(AstroBatch* b, const float* features, int32_t n_items, int32_t rows, float* q_out, void* stream);
 
+/* The same network on gathered views of a perspective-0 feature batch (astro_observe_shared's output, or an
+ * AstroRecordRing's observations): output e is the network on item index[e] as ship view[e] sees it, with ship 1's view
+ * = ship 0's with the two ship column groups (columns 1-5 and 6-10) exchanged — the value of the materialised view
+ * through astro_value_forward, bit for bit, without the view in memory.  Same weights and kernel as astro_value_forward.
+ *   features f32 [n_items][rows][din] device, contiguous (may be NULL when n_items = 0)
+ *   index    i64 [n_out] device, or NULL (output e = item e; then n_out <= n_items).  index -1 is an item whose every entry is -1 (the padding of
+ *            a finished game) and reads nothing; any other value outside 0 .. n_items - 1 is never read and its outputs
+ *            are NaN
+ *   view     u8 [n_out] device, 0 = ship 0, any other value ship 1; or NULL (ship 0 everywhere).  Duel batches (din 15) only
+ *   q_out    f32 [n_out][nout] device
+ * ASTRO_E_INVALID for a view array on solo features, negative sizes, rows < 1, n_out > n_items without an index, or a missing
+ * features / q_out pointer (the argument checks come before the batch's, so they hold for any handle). */
+int astro_value_forward_views(AstroBatch* b, const float* features, int32_t n_items, int32_t rows, const int64_t* index,
+                              const uint8_t* view, int32_t n_out, float* q_out, void* stream);
+
 /* The same counters summed over the N processes of one node (one GPU each; "NCCL used only for the optional episode-stats
  * reduction" in the north star — this is that reduction without NCCL): ONE kernel per rank that stores the rank's counters
  * into every rank's exchange buffer through peer memory (NVLink / NVSwitch, buffers mapped by CUDA IPC), waits for the other
